@@ -21,6 +21,10 @@ One "step" = one pass of that path over that batch.
   cpu_baseline: the float64 numpy oracle (a port: the reference has no windowed/overlapped path)
             on a bounded slice, single core, timed on this box.
 
+`--steps K` is the number of timed steps of each config-2 leg (device-resident, ring, one-shot call); the sustained
+leg runs for >= 2 s instead (`--no-sustained` skips it).
+`--dump-outputs DIR` writes what the device-resident step handed back in its last timed step as DIR/<name>.npy
+(float32 / float64; the inputs are seeded, so two builds can be compared output for output).
 `--impl reference` times the CPU oracle port with all host cores (multiprocessing over frame
 blocks) on the same config and prints the same line with "impl": "reference".
 Multi-GPU: config 2 is one ordered stream, so for `value` / `e2e` the ranks are independent replicas (one stream per
@@ -39,10 +43,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 NFFT, HOP, FS, FC = 4096, 1024, 61.44e6, 2.4e9
 L_STEP = 61_440_000
 VMIN, VMAX = 20.0, 130.0
+DUMP_ROWS = 2048                                  # seeded sample of the 59 997 waterfall rows: 32 MiB as float32
 BYTES_PER_SAMPLE = 4 + (NFFT // HOP) * 1          # int16 IQ in + four u8 rows touched per sample
 FLOP_PER_SAMPLE = (NFFT // HOP) * (5 * 12 + 20)   # SURVEY.md 8(d)
 METRIC = "IQ Msamples/s through windowed FFT->PSD->waterfall"
@@ -256,10 +262,25 @@ def traffic_record(kernel_name):
         return None, f"no traffic record: {exc}"
 
 
+def dump_outputs(out_dir, wf_rows, welch_acc, maxhold, pxx, pdb, feat):
+    """The outputs of one device-resident step as DIR/<name>.npy: a fixed, seeded sample of the uint8 waterfall rows
+    (values as float32, row indices beside them), the Welch sum, max-hold, PSD, PSD in dB and the classifier features
+    (the numeric fields of spx_features in declaration order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = wf_rows.to_host()
+    idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], min(DUMP_ROWS, rows.shape[0]), replace=False))
+    out = {"wf_rows_sample": rows[idx].astype(np.float32), "wf_rows_sample_index": idx.astype(np.float64),
+           "welch_acc": welch_acc.to_host().reshape(-1), "maxhold": maxhold.to_host().reshape(-1),
+           "pxx": pxx.to_host(), "pxx_db": pdb.to_host(),
+           "features": np.array([float(v) for k, v in feat.items() if k != "peaks"], np.float64)}
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of each config-2 leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--variant", type=int, default=int(os.environ.get("SPX_VARIANT", "-1")))
@@ -268,7 +289,12 @@ def main():
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--no-views", action="store_true", help="skip the config-3 block (I/Q histogram, frame stats)")
     ap.add_argument("--sharded-log2", type=int, default=30, help="config-5 capture length (2^30 is BASELINE's size)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
@@ -352,6 +378,9 @@ def main():
     nat.device_sync(dev)
     feat = fq[last_slot[1]].results(last_slot[0])[0]
     kernel_ms = [t.elapsed_ms() for t in kernel_timers]
+    if args.dump_outputs and rank == 0:     # before the sustained leg overwrites these buffers
+        b = last_slot[1]
+        dump_outputs(args.dump_outputs, d_wf, d_we[b], d_mh[b], d_pxx[b], d_pdb[b], feat)
     dt_dev = barrier_max(dist, local, dt_dev)
 
     # ---------------- sustained leg: the same step back to back for >= 2 s (a 13 ms burst cannot show a power / thermal
@@ -388,7 +417,7 @@ def main():
     RING_SLOTS = 6      # five in flight + the one the producer fills: with fewer the two upload streams cannot both stay busy
     rg = ringmod.StreamRing(pl, n_slots=RING_SLOTS, slot_samples=SLOT, wf_rows=True, welch=True, maxhold=True, vmin=VMIN, vmax=VMAX,
                             features=True, sample_rate=FS)
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
 
     ring_state = {"pending": 0, "last": None}
 
@@ -433,7 +462,7 @@ def main():
     h_wf = nat.pinned_empty((F, NFFT), np.uint8)
     h_we = nat.pinned_empty((1, NFFT), np.float64)
     h_mh = nat.pinned_empty((1, NFFT), np.float32)
-    call_steps = 3
+    call_steps = args.steps
 
     def e2e_step():
         r = pl.stft(host_in, wf_rows=h_wf, welch=h_we, maxhold=h_mh, vmin=VMIN, vmax=VMAX)

@@ -7,10 +7,10 @@ values (noise floor, threshold, bin indices, peak list) that the CUDA feature ke
 checked against.  The label rules / temporal smoothing (classifier.py:60-161) are scalar
 host logic and are checked end-to-end against the imported reference instead.
 
-Pinned by: importing the reference module in the build container
-(``tests/test_oracle.py::test_classifier_oracle_vs_reference``, skipped when
-/root/reference is absent) and by ``tests/golden/classifier_cases.json`` generated from the
-reference by ``tests/golden/make_golden.py`` (includes SURVEY.md 8(c) KA-1 / KA-2).
+Pinned by the reference's own outputs, stored: ``tests/golden/classifier_random.json``
+(its helpers on random spectra with ties, ``tests/test_oracle.py::test_classifier_oracle_vs_reference_random``)
+and ``tests/golden/classifier_cases.json`` generated from the reference by
+``tests/golden/make_golden.py`` (includes SURVEY.md 8(c) KA-1 / KA-2).
 """
 from __future__ import annotations
 

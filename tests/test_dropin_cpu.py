@@ -1,9 +1,9 @@
-"""CPU tests of the drop-in boundary: the reference's own mock-based streamer tests run against OUR
-`app.sdr.streamer`, the C ABI exports every symbol include/spx.h declares, and the product fails
+"""CPU tests of the drop-in boundary: the streamer surface of `app.sdr.streamer` behaves like the
+reference's, the C ABI exports every symbol include/spx.h declares, and the product fails
 loudly without a GPU (no CPU fallback)."""
+import hashlib
 import os
 import re
-import subprocess
 import sys
 from unittest.mock import MagicMock
 
@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REFERENCE_TEST_CLASSIFIER_SHA256 = "81b5422a44e9c1b337f15d66b1cca256576cb665007569d4318e57a9e3123678"
 
 
 def test_abi_exports_every_declared_symbol():
@@ -133,28 +133,12 @@ def test_two_consumers_share_the_queue_like_the_reference():
     assert s.peek_latest() == {"i": 2} and s.data_queue.qsize() == 1
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_reference_streamer_suite_passes_on_drop_in():
-    """Run the reference's tests/test_streamer.py unchanged with `app` resolving to this repo."""
-    env = dict(os.environ, PYTHONPATH=ROOT)
-    res = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider",
-                          os.path.join(REF, "tests", "test_streamer.py"), "--rootdir", ROOT],
-                         cwd=ROOT, env=env, capture_output=True, text=True)
-    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-    assert "6 passed" in res.stdout
-
-
 def test_vendored_reference_test_is_verbatim():
-    """tests/golden/reference_test_classifier.py is the reference's tests/test_classifier.py byte for byte (checked when
-    /root/reference is present, i.e. in the build container)."""
-    import os
-    ref = "/root/reference/tests/test_classifier.py"
-    if not os.path.exists(ref):
-        import pytest
-        pytest.skip("reference tree not present on this box")
+    """tests/golden/reference_test_classifier.py is the reference's tests/test_classifier.py byte for byte: the digest
+    is the reference file's SHA-256."""
     here = os.path.join(os.path.dirname(__file__), "golden", "reference_test_classifier.py")
-    with open(ref, "rb") as a, open(here, "rb") as b:
-        assert a.read() == b.read()
+    with open(here, "rb") as fh:
+        assert hashlib.sha256(fh.read()).hexdigest() == REFERENCE_TEST_CLASSIFIER_SHA256
 
 
 def test_failed_library_load_is_cached(monkeypatch, tmp_path):

@@ -1,7 +1,6 @@
-"""CPU tests: the oracle against the reference's golden vectors, scipy, and (when present)
-the reference itself.  No GPU needed."""
+"""CPU tests: the oracle against the reference's golden vectors and scipy.  No GPU needed."""
+import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -10,7 +9,7 @@ import scipy.signal
 from oracle import classifier_ref as cref
 from oracle import spectral_ref as sref
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def test_stream_frames_match_reference_golden(golden_stream):
@@ -145,31 +144,23 @@ def test_known_answers_ka1_ka2(golden_classifier):
     assert g["peak_count"] == 2 and round(g["snr_db"], 2) == 41.36
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 def test_classifier_oracle_vs_reference_random():
-    """Import the reference and compare helper-by-helper on random spectra."""
-    saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "app" or k.startswith("app.")}
-    sys.path.insert(0, REF)
-    try:
-        from app.processing import classifier as rc
-    finally:
-        sys.path.pop(0)
-        for k in [k for k in sys.modules if k == "app" or k.startswith("app.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-    rng = np.random.default_rng(5)
-    for n in (3, 7, 100, 299, 300, 1024, 5000):
-        for _ in range(4):
-            p = rng.normal(-80, 3, n)
-            p[rng.integers(0, n, size=max(1, n // 50))] += rng.uniform(5, 50)
-            p = np.round(p, 1)  # force ties
-            f = np.linspace(1e9, 1.02e9, n)
-            g = cref.features(f, p)
-            nf = rc._estimate_noise_floor(p)
-            assert g["noise_floor_db"] == nf
-            assert g["peaks"] == rc._find_peaks(p, g["adaptive_thr"], g["min_distance_bins"])
-            for d, key in ((3, "bw3"), (10, "bw10"), (20, "bw20")):
-                assert g[key] == rc._occupied_bandwidth(f, p, d)
-            assert abs(g["flatness"] - rc._spectral_flatness(p)) <= 1e-15
-            assert abs(g["kurtosis"] - rc._spectral_kurtosis(p)) <= 1e-12 * max(1, abs(g["kurtosis"]))
-            assert g["peak_spacing_std_hz"] == rc._peak_spacing_std(f, g["peaks"])
+    """Helper by helper against the reference's classifier on random spectra with ties (n = 3 ... 5000): its noise
+    floor, peak pick, occupied bandwidths, flatness, kurtosis and peak spacing on these inputs are stored in
+    tests/golden/classifier_random.{npz,json}."""
+    z = np.load(os.path.join(GOLDEN, "classifier_random.npz"))
+    with open(os.path.join(GOLDEN, "classifier_random.json")) as fh:
+        cases = json.load(fh)["cases"]
+    assert len(cases) == 28
+    for want in cases:
+        p = z[want["key"]] / 10.0       # dB rounded to 0.1 (forces ties), stored as int16 tenths
+        assert p.size == want["n"]
+        f = np.linspace(1e9, 1.02e9, p.size)
+        g = cref.features(f, p)
+        assert g["noise_floor_db"] == want["noise_floor_db"], want["key"]
+        assert (g["adaptive_thr"], g["min_distance_bins"]) == (want["adaptive_thr"], want["min_distance_bins"]), want["key"]
+        assert g["peaks"] == want["peaks"], want["key"]
+        assert [g["bw3"], g["bw10"], g["bw20"]] == want["bw"], want["key"]
+        assert abs(g["flatness"] - want["flatness"]) <= 1e-15, want["key"]
+        assert abs(g["kurtosis"] - want["kurtosis"]) <= 1e-12 * max(1, abs(g["kurtosis"])), want["key"]
+        assert g["peak_spacing_std_hz"] == want["peak_spacing_std_hz"], want["key"]

@@ -151,6 +151,14 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
     float* d_max = a->maxhold ? (float*)pl->st_max.ptr : nullptr;
     long long h2d = 0, d2h = 0;
 
+    // plan-owned scratch (four-step / K2v2 / Bluestein buffers): a device-resident call on a caller stream may still be
+    // using it, so the kernels queued here on s_compute wait for that call first, as the device path does
+    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0;
+    if (owns_scratch) {
+        if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
+        if (pl->scratch_stream_valid && pl->scratch_stream != pl->s_compute) SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, pl->ev_scratch, 0));
+    }
+
     // accumulators: start from zero or from the caller's running values
     if (d_welch) {
         if (a->accumulate) {
@@ -245,6 +253,11 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
     if (d_max) {
         SPX_CUDA(cudaMemcpyAsync(a->maxhold, d_max, (size_t)S * N * sizeof(float), cudaMemcpyDeviceToHost, pl->s_compute));
         d2h += S * N * (long long)sizeof(float);
+    }
+    if (owns_scratch) {
+        SPX_CUDA(cudaEventRecord(pl->ev_scratch, pl->s_compute));
+        pl->scratch_stream = pl->s_compute;
+        pl->scratch_stream_valid = true;
     }
     SPX_CUDA(cudaStreamSynchronize(pl->s_h2d));
     SPX_CUDA(cudaStreamSynchronize(pl->s_h2d_alt));

@@ -364,7 +364,9 @@ def test_large_n_four_step_parity(sp, nfft, hop, kind, fmt):
 
 
 def test_large_n_tone_bins_and_batches(sp):
-    """integer bin placement for N = 65536 and batching through a small scratch (several A/B launches)."""
+    """integer bin placement for N = 65536: a pure tone at bin k lands at fftshift position (k + N/2) mod N, for bins at
+    and around the 256-point sub-transform boundaries, DC, Nyquist and the last bin (one frame each, dB rows, K2).
+    Batching through several scratch batches is tested in test_dispatch_paths_gpu.py."""
     n = 65536
     t = np.arange(n)
     pl = sp.SpectralPlan(n, n, "rect")

@@ -213,6 +213,17 @@ typedef struct {
  * mlab.psd behind process_sigmf_data.py:188, batched over all frames of the input. */
 SPX_API int spx_stft_exec(spx_plan* plan, spx_stft_args* args);
 
+/* spx_stft_exec plus the persistence spectrum of the call's uint8 waterfall levels (counts[n_streams][256][nfft],
+ * uint32, in args->mem space; args->accumulate applies to it as to welch_acc / maxhold).  args->wf_rows may be NULL:
+ * the rows are then produced into plan-owned device scratch and never leave the GPU.
+ *   counts[s][q][j] = number of frames f of stream s whose level wf_rows[s*F + f][j] is q, so every column sums to F.
+ * Level q holds dB values in [vmin + q*D, vmin + (q+1)*D), D = (vmax - vmin)/256; level 0 also holds everything below
+ * vmin and NaN, level 255 everything at or above vmax - D.  Needs vmax > vmin even without wf_rows; peer_outputs != 0
+ * returns SPX_E_UNSUPPORTED.  Without caller rows, a device-resident call transforms the frames in batches through a
+ * row buffer of SPX_PERSIST_ROWS_BYTES (plan-creation environment variable, default 64 MiB), and a host-memory call
+ * copies back only the counts and the accumulators (d2h_bytes_out). */
+SPX_API int spx_stft_exec_persistence(spx_plan* plan, spx_stft_args* args, uint32_t* counts);
+
 /* Measurement helper: runs spx_stft_exec (SPX_MEM_DEVICE buffers only) warmup+iters times on the
  * launch stream, each bracketed by CUDA events; optionally READS a 256 MiB buffer before every
  * iteration to flush the 126 MB L2 without leaving dirty lines behind.  ms_each[iters] receives the device time of

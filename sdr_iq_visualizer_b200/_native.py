@@ -111,6 +111,7 @@ _SIGNATURES = {
     "spx_plan_destroy": (C.c_int, [C.c_void_p]),
     "spx_plan_sync": (C.c_int, [C.c_void_p]),
     "spx_stft_exec": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args)]),
+    "spx_stft_exec_persistence": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.c_void_p]),
     "spx_stft_time": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.c_int32, C.c_int32, C.c_int32,
                                 C.POINTER(C.c_float)]),
     "spx_welch_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,

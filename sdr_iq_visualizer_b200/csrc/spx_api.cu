@@ -130,8 +130,45 @@ int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long l
 
 static size_t in_elt(const spx_plan* pl) { return pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8; }
 
+// ------------------------------------------------------------------ persistence spectrum without caller rows
+// The STFT of frames [0, F) of every stream goes in batches through the plan's row buffer (SPX_PERSIST_ROWS_BYTES), each
+// batch followed by its histogram on the same stream, so the uint8 rows never leave the GPU.  The buffer holds
+// max(1, bytes / (S N)) frames of the S streams of a batch: it exceeds SPX_PERSIST_ROWS_BYTES only when a single frame
+// of every stream does (S N > bytes).  A batch starts f0 * hop samples into every stream: f0 * hop * elt keeps the input alignment (128 bytes for
+// K1v2, 16 bytes for K1's staged loads and K2v2) and K2v2's hop % 256 of the unbatched call, and a batch covers all
+// streams with the call's stride, so each batch runs the kernel family the unbatched call would.  Exception: float rows
+// (db_rows / spec_rows) of several streams must land at rows s * F + f, so those batches run one stream at a time.
+static long long persist_batch_frames(const spx_plan* pl, long long Sb, long long F) {
+    long long fb = (long long)(pl->persist_rows_bytes / ((size_t)Sb * pl->cfg.nfft));
+    if (fb < 1) fb = 1;
+    return fb < F ? fb : F;
+}
+
+static int persist_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, float* db_rows,
+                           float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, uint32_t* counts,
+                           cudaStream_t st) {
+    const int N = pl->cfg.nfft, hop = pl->cfg.hop;
+    const size_t elt = in_elt(pl);
+    const long long Sb = S > 1 && (db_rows || spec_rows) ? 1 : S;
+    const long long fb = persist_batch_frames(pl, Sb, F);
+    SPX_TRY(pl->st_persist.reserve((size_t)(Sb * fb) * N));   // a no-op when the host pipeline reserved it up front
+    unsigned char* rows = (unsigned char*)pl->st_persist.ptr;
+    for (long long s = 0; s < S; s += Sb) {
+        for (long long f0 = 0; f0 < F; f0 += fb) {
+            const long long nf = F - f0 < fb ? F - f0 : fb;
+            const size_t r0 = (size_t)(s * F + f0) * N;
+            SPX_TRY(stft_launch_device(pl, in + (size_t)(s * stride + f0 * hop) * elt, Sb, stride, nf,
+                                       db_rows ? db_rows + r0 : nullptr, rows, spec_rows ? spec_rows + r0 : nullptr,
+                                       welch_acc ? welch_acc + s * N : nullptr, maxhold ? maxhold + s * N : nullptr, vmin,
+                                       vmax, st));
+            SPX_TRY(persist_launch(pl, rows, Sb, nf, counts + (size_t)s * 256 * N, st));
+        }
+    }
+    return SPX_OK;
+}
+
 // ------------------------------------------------------------------ host-memory pipeline
-static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
+static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t* counts) {
     const int N = pl->cfg.nfft, hop = pl->cfg.hop;
     const size_t elt = in_elt(pl);
     const long long S = a->n_streams, L = a->n_samples;
@@ -151,9 +188,10 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
     float* d_max = a->maxhold ? (float*)pl->st_max.ptr : nullptr;
     long long h2d = 0, d2h = 0;
 
-    // plan-owned scratch (four-step / K2v2 / Bluestein buffers): a device-resident call on a caller stream may still be
-    // using it, so the kernels queued here on s_compute wait for that call first, as the device path does
-    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0;
+    // plan-owned scratch (four-step / K2v2 / Bluestein buffers, the persistence row buffer): a device-resident call on a
+    // caller stream may still be using it, so the kernels queued here on s_compute wait for that call first, as the
+    // device path does
+    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || (counts && !a->wf_rows);
     if (owns_scratch) {
         if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
         if (pl->scratch_stream_valid && pl->scratch_stream != pl->s_compute) SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, pl->ev_scratch, 0));
@@ -176,10 +214,30 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
             SPX_CUDA(cudaMemsetAsync(d_max, 0, (size_t)S * N * sizeof(float), pl->s_compute));
         }
     }
+    // persistence counts: from the caller's running values only when accumulating
+    const size_t count_bytes = (size_t)S * 256 * N * sizeof(uint32_t);
+    uint32_t* d_counts = nullptr;
+    if (counts) {
+        SPX_TRY(pl->st_counts.reserve(count_bytes));
+        d_counts = (uint32_t*)pl->st_counts.ptr;
+        if (a->accumulate) {
+            SPX_CUDA(cudaMemcpyAsync(d_counts, counts, count_bytes, cudaMemcpyHostToDevice, pl->s_compute));
+            h2d += (long long)count_bytes;
+        } else {
+            SPX_CUDA(cudaMemsetAsync(d_counts, 0, count_bytes, pl->s_compute));
+        }
+    }
 
     // piece size: big enough to amortise launches, small enough to overlap (about 8-16 MiB)
     long long piece = (long long)(pl->piece_bytes / elt);
     if (piece < (long long)N * 4) piece = (long long)N * 4;
+    // counts without rows: one row buffer for every piece, sized for the largest (a piece spans at most `piece` samples,
+    // so at most piece / hop + 1 frames), reserved here -- growing it between pieces would free device memory, which
+    // synchronises the device in the middle of the pipeline
+    if (counts && !a->wf_rows) {
+        const long long most = piece / hop + 2 < F ? piece / hop + 2 : F;
+        SPX_TRY(pl->st_persist.reserve((size_t)persist_batch_frames(pl, 1, most) * N));
+    }
     struct Piece { long long s, f_lo, f_hi; };
     std::vector<Piece> pieces;
     size_t ev = 0;
@@ -215,10 +273,18 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
             SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, e_in, 0));
             const size_t r0 = (size_t)(s * F + f_lo);
             NvtxRange r_k("spx STFT kernel piece");
-            SPX_TRY(stft_launch_device(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo,
-                                       d_db ? d_db + r0 * N : nullptr, d_wf ? d_wf + r0 * N : nullptr,
-                                       d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
-                                       d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, pl->s_compute));
+            if (d_counts && !d_wf) {   // counts without rows: the piece's rows go through the plan's row buffer
+                SPX_TRY(persist_batches(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, d_db ? d_db + r0 * N : nullptr,
+                                        d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
+                                        d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, d_counts + (size_t)s * 256 * N,
+                                        pl->s_compute));
+            } else {
+                SPX_TRY(stft_launch_device(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo,
+                                           d_db ? d_db + r0 * N : nullptr, d_wf ? d_wf + r0 * N : nullptr,
+                                           d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
+                                           d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, pl->s_compute));
+                if (d_counts) SPX_TRY(persist_launch(pl, d_wf + r0 * N, 1, f_hi - f_lo, d_counts + (size_t)s * 256 * N, pl->s_compute));
+            }
             SPX_CUDA(cudaEventRecord(e_k, pl->s_compute));
             pieces.push_back({s, f_lo, f_hi});
             f_lo = f_hi;
@@ -253,6 +319,10 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F) {
     if (d_max) {
         SPX_CUDA(cudaMemcpyAsync(a->maxhold, d_max, (size_t)S * N * sizeof(float), cudaMemcpyDeviceToHost, pl->s_compute));
         d2h += S * N * (long long)sizeof(float);
+    }
+    if (d_counts) {
+        SPX_CUDA(cudaMemcpyAsync(counts, d_counts, count_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
+        d2h += (long long)count_bytes;
     }
     if (owns_scratch) {
         SPX_CUDA(cudaEventRecord(pl->ev_scratch, pl->s_compute));
@@ -550,6 +620,10 @@ int spx_plan_create(spx_plan** out, const spx_plan_config* cfg) {
     if (const char* e = getenv("SPX_PEER_PIECE_BYTES")) { long long v = atoll(e); if (v >= 4096) pl->peer_piece_bytes = (size_t)v; }
     if (const char* e = getenv("SPX_H2D_PIECE_BYTES")) { long long v = atoll(e); if (v >= 65536) pl->piece_bytes = (size_t)v; }
     if (const char* e = getenv("SPX_BIG_SCRATCH_BYTES")) { long long v = atoll(e); if (v >= (1 << 20)) pl->big_scratch_bytes = (size_t)v; }
+    if (const char* e = getenv("SPX_PERSIST_ROWS_BYTES")) {   // at least one row
+        long long v = atoll(e);
+        if (v > 0) pl->persist_rows_bytes = (size_t)v > (size_t)cfg->nfft ? (size_t)v : (size_t)cfg->nfft;
+    }
     int rc = SPX_OK;
     do {
         cudaError_t e;
@@ -609,6 +683,7 @@ int spx_plan_destroy(spx_plan* pl) {
     pl->st_big.release();
     pl->st_in.release(); pl->st_db.release(); pl->st_wf.release(); pl->st_spec.release();
     pl->st_welch.release(); pl->st_max.release(); pl->st_misc.release(); pl->st_flush.release();
+    pl->st_counts.release(); pl->st_persist.release();
     delete pl;
     return SPX_OK;
 }
@@ -716,14 +791,17 @@ int spx_plan_window_sums(spx_plan* pl, double* sum_w2, double* sum_w) {
     return SPX_OK;
 }
 
-int spx_stft_exec(spx_plan* pl, spx_stft_args* a) {
+// spx_stft_exec, plus the persistence counts [S][256][N] of the call's uint8 levels when `counts` is not NULL
+static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
     if (!pl || !a) return spx_set_error(SPX_E_INVALID, "NULL argument");
     if (a->struct_size != sizeof(spx_stft_args))
         return spx_set_error(SPX_E_INVALID, "spx_stft_args.struct_size %u != %zu", a->struct_size, sizeof(spx_stft_args));
+    if (counts && a->peer_outputs) return spx_set_error(SPX_E_UNSUPPORTED, "persistence with peer_outputs is not supported");
     if (a->n_streams < 1) return spx_set_error(SPX_E_INVALID, "n_streams must be >= 1");
     if (a->n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
     if (a->mem != SPX_MEM_HOST && a->mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", a->mem);
     if ((a->wf_rows != nullptr) && !(a->vmax > a->vmin)) return spx_set_error(SPX_E_INVALID, "wf_rows needs vmax > vmin");
+    if (counts && !(a->vmax > a->vmin)) return spx_set_error(SPX_E_INVALID, "persistence needs vmax > vmin");
     if (a->n_streams > 1 && a->stream_stride < a->n_samples && a->mem == SPX_MEM_HOST)
         return spx_set_error(SPX_E_INVALID, "stream_stride < n_samples");
     const long long F = spx_frame_count(a->n_samples, pl->cfg.nfft, pl->cfg.hop);
@@ -734,12 +812,15 @@ int spx_stft_exec(spx_plan* pl, spx_stft_args* a) {
     SPX_CUDA(cudaSetDevice(pl->cfg.device));
     const int N = pl->cfg.nfft;
     const long long S = a->n_streams;
+    const size_t count_bytes = (size_t)S * 256 * N * sizeof(uint32_t);
     if (a->in == nullptr && F > 0) return spx_set_error(SPX_E_INVALID, "in is NULL");
     if (a->mem == SPX_MEM_DEVICE) {
         cudaStream_t st = a->stream ? (cudaStream_t)a->stream : pl->s_compute;
-        // Plan-owned scratch (four-step / K2v2 scratch and counters, Bluestein buffers, peer staging) is shared by every
-        // call on this plan: a call on another stream than the previous one waits for that one's kernels first.
-        const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || a->peer_outputs;
+        // Plan-owned scratch (four-step / K2v2 scratch and counters, Bluestein buffers, peer staging, the persistence row
+        // buffer) is shared by every call on this plan: a call on another stream than the previous one waits for that
+        // one's kernels first.
+        const bool own_rows = counts && !a->wf_rows;
+        const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || a->peer_outputs || own_rows;
         if (owns_scratch) {
             if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
             if (pl->scratch_stream_valid && pl->scratch_stream != st) SPX_CUDA(cudaStreamWaitEvent(st, pl->ev_scratch, 0));
@@ -747,11 +828,16 @@ int spx_stft_exec(spx_plan* pl, spx_stft_args* a) {
         if (!a->accumulate) {
             if (a->welch_acc) SPX_CUDA(cudaMemsetAsync(a->welch_acc, 0, (size_t)S * N * sizeof(double), st));
             if (a->maxhold) SPX_CUDA(cudaMemsetAsync(a->maxhold, 0, (size_t)S * N * sizeof(float), st));
+            if (counts) SPX_CUDA(cudaMemsetAsync(counts, 0, count_bytes, st));
         }
         int rc;
-        if (a->peer_outputs && !a->db_rows && !a->spec_rows && F > 0) rc = stft_exec_device_peer(pl, a, F, st);
+        if (own_rows) rc = persist_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->db_rows,
+                                           reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold, a->vmin, a->vmax,
+                                           counts, st);
+        else if (a->peer_outputs && !a->db_rows && !a->spec_rows && F > 0) rc = stft_exec_device_peer(pl, a, F, st);
         else rc = stft_launch_device(pl, a->in, S, a->stream_stride, F, a->db_rows, a->wf_rows, reinterpret_cast<float2*>(a->spec_rows),
                                      a->welch_acc, a->maxhold, a->vmin, a->vmax, st, a->peer_outputs ? 1 : 0);
+        if (rc == SPX_OK && counts && !own_rows) rc = persist_launch(pl, a->wf_rows, S, F, counts, st);
         if (rc == SPX_OK && owns_scratch) {
             SPX_CUDA(cudaEventRecord(pl->ev_scratch, st));
             pl->scratch_stream = st;
@@ -763,10 +849,18 @@ int spx_stft_exec(spx_plan* pl, spx_stft_args* a) {
         if (!a->accumulate) {
             if (a->welch_acc) memset(a->welch_acc, 0, (size_t)S * N * sizeof(double));
             if (a->maxhold) memset(a->maxhold, 0, (size_t)S * N * sizeof(float));
+            if (counts) memset(counts, 0, count_bytes);
         }
         return SPX_OK;
     }
-    return stft_exec_host(pl, a, F);
+    return stft_exec_host(pl, a, F, counts);
+}
+
+int spx_stft_exec(spx_plan* pl, spx_stft_args* a) { return stft_exec(pl, a, nullptr); }
+
+int spx_stft_exec_persistence(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
+    if (!counts) return spx_set_error(SPX_E_INVALID, "counts is NULL");
+    return stft_exec(pl, a, counts);
 }
 
 int spx_stft_time(spx_plan* pl, spx_stft_args* a, int32_t warmup, int32_t iters, int32_t flush_l2, float* ms_each) {

@@ -33,8 +33,12 @@ struct spx_plan {
     std::vector<cudaEvent_t> events;
     size_t piece_bytes = 16u << 20;  // H2D piece size of the host pipeline
     size_t peer_piece_bytes = 48u << 20;  // uint8 rows per piece of the peer-output pipeline (two staging buffers)
+    size_t persist_rows_bytes = 64u << 20;  // uint8 row buffer of a device-resident persistence call without caller rows
     // staging for SPX_MEM_HOST execution (grow-only)
     spx::DevBuf st_in, st_db, st_wf, st_spec, st_welch, st_max, st_misc, st_flush;
+    // persistence spectrum: counts staging of the host path, and the plan-owned row buffer (device path without caller
+    // rows; host path without caller rows, one piece)
+    spx::DevBuf st_counts, st_persist;
     // large-N (four-step) path, nfft >= 16384
     int big_n1 = 0, big_n2 = 0;
     float2* d_big_tw = nullptr;  // one allocation holding the four tables below
@@ -71,6 +75,8 @@ int big2_plan_init(spx_plan* pl);
 bool big2_eligible(const spx_plan* pl, const void* in, const float* db_rows, const float2* spec_rows);
 int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, unsigned char* wf_rows, double* welch_acc,
                        float* maxhold, float vmin, float vmax, cudaStream_t st, int sys_atomics);
+int persist_launch(const spx_plan* pl, const uint8_t* rows, long long n_streams, long long frames, uint32_t* counts,
+                   cudaStream_t st);
 int welch_finalize_launch(const double* acc, int n, double inv_norm, double* pxx, double* pxx_db, cudaStream_t st);
 int bluestein_plan_init(spx_plan* pl);
 int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,

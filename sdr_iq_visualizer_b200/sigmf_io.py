@@ -226,16 +226,19 @@ class RecordingSpectra:
     center_freq: float = 0.0
     h2d_bytes: int = 0
     d2h_bytes: int = 0
+    persistence: Optional[np.ndarray] = None  # uint32 [256, N] frames per waterfall level and bin
 
 
 def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, window="hann", waterfall: bool = False,
                       vmin: float = -120.0, vmax: float = 0.0, maxhold: bool = True, hist_r: Optional[float] = None,
                       hist_bins: int = 256, max_samples: Optional[int] = None, max_chunk_samples: int = 1 << 26,
-                      device: int = 0) -> RecordingSpectra:
+                      device: int = 0, persistence: bool = False) -> RecordingSpectra:
     """The offline path of process_sigmf_data.py on the GPU, for the whole file: Welch PSD with
     ``plt.psd(data, NFFT, Fs, Fc)`` semantics (Hann, ``noverlap = nfft - hop``, default no overlap), plus
     optional max-hold, uint8 waterfall rows and the I/Q density histogram.  ``max_samples`` restores
-    the reference's truncation (10 000 there) when wanted."""
+    the reference's truncation (10 000 there) when wanted.  ``persistence``: the persistence spectrum of the whole
+    capture (frames per waterfall level of ``[vmin, vmax]`` and bin, uint32 [256, N]), accumulated on the GPU over the
+    file's chunks without bringing the F x N rows to the host (unless ``waterfall`` asks for them too)."""
     rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
     hop = int(hop or nfft)
     if max_samples is not None and max_samples < rec.n_samples:
@@ -243,22 +246,27 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
     fs, fc = rec.sample_rate, rec.center_freq
     freqs = sp.freq_axis(nfft, fs, fc)
     L = rec.n_samples
+    if persistence:
+        sp.nat.require_device()   # no CPU fallback, whatever the file length
     if L < nfft:   # mlab zero-pads a short input to one frame
         f, pxx = sp.welch_psd(rec.raw_slice() if rec.in_fmt == FMT_CI16 else rec.read_samples(), nfft, hop, window, fs, fc,
                               in_fmt=rec.in_fmt, in_scale=rec.in_scale, device=device)
-        return RecordingSpectra(f, pxx, 1, sample_rate=fs, center_freq=fc)
+        # no full frame in the capture: the persistence spectrum counts none (the PSD's single frame is zero-padded)
+        return RecordingSpectra(f, pxx, 1, sample_rate=fs, center_freq=fc,
+                                persistence=np.zeros((256, nfft), np.uint32) if persistence else None)
     pl = sp.get_plan(nfft, hop, window, rec.in_fmt, rec.in_scale, sp.DB_EPS_REFERENCE, device)
     F = (L - nfft) // hop + 1
     welch = np.zeros((1, nfft), np.float64)
     mh = np.zeros((1, nfft), np.float32) if maxhold else False
     rows = np.empty((F, nfft), np.uint8) if waterfall else None
     hist = np.zeros((hist_bins, hist_bins), np.uint32) if hist_r is not None else None
+    counts = np.zeros((1, 256, nfft), np.uint32) if persistence else False
     h2d = d2h = 0
     first = True
     for f0, nf, raw in rec.frame_chunks(nfft, hop, max_chunk_samples):
         x = raw if rec.in_fmt == FMT_CI16 else raw.view(np.complex64)
         r = pl.stft(x, welch=welch, maxhold=mh, wf_rows=(rows[f0:f0 + nf] if waterfall else False), vmin=vmin, vmax=vmax,
-                    accumulate=not first)
+                    persistence=counts, accumulate=not first)
         h2d += r.h2d_bytes
         d2h += r.d2h_bytes
         first = False
@@ -269,7 +277,8 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
             x = raw if rec.in_fmt == FMT_CI16 else raw.view(np.complex64)
             td.iq_hist2d(x, hist_r, hist_bins, in_fmt=rec.in_fmt, in_scale=rec.in_scale, out=hist, accumulate=True, device=device)
     pxx, _ = pl.welch_finalize(welch[0], F, fs, want_db=False)
-    return RecordingSpectra(freqs, pxx, F, mh[0] if maxhold else None, rows, hist, fs, fc, h2d, d2h)
+    return RecordingSpectra(freqs, pxx, F, mh[0] if maxhold else None, rows, hist, fs, fc, h2d, d2h,
+                            counts[0] if persistence else None)
 
 
 def psd(path_or_rec, NFFT: int = 1024, noverlap: int = 0, max_samples: Optional[int] = None, device: int = 0):

@@ -79,6 +79,7 @@ class StftResult:
     maxhold: Optional[object] = None     # float32 [S, N]
     h2d_bytes: int = 0
     d2h_bytes: int = 0
+    persistence: Optional[object] = None  # uint32  [S, 256, N] frames per waterfall level and bin
 
 
 class SpectralPlan:
@@ -163,10 +164,17 @@ class SpectralPlan:
     # -- execution
     def stft(self, x, *, n_streams: int = 1, db_rows=False, wf_rows=False, spectrum=False, welch=False,
              maxhold=False, vmin: float = -100.0, vmax: float = 0.0, accumulate: bool = False,
-             stream: int = 0, n_samples: Optional[int] = None, peer_outputs: int = 0, _time=None) -> StftResult:
+             stream: int = 0, n_samples: Optional[int] = None, peer_outputs: int = 0, persistence=False,
+             _time=None) -> StftResult:
         """Windowed STFT of ``x`` (1 stream, or ``n_streams`` equal-length streams laid out back to
         back).  Each output flag is False (not wanted), True (allocate) or a caller buffer to fill
-        (numpy for host input, DeviceArray / CUDA tensor for device input)."""
+        (numpy for host input, DeviceArray / CUDA tensor for device input).
+
+        ``persistence``: uint32 ``[n_streams, 256, nfft]``, for every bin the number of frames at each uint8 waterfall
+        level of ``[vmin, vmax]`` (a persistence / density spectrum; every column sums to the frame count).  It is an
+        accumulator like ``welch`` and ``maxhold``.  It does not need ``wf_rows``: without them the rows stay on the GPU."""
+        if persistence is not False and persistence is not None and _time is not None:
+            raise ValueError("persistence cannot be timed with _time (spx_stft_time runs spx_stft_exec)")
         if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
             x = self._host_input(x)
         in_ptr, mem = nat.as_ptr(x)
@@ -196,6 +204,7 @@ class SpectralPlan:
         o_sp = out(spectrum, (rows, N), np.complex64, "spectrum")
         o_we = out(welch, (n_streams, N), np.float64, "welch", accumulator=True)
         o_mh = out(maxhold, (n_streams, N), np.float32, "maxhold", accumulator=True)
+        o_pe = out(persistence, (n_streams, 256, N), np.uint32, "persistence", accumulator=True)
         a = nat.spx_stft_args()
         a.struct_size = C.sizeof(nat.spx_stft_args)
         a.mem = mem
@@ -217,10 +226,12 @@ class SpectralPlan:
             ms = (C.c_float * iters)()
             nat.check(nat.lib().spx_stft_time(self._h, C.byref(a), warmup, iters, 1 if flush else 0, ms))
             self.last_times_ms = [float(v) for v in ms]
+        elif o_pe is not None:
+            nat.check(nat.lib().spx_stft_exec_persistence(self._h, C.byref(a), nat.as_ptr(o_pe)[0]))
         else:
             nat.check(nat.lib().spx_stft_exec(self._h, C.byref(a)))
         return StftResult(int(a.n_frames_out), n_streams, o_db, o_wf, o_sp, o_we, o_mh,
-                          int(a.h2d_bytes_out), int(a.d2h_bytes_out))
+                          int(a.h2d_bytes_out), int(a.d2h_bytes_out), o_pe)
 
     def time_stft(self, x, *, warmup: int = 3, iters: int = 10, flush_l2: bool = False, **kw):
         """Device-resident timing of the exact launch ``stft`` would make: CUDA events on the launch

@@ -73,6 +73,26 @@ class WaterfallBlock:
                 "db_range": (self.vmin, self.vmax)}
 
 
+def persistence_payload(counts, n_frames: int, vmin: float, vmax: float, freqs_mhz=None) -> dict:
+    """Arguments of a ``go.Heatmap`` of a persistence spectrum (``SpectralPlan.stft(persistence=...)``, one stream's
+    uint32 [256, N] counts, or [1, 256, N]), in the style of ``WaterfallBlock.heatmap_payload``: ``z`` is the fraction of the
+    ``n_frames`` frames at each level and bin (float32 [256, N], rows = levels), ``y`` the lower dB edge of each level
+    (level q covers [vmin + q*D, vmin + (q+1)*D), D = (vmax - vmin)/256; level 0 also holds everything below vmin,
+    level 255 everything above).  Decay and log colour scaling are left to the caller."""
+    c = np.asarray(counts)
+    if c.ndim == 3:   # [S][256][N]: one stream only, so that no stream is dropped unseen (pass counts[s] for the others)
+        if c.shape[0] != 1:
+            raise ValueError(f"counts: {c.shape[0]} streams; pass one stream's [256, N] counts")
+        c = c[0]
+    if c.ndim != 2 or c.shape[0] != 256:
+        raise ValueError(f"counts: expected shape (256, N), got {c.shape}")
+    z = c.astype(np.float32) / np.float32(max(int(n_frames), 1))
+    y = vmin + np.arange(256, dtype=np.float64) * ((vmax - vmin) / 256.0)
+    lut = _spectral.viridis_lut()
+    scale = [[i / 255.0, "rgb(%d,%d,%d)" % tuple(lut[i])] for i in range(0, 256, 15)]
+    return {"z": z, "x": freqs_mhz, "y": y, "zmin": 0.0, "zmax": 1.0, "colorscale": scale, "db_range": (vmin, vmax)}
+
+
 def constellation_density(samples, r: Optional[float] = None, bins: int = 256, in_fmt: int = _spectral.FMT_CF32,
                           in_scale: float = 1.0, device: int = 0) -> dict:
     """Exact I/Q density over ALL samples (kernel K4) instead of a random 2000-point scatter (:199-214).

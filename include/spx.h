@@ -224,6 +224,44 @@ SPX_API int spx_stft_exec(spx_plan* plan, spx_stft_args* args);
  * copies back only the counts and the accumulators (d2h_bytes_out). */
 SPX_API int spx_stft_exec_persistence(spx_plan* plan, spx_stft_args* args, uint32_t* counts);
 
+/* Pooled spectrogram (display detectors).  Row g of stream s pools frames [gK, min((g+1)K, F_total)) and column c pools
+ * bins [cB, (c+1)B) (fftshift order) of the power P = |X|^2 that the dB rows encode:
+ *   SPX_POOL_MEAN: acc[s][g][c] = sum of P over the cell (NaN propagates, as in welch_acc)
+ *   SPX_POOL_MAX:  acc[s][g][c] = max of the dB value over the cell (NaN skipped; -inf when nothing or only NaN)
+ * The power is recovered from the float32 dB rows as (10^(d/20) - db_eps)^2, clipped at 0. */
+#define SPX_POOL_MEAN 0
+#define SPX_POOL_MAX 1
+
+typedef struct {
+    uint32_t struct_size;     /* sizeof(spx_pool_args) */
+    int32_t mode;             /* SPX_POOL_* */
+    int64_t frames_per_row;   /* K >= 1 */
+    int32_t bins_per_col;     /* B >= 1, nfft % B == 0 */
+    int32_t reserved;
+    int64_t first_frame;      /* global index of this call's frame 0 (>= 0): calls on consecutive pieces of a capture
+                                 pool into one accumulator, a row may span calls */
+    int64_t n_rows;           /* G the accumulator holds; every frame of the call must fall in a row < G */
+    double* acc;              /* [n_streams][G][nfft / B], args->mem space; args->accumulate applies (0: set to the mode's
+                                 identity, 0 or -inf, before adding) */
+} spx_pool_args;
+
+/* spx_stft_exec plus the pooled accumulator of the call's frames.  args->db_rows may be NULL: the dB rows then go in
+ * batches through a plan-owned float row buffer of SPX_POOL_ROWS_BYTES (plan-creation environment variable, default
+ * 256 MiB) and never leave the GPU; a host-memory call then copies back only the accumulator, the other accumulators and
+ * the rows that were asked for (d2h_bytes_out).  SPX_E_INVALID for K < 1, B < 1, nfft % B != 0, an unknown mode,
+ * first_frame < 0 or a frame in a row >= n_rows; SPX_E_UNSUPPORTED for peer_outputs.  N = 65536 runs the two-kernel
+ * four-step path (float rows). */
+SPX_API int spx_stft_exec_pooled(spx_plan* plan, spx_stft_args* args, spx_pool_args* pool);
+
+/* Pooled dB (db_out, float32) and/or levels (wf_out, uint8; needs vmax > vmin) of an accumulator, both
+ * [n_streams][n_rows][nfft / B] in `mem` space:
+ *   mean: 20 log10(sqrt(acc / (n_g B)) + db_eps), n_g = the frames of row g;   max: acc
+ *   level = clip(floor((dB - vmin) * 256 / (vmax - vmin)), 0, 255), NaN -> 0, computed in float64 from the float32 dB.
+ * n_rows must be ceil(n_frames_total / frames_per_row). */
+SPX_API int spx_pool_finalize(spx_plan* plan, int32_t mem, int32_t mode, const double* acc, int32_t n_streams,
+                              int64_t n_rows, int64_t n_frames_total, int64_t frames_per_row, int32_t bins_per_col,
+                              float* db_out, uint8_t* wf_out, float vmin, float vmax, void* stream);
+
 /* Measurement helper: runs spx_stft_exec (SPX_MEM_DEVICE buffers only) warmup+iters times on the
  * launch stream, each bracketed by CUDA events; optionally READS a 256 MiB buffer before every
  * iteration to flush the 126 MB L2 without leaving dirty lines behind.  ms_each[iters] receives the device time of

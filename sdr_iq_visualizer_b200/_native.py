@@ -53,6 +53,15 @@ class spx_stft_args(C.Structure):
                 ("d2h_bytes_out", C.c_int64), ("peer_outputs", C.c_int32), ("reserved", C.c_int32)]
 
 
+class spx_pool_args(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("mode", C.c_int32), ("frames_per_row", C.c_int64),
+                ("bins_per_col", C.c_int32), ("reserved", C.c_int32), ("first_frame", C.c_int64), ("n_rows", C.c_int64),
+                ("acc", C.c_void_p)]
+
+
+POOL_MEAN, POOL_MAX = 0, 1
+
+
 class spx_features(C.Structure):
     _fields_ = [("n", C.c_int32), ("argmax", C.c_int32), ("peak_db", C.c_double), ("noise_floor_db", C.c_double),
                 ("snr_db", C.c_double), ("adaptive_thr", C.c_double), ("p20_lo", C.c_double), ("p20_hi", C.c_double),
@@ -112,6 +121,9 @@ _SIGNATURES = {
     "spx_plan_sync": (C.c_int, [C.c_void_p]),
     "spx_stft_exec": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args)]),
     "spx_stft_exec_persistence": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.c_void_p]),
+    "spx_stft_exec_pooled": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.POINTER(spx_pool_args)]),
+    "spx_pool_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_int64,
+                                    C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p]),
     "spx_stft_time": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.c_int32, C.c_int32, C.c_int32,
                                 C.POINTER(C.c_float)]),
     "spx_welch_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,

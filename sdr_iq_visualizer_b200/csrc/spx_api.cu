@@ -18,6 +18,7 @@
 #include <nvtx3/nvToolsExt.h>
 
 #include "spx_plan.h"
+#include "spx_pool_device.cuh"
 #include "spx_stft_kernel.cuh"
 #include "spx_tables.h"
 
@@ -130,45 +131,76 @@ int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long l
 
 static size_t in_elt(const spx_plan* pl) { return pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8; }
 
-// ------------------------------------------------------------------ persistence spectrum without caller rows
-// The STFT of frames [0, F) of every stream goes in batches through the plan's row buffer (SPX_PERSIST_ROWS_BYTES), each
-// batch followed by its histogram on the same stream, so the uint8 rows never leave the GPU.  The buffer holds
-// max(1, bytes / (S N)) frames of the S streams of a batch: it exceeds SPX_PERSIST_ROWS_BYTES only when a single frame
-// of every stream does (S N > bytes).  A batch starts f0 * hop samples into every stream: f0 * hop * elt keeps the input alignment (128 bytes for
-// K1v2, 16 bytes for K1's staged loads and K2v2) and K2v2's hop % 256 of the unbatched call, and a batch covers all
-// streams with the call's stride, so each batch runs the kernel family the unbatched call would.  Exception: float rows
-// (db_rows / spec_rows) of several streams must land at rows s * F + f, so those batches run one stream at a time.
-static long long persist_batch_frames(const spx_plan* pl, long long Sb, long long F) {
-    long long fb = (long long)(pl->persist_rows_bytes / ((size_t)Sb * pl->cfg.nfft));
+// ------------------------------------------------------------------ row consumers without caller rows
+// The persistence spectrum consumes uint8 rows and the pooled spectrogram float dB rows.  Without caller rows of that kind
+// the STFT of frames [0, F) of every stream goes in batches through the plan's row buffer (SPX_PERSIST_ROWS_BYTES of
+// uint8 rows, or SPX_POOL_ROWS_BYTES of float rows), each batch followed by its consumer kernel on the same stream, so
+// those rows never leave the GPU.  The buffer holds max(1, bytes / (S row)) frames of the S streams of a batch: it
+// exceeds its size only when a single frame of every stream does.  A batch starts f0 * hop samples into every stream:
+// f0 * hop * elt keeps the input alignment (128 bytes for K1v2, 16 bytes for K1's staged loads and K2v2) and K2v2's
+// hop % 256 of the unbatched call, and a batch covers all streams with the call's stride, so each batch runs the kernel
+// family the unbatched call would.  Exception: caller rows of several streams must land at rows s * F + f, so those
+// batches run one stream at a time.
+enum RowKind { ROWS_U8, ROWS_DB };
+
+static long long row_batch_frames(const spx_plan* pl, RowKind kind, long long Sb, long long F) {
+    const size_t row = (size_t)pl->cfg.nfft * (kind == ROWS_DB ? sizeof(float) : 1);
+    long long fb = (long long)((kind == ROWS_DB ? pl->pool_rows_bytes : pl->persist_rows_bytes) / ((size_t)Sb * row));
     if (fb < 1) fb = 1;
     return fb < F ? fb : F;
 }
 
-static int persist_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, float* db_rows,
-                           float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, uint32_t* counts,
-                           cudaStream_t st) {
+// consume(rows, s, Sb, f0, nf): rows [Sb][nf][N] of streams s .. s + Sb - 1, frames f0 .. f0 + nf - 1, in the buffer
+template <class Consume>
+static int row_batches(spx_plan* pl, RowKind kind, const char* in, long long S, long long stride, long long F,
+                       float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
+                       float vmin, float vmax, cudaStream_t st, Consume consume) {
     const int N = pl->cfg.nfft, hop = pl->cfg.hop;
     const size_t elt = in_elt(pl);
-    const long long Sb = S > 1 && (db_rows || spec_rows) ? 1 : S;
-    const long long fb = persist_batch_frames(pl, Sb, F);
-    SPX_TRY(pl->st_persist.reserve((size_t)(Sb * fb) * N));   // a no-op when the host pipeline reserved it up front
-    unsigned char* rows = (unsigned char*)pl->st_persist.ptr;
+    const long long Sb = S > 1 && (db_rows || wf_rows || spec_rows) ? 1 : S;
+    const long long fb = row_batch_frames(pl, kind, Sb, F);
+    const size_t row = (size_t)N * (kind == ROWS_DB ? sizeof(float) : 1);
+    SPX_TRY(pl->st_rows.reserve((size_t)(Sb * fb) * row));   // a no-op when the host pipeline reserved it up front
+    void* rows = pl->st_rows.ptr;
     for (long long s = 0; s < S; s += Sb) {
         for (long long f0 = 0; f0 < F; f0 += fb) {
             const long long nf = F - f0 < fb ? F - f0 : fb;
             const size_t r0 = (size_t)(s * F + f0) * N;
             SPX_TRY(stft_launch_device(pl, in + (size_t)(s * stride + f0 * hop) * elt, Sb, stride, nf,
-                                       db_rows ? db_rows + r0 : nullptr, rows, spec_rows ? spec_rows + r0 : nullptr,
-                                       welch_acc ? welch_acc + s * N : nullptr, maxhold ? maxhold + s * N : nullptr, vmin,
-                                       vmax, st));
-            SPX_TRY(persist_launch(pl, rows, Sb, nf, counts + (size_t)s * 256 * N, st));
+                                       kind == ROWS_DB ? (float*)rows : (db_rows ? db_rows + r0 : nullptr),
+                                       kind == ROWS_U8 ? (unsigned char*)rows : (wf_rows ? wf_rows + r0 : nullptr),
+                                       spec_rows ? spec_rows + r0 : nullptr, welch_acc ? welch_acc + s * N : nullptr,
+                                       maxhold ? maxhold + s * N : nullptr, vmin, vmax, st));
+            SPX_TRY(consume(rows, s, Sb, f0, nf));
         }
     }
     return SPX_OK;
 }
 
+static int persist_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, float* db_rows,
+                           float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, uint32_t* counts,
+                           cudaStream_t st) {
+    const int N = pl->cfg.nfft;
+    return row_batches(pl, ROWS_U8, in, S, stride, F, db_rows, nullptr, spec_rows, welch_acc, maxhold, vmin, vmax, st,
+                       [&](void* rows, long long s, long long Sb, long long, long long nf) {
+                           return persist_launch(pl, (const uint8_t*)rows, Sb, nf, counts + (size_t)s * 256 * N, st);
+                       });
+}
+
+// acc: the accumulator of stream 0 of these streams; frame0: the global index of frame 0 of `in`
+static int pool_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, unsigned char* wf_rows,
+                        float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, const PoolCall& pc,
+                        double* acc, long long frame0, cudaStream_t st) {
+    const long long cells = pc.n_rows * (pl->cfg.nfft / pc.bins_per_col);
+    return row_batches(pl, ROWS_DB, in, S, stride, F, nullptr, wf_rows, spec_rows, welch_acc, maxhold, vmin, vmax, st,
+                       [&](void* rows, long long s, long long Sb, long long f0, long long nf) {
+                           return pool_launch(pl, (const float*)rows, Sb, nf, nf, frame0 + f0, pc, acc + (size_t)s * cells,
+                                              st);
+                       });
+}
+
 // ------------------------------------------------------------------ host-memory pipeline
-static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t* counts) {
+static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t* counts, const PoolCall* pc) {
     const int N = pl->cfg.nfft, hop = pl->cfg.hop;
     const size_t elt = in_elt(pl);
     const long long S = a->n_streams, L = a->n_samples;
@@ -188,10 +220,10 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
     float* d_max = a->maxhold ? (float*)pl->st_max.ptr : nullptr;
     long long h2d = 0, d2h = 0;
 
-    // plan-owned scratch (four-step / K2v2 / Bluestein buffers, the persistence row buffer): a device-resident call on a
-    // caller stream may still be using it, so the kernels queued here on s_compute wait for that call first, as the
-    // device path does
-    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || (counts && !a->wf_rows);
+    // plan-owned scratch (four-step / K2v2 / Bluestein buffers, the row buffer): a device-resident call on a caller stream
+    // may still be using it, so the kernels queued here on s_compute wait for that call first, as the device path does
+    const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
+    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || own_u8 || own_db;
     if (owns_scratch) {
         if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
         if (pl->scratch_stream_valid && pl->scratch_stream != pl->s_compute) SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, pl->ev_scratch, 0));
@@ -227,16 +259,31 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
             SPX_CUDA(cudaMemsetAsync(d_counts, 0, count_bytes, pl->s_compute));
         }
     }
+    // pooled accumulator: the same rule, the mode's identity when not accumulating
+    const long long pool_cells = pc ? pc->n_rows * (N / pc->bins_per_col) : 0;
+    const size_t pool_bytes = (size_t)(S * pool_cells) * sizeof(double);
+    double* d_pool = nullptr;
+    if (pc) {
+        SPX_TRY(pl->st_pool.reserve(pool_bytes));
+        d_pool = (double*)pl->st_pool.ptr;
+        if (a->accumulate) {
+            SPX_CUDA(cudaMemcpyAsync(d_pool, pc->acc, pool_bytes, cudaMemcpyHostToDevice, pl->s_compute));
+            h2d += (long long)pool_bytes;
+        } else {
+            SPX_TRY(pool_fill_launch(d_pool, S * pool_cells, pc->mode, pl->s_compute));
+        }
+    }
 
     // piece size: big enough to amortise launches, small enough to overlap (about 8-16 MiB)
     long long piece = (long long)(pl->piece_bytes / elt);
     if (piece < (long long)N * 4) piece = (long long)N * 4;
-    // counts without rows: one row buffer for every piece, sized for the largest (a piece spans at most `piece` samples,
-    // so at most piece / hop + 1 frames), reserved here -- growing it between pieces would free device memory, which
-    // synchronises the device in the middle of the pipeline
-    if (counts && !a->wf_rows) {
+    // counts / pooling without rows: one row buffer for every piece, sized for the largest (a piece spans at most `piece`
+    // samples, so at most piece / hop + 1 frames), reserved here -- growing it between pieces would free device memory,
+    // which synchronises the device in the middle of the pipeline
+    if (own_u8 || own_db) {
         const long long most = piece / hop + 2 < F ? piece / hop + 2 : F;
-        SPX_TRY(pl->st_persist.reserve((size_t)persist_batch_frames(pl, 1, most) * N));
+        const RowKind kind = own_db ? ROWS_DB : ROWS_U8;
+        SPX_TRY(pl->st_rows.reserve((size_t)row_batch_frames(pl, kind, 1, most) * N * (own_db ? sizeof(float) : 1)));
     }
     struct Piece { long long s, f_lo, f_hi; };
     std::vector<Piece> pieces;
@@ -273,17 +320,25 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
             SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, e_in, 0));
             const size_t r0 = (size_t)(s * F + f_lo);
             NvtxRange r_k("spx STFT kernel piece");
-            if (d_counts && !d_wf) {   // counts without rows: the piece's rows go through the plan's row buffer
+            if (own_u8) {   // counts without rows: the piece's rows go through the plan's row buffer
                 SPX_TRY(persist_batches(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, d_db ? d_db + r0 * N : nullptr,
                                         d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
                                         d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, d_counts + (size_t)s * 256 * N,
                                         pl->s_compute));
+            } else if (own_db) {   // pooling without dB rows: likewise, float rows
+                SPX_TRY(pool_batches(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, d_wf ? d_wf + r0 * N : nullptr,
+                                     d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
+                                     d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, *pc, d_pool + (size_t)(s * pool_cells),
+                                     pc->first_frame + f_lo, pl->s_compute));
             } else {
                 SPX_TRY(stft_launch_device(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo,
                                            d_db ? d_db + r0 * N : nullptr, d_wf ? d_wf + r0 * N : nullptr,
                                            d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
                                            d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, pl->s_compute));
                 if (d_counts) SPX_TRY(persist_launch(pl, d_wf + r0 * N, 1, f_hi - f_lo, d_counts + (size_t)s * 256 * N, pl->s_compute));
+                if (d_pool)
+                    SPX_TRY(pool_launch(pl, d_db + r0 * N, 1, f_hi - f_lo, f_hi - f_lo, pc->first_frame + f_lo, *pc,
+                                        d_pool + (size_t)(s * pool_cells), pl->s_compute));
             }
             SPX_CUDA(cudaEventRecord(e_k, pl->s_compute));
             pieces.push_back({s, f_lo, f_hi});
@@ -323,6 +378,10 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
     if (d_counts) {
         SPX_CUDA(cudaMemcpyAsync(counts, d_counts, count_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
         d2h += (long long)count_bytes;
+    }
+    if (d_pool) {
+        SPX_CUDA(cudaMemcpyAsync(pc->acc, d_pool, pool_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
+        d2h += (long long)pool_bytes;
     }
     if (owns_scratch) {
         SPX_CUDA(cudaEventRecord(pl->ev_scratch, pl->s_compute));
@@ -624,6 +683,11 @@ int spx_plan_create(spx_plan** out, const spx_plan_config* cfg) {
         long long v = atoll(e);
         if (v > 0) pl->persist_rows_bytes = (size_t)v > (size_t)cfg->nfft ? (size_t)v : (size_t)cfg->nfft;
     }
+    if (const char* e = getenv("SPX_POOL_ROWS_BYTES")) {   // at least one row
+        long long v = atoll(e);
+        const size_t row = (size_t)cfg->nfft * sizeof(float);
+        if (v > 0) pl->pool_rows_bytes = (size_t)v > row ? (size_t)v : row;
+    }
     int rc = SPX_OK;
     do {
         cudaError_t e;
@@ -683,7 +747,7 @@ int spx_plan_destroy(spx_plan* pl) {
     pl->st_big.release();
     pl->st_in.release(); pl->st_db.release(); pl->st_wf.release(); pl->st_spec.release();
     pl->st_welch.release(); pl->st_max.release(); pl->st_misc.release(); pl->st_flush.release();
-    pl->st_counts.release(); pl->st_persist.release();
+    pl->st_counts.release(); pl->st_pool.release(); pl->st_rows.release();
     delete pl;
     return SPX_OK;
 }
@@ -791,12 +855,14 @@ int spx_plan_window_sums(spx_plan* pl, double* sum_w2, double* sum_w) {
     return SPX_OK;
 }
 
-// spx_stft_exec, plus the persistence counts [S][256][N] of the call's uint8 levels when `counts` is not NULL
-static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
+// spx_stft_exec, plus the persistence counts [S][256][N] of the call's uint8 levels when `counts` is not NULL, or the
+// pooled accumulator when `pc` is not NULL (never both)
+static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts, const PoolCall* pc) {
     if (!pl || !a) return spx_set_error(SPX_E_INVALID, "NULL argument");
     if (a->struct_size != sizeof(spx_stft_args))
         return spx_set_error(SPX_E_INVALID, "spx_stft_args.struct_size %u != %zu", a->struct_size, sizeof(spx_stft_args));
     if (counts && a->peer_outputs) return spx_set_error(SPX_E_UNSUPPORTED, "persistence with peer_outputs is not supported");
+    if (pc && a->peer_outputs) return spx_set_error(SPX_E_UNSUPPORTED, "pooling with peer_outputs is not supported");
     if (a->n_streams < 1) return spx_set_error(SPX_E_INVALID, "n_streams must be >= 1");
     if (a->n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
     if (a->mem != SPX_MEM_HOST && a->mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", a->mem);
@@ -805,6 +871,9 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
     if (a->n_streams > 1 && a->stream_stride < a->n_samples && a->mem == SPX_MEM_HOST)
         return spx_set_error(SPX_E_INVALID, "stream_stride < n_samples");
     const long long F = spx_frame_count(a->n_samples, pl->cfg.nfft, pl->cfg.hop);
+    if (pc && F > 0 && pool_row_of(pc->first_frame + F - 1, pc->frames_per_row) >= pc->n_rows)
+        return spx_set_error(SPX_E_INVALID, "frames %lld .. %lld fall outside the %lld pooled rows of %lld frames",
+                             pc->first_frame, pc->first_frame + F - 1, pc->n_rows, pc->frames_per_row);
     a->n_frames_out = F;
     a->h2d_bytes_out = 0;
     a->d2h_bytes_out = 0;
@@ -813,13 +882,15 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
     const int N = pl->cfg.nfft;
     const long long S = a->n_streams;
     const size_t count_bytes = (size_t)S * 256 * N * sizeof(uint32_t);
+    const long long pool_cells = pc ? pc->n_rows * (N / pc->bins_per_col) : 0;
     if (a->in == nullptr && F > 0) return spx_set_error(SPX_E_INVALID, "in is NULL");
     if (a->mem == SPX_MEM_DEVICE) {
         cudaStream_t st = a->stream ? (cudaStream_t)a->stream : pl->s_compute;
-        // Plan-owned scratch (four-step / K2v2 scratch and counters, Bluestein buffers, peer staging, the persistence row
-        // buffer) is shared by every call on this plan: a call on another stream than the previous one waits for that
-        // one's kernels first.
-        const bool own_rows = counts && !a->wf_rows;
+        // Plan-owned scratch (four-step / K2v2 scratch and counters, Bluestein buffers, peer staging, the row buffer) is
+        // shared by every call on this plan: a call on another stream than the previous one waits for that one's kernels
+        // first.
+        const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
+        const bool own_rows = own_u8 || own_db;
         const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || a->peer_outputs || own_rows;
         if (owns_scratch) {
             if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
@@ -829,15 +900,20 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
             if (a->welch_acc) SPX_CUDA(cudaMemsetAsync(a->welch_acc, 0, (size_t)S * N * sizeof(double), st));
             if (a->maxhold) SPX_CUDA(cudaMemsetAsync(a->maxhold, 0, (size_t)S * N * sizeof(float), st));
             if (counts) SPX_CUDA(cudaMemsetAsync(counts, 0, count_bytes, st));
+            if (pc) SPX_TRY(pool_fill_launch(pc->acc, S * pool_cells, pc->mode, st));
         }
         int rc;
-        if (own_rows) rc = persist_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->db_rows,
+        if (own_db) rc = pool_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->wf_rows,
+                                      reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold, a->vmin, a->vmax, *pc,
+                                      pc->acc, pc->first_frame, st);
+        else if (own_u8) rc = persist_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->db_rows,
                                            reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold, a->vmin, a->vmax,
                                            counts, st);
         else if (a->peer_outputs && !a->db_rows && !a->spec_rows && F > 0) rc = stft_exec_device_peer(pl, a, F, st);
         else rc = stft_launch_device(pl, a->in, S, a->stream_stride, F, a->db_rows, a->wf_rows, reinterpret_cast<float2*>(a->spec_rows),
                                      a->welch_acc, a->maxhold, a->vmin, a->vmax, st, a->peer_outputs ? 1 : 0);
         if (rc == SPX_OK && counts && !own_rows) rc = persist_launch(pl, a->wf_rows, S, F, counts, st);
+        if (rc == SPX_OK && pc && !own_rows) rc = pool_launch(pl, a->db_rows, S, F, F, pc->first_frame, *pc, pc->acc, st);
         if (rc == SPX_OK && owns_scratch) {
             SPX_CUDA(cudaEventRecord(pl->ev_scratch, st));
             pl->scratch_stream = st;
@@ -850,17 +926,73 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
             if (a->welch_acc) memset(a->welch_acc, 0, (size_t)S * N * sizeof(double));
             if (a->maxhold) memset(a->maxhold, 0, (size_t)S * N * sizeof(float));
             if (counts) memset(counts, 0, count_bytes);
+            const double id = pc && pc->mode == SPX_POOL_MAX ? -INFINITY : 0.0;
+            for (long long i = 0; i < S * pool_cells; ++i) pc->acc[i] = id;
         }
         return SPX_OK;
     }
-    return stft_exec_host(pl, a, F, counts);
+    return stft_exec_host(pl, a, F, counts, pc);
 }
 
-int spx_stft_exec(spx_plan* pl, spx_stft_args* a) { return stft_exec(pl, a, nullptr); }
+int spx_stft_exec(spx_plan* pl, spx_stft_args* a) { return stft_exec(pl, a, nullptr, nullptr); }
 
 int spx_stft_exec_persistence(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
     if (!counts) return spx_set_error(SPX_E_INVALID, "counts is NULL");
-    return stft_exec(pl, a, counts);
+    return stft_exec(pl, a, counts, nullptr);
+}
+
+// K, B and the mode of a pooled call or its finalisation
+static int check_pool_shape(const spx_plan* pl, int mode, long long K, int B) {
+    if (mode != SPX_POOL_MEAN && mode != SPX_POOL_MAX) return spx_set_error(SPX_E_INVALID, "unknown pool mode %d", mode);
+    if (K < 1) return spx_set_error(SPX_E_INVALID, "frames_per_row %lld must be >= 1", K);
+    if (B < 1 || pl->cfg.nfft % B != 0)
+        return spx_set_error(SPX_E_INVALID, "bins_per_col %d must be >= 1 and divide nfft %d", B, pl->cfg.nfft);
+    return SPX_OK;
+}
+
+int spx_stft_exec_pooled(spx_plan* pl, spx_stft_args* a, spx_pool_args* p) {
+    if (!pl || !a || !p) return spx_set_error(SPX_E_INVALID, "NULL argument");
+    if (p->struct_size != sizeof(spx_pool_args))
+        return spx_set_error(SPX_E_INVALID, "spx_pool_args.struct_size %u != %zu", p->struct_size, sizeof(spx_pool_args));
+    SPX_TRY(check_pool_shape(pl, p->mode, p->frames_per_row, p->bins_per_col));
+    if (p->first_frame < 0 || p->n_rows < 0) return spx_set_error(SPX_E_INVALID, "first_frame and n_rows must be >= 0");
+    if (!p->acc) return spx_set_error(SPX_E_INVALID, "acc is NULL");
+    const PoolCall pc{p->mode, p->frames_per_row, p->bins_per_col, p->first_frame, p->n_rows, p->acc};
+    return stft_exec(pl, a, nullptr, &pc);
+}
+
+int spx_pool_finalize(spx_plan* pl, int32_t mem, int32_t mode, const double* acc, int32_t n_streams, int64_t n_rows,
+                      int64_t n_frames_total, int64_t frames_per_row, int32_t bins_per_col, float* db_out, uint8_t* wf_out,
+                      float vmin, float vmax, void* stream) {
+    if (!pl || !acc) return spx_set_error(SPX_E_INVALID, "NULL argument");
+    SPX_TRY(check_pool_shape(pl, mode, frames_per_row, bins_per_col));
+    if (mem != SPX_MEM_HOST && mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", mem);
+    if (n_streams < 1 || n_frames_total < 0) return spx_set_error(SPX_E_INVALID, "n_streams must be >= 1, n_frames_total >= 0");
+    if (n_rows != (n_frames_total + frames_per_row - 1) / frames_per_row)
+        return spx_set_error(SPX_E_INVALID, "n_rows %lld != ceil(%lld frames / %lld)", (long long)n_rows,
+                             (long long)n_frames_total, (long long)frames_per_row);
+    if (wf_out && !(vmax > vmin)) return spx_set_error(SPX_E_INVALID, "wf_out needs vmax > vmin");
+    std::lock_guard<std::mutex> g(pl->mu);
+    SPX_CUDA(cudaSetDevice(pl->cfg.device));
+    const size_t n = (size_t)n_streams * (size_t)n_rows * (size_t)(pl->cfg.nfft / bins_per_col);
+    if (mem == SPX_MEM_DEVICE) {
+        cudaStream_t st = stream ? (cudaStream_t)stream : pl->s_compute;
+        return pool_finalize_launch(pl, acc, n_streams, n_rows, n_frames_total, frames_per_row, bins_per_col, mode, vmin,
+                                    vmax, db_out, wf_out, st);
+    }
+    if (n == 0 || (!db_out && !wf_out)) return SPX_OK;
+    // host memory: [acc | dB | levels] staged in one buffer
+    SPX_TRY(pl->st_misc.reserve(n * (sizeof(double) + sizeof(float) + 1)));
+    double* d_acc = (double*)pl->st_misc.ptr;
+    float* d_db = (float*)(d_acc + n);
+    uint8_t* d_wf = (uint8_t*)(d_db + n);
+    SPX_CUDA(cudaMemcpyAsync(d_acc, acc, n * sizeof(double), cudaMemcpyHostToDevice, pl->s_compute));
+    SPX_TRY(pool_finalize_launch(pl, d_acc, n_streams, n_rows, n_frames_total, frames_per_row, bins_per_col, mode, vmin, vmax,
+                                 db_out ? d_db : nullptr, wf_out ? d_wf : nullptr, pl->s_compute));
+    if (db_out) SPX_CUDA(cudaMemcpyAsync(db_out, d_db, n * sizeof(float), cudaMemcpyDeviceToHost, pl->s_compute));
+    if (wf_out) SPX_CUDA(cudaMemcpyAsync(wf_out, d_wf, n, cudaMemcpyDeviceToHost, pl->s_compute));
+    SPX_CUDA(cudaStreamSynchronize(pl->s_compute));
+    return SPX_OK;
 }
 
 int spx_stft_time(spx_plan* pl, spx_stft_args* a, int32_t warmup, int32_t iters, int32_t flush_l2, float* ms_each) {

@@ -34,11 +34,12 @@ struct spx_plan {
     size_t piece_bytes = 16u << 20;  // H2D piece size of the host pipeline
     size_t peer_piece_bytes = 48u << 20;  // uint8 rows per piece of the peer-output pipeline (two staging buffers)
     size_t persist_rows_bytes = 64u << 20;  // uint8 row buffer of a device-resident persistence call without caller rows
+    size_t pool_rows_bytes = 256u << 20;    // float dB row buffer of a pooled call without caller dB rows (measured, DESIGN.md K8)
     // staging for SPX_MEM_HOST execution (grow-only)
     spx::DevBuf st_in, st_db, st_wf, st_spec, st_welch, st_max, st_misc, st_flush;
-    // persistence spectrum: counts staging of the host path, and the plan-owned row buffer (device path without caller
-    // rows; host path without caller rows, one piece)
-    spx::DevBuf st_counts, st_persist;
+    // persistence spectrum / pooled spectrogram: counts and accumulator staging of the host path, and the plan-owned row
+    // buffer (uint8 levels or float dB rows; device path without caller rows; host path without caller rows, one piece)
+    spx::DevBuf st_counts, st_pool, st_rows;
     // large-N (four-step) path, nfft >= 16384
     int big_n1 = 0, big_n2 = 0;
     float2* d_big_tw = nullptr;  // one allocation holding the four tables below
@@ -77,6 +78,20 @@ int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long
                        float* maxhold, float vmin, float vmax, cudaStream_t st, int sys_atomics);
 int persist_launch(const spx_plan* pl, const uint8_t* rows, long long n_streams, long long frames, uint32_t* counts,
                    cudaStream_t st);
+// a pooled call (spx_pool_args, checked); acc is [S][n_rows][nfft / bins_per_col] in the call's memory space
+struct PoolCall {
+    int mode;
+    long long frames_per_row;
+    int bins_per_col;
+    long long first_frame, n_rows;
+    double* acc;
+};
+int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long long rows_per_stream, long long frames,
+                long long frame0, const PoolCall& pc, double* acc, cudaStream_t st);
+int pool_fill_launch(double* acc, long long n, int mode, cudaStream_t st);
+int pool_finalize_launch(const spx_plan* pl, const double* acc, long long n_streams, long long G, long long F_total,
+                         long long K, int B, int mode, float vmin, float vmax, float* db_out, uint8_t* wf_out,
+                         cudaStream_t st);
 int welch_finalize_launch(const double* acc, int n, double inv_norm, double* pxx, double* pxx_db, cudaStream_t st);
 int bluestein_plan_init(spx_plan* pl);
 int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,

@@ -227,18 +227,38 @@ class RecordingSpectra:
     h2d_bytes: int = 0
     d2h_bytes: int = 0
     persistence: Optional[np.ndarray] = None  # uint32 [256, N] frames per waterfall level and bin
+    overview_db: Optional[np.ndarray] = None  # float32 [G, N/B] pooled spectrogram (dB)
+    overview_wf: Optional[np.ndarray] = None  # uint8 [G, N/B] its levels of [vmin, vmax]
+    overview_frames_per_row: int = 0          # K
+    overview_bins_per_col: int = 0            # B
+
+
+def overview_pooling(n_frames: int, nfft: int, rows: int, cols: int) -> tuple:
+    """(K, B) of an overview of about ``rows`` x ``cols`` pixels: K = ceil(F / rows) frames per row, B = the largest
+    divisor of nfft that is <= nfft / cols bins per column (1 when cols > nfft)."""
+    rows, cols, nfft = int(rows), int(cols), int(nfft)
+    if rows < 1 or cols < 1:
+        raise ValueError(f"overview: rows and cols must be >= 1, got {(rows, cols)}")
+    K = max(1, -(-int(n_frames) // rows))
+    top = max(1, nfft // cols)
+    B = max(d for d in range(1, top + 1) if nfft % d == 0)
+    return K, B
 
 
 def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, window="hann", waterfall: bool = False,
                       vmin: float = -120.0, vmax: float = 0.0, maxhold: bool = True, hist_r: Optional[float] = None,
                       hist_bins: int = 256, max_samples: Optional[int] = None, max_chunk_samples: int = 1 << 26,
-                      device: int = 0, persistence: bool = False) -> RecordingSpectra:
+                      device: int = 0, persistence: bool = False, overview: Optional[tuple] = None,
+                      overview_mode: str = "mean") -> RecordingSpectra:
     """The offline path of process_sigmf_data.py on the GPU, for the whole file: Welch PSD with
     ``plt.psd(data, NFFT, Fs, Fc)`` semantics (Hann, ``noverlap = nfft - hop``, default no overlap), plus
     optional max-hold, uint8 waterfall rows and the I/Q density histogram.  ``max_samples`` restores
     the reference's truncation (10 000 there) when wanted.  ``persistence``: the persistence spectrum of the whole
     capture (frames per waterfall level of ``[vmin, vmax]`` and bin, uint32 [256, N]), accumulated on the GPU over the
-    file's chunks without bringing the F x N rows to the host (unless ``waterfall`` asks for them too)."""
+    file's chunks without bringing the F x N rows to the host (unless ``waterfall`` asks for them too).
+    ``overview=(rows, cols)``: a pooled spectrogram of about that many pixels (``overview_pooling`` picks K and B;
+    ``overview_mode`` "mean" or "max" detector), accumulated on the GPU over the file's chunks in the same way; its dB
+    and levels of ``[vmin, vmax]`` are ``overview_db`` / ``overview_wf``."""
     rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
     hop = int(hop or nfft)
     if max_samples is not None and max_samples < rec.n_samples:
@@ -246,14 +266,23 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
     fs, fc = rec.sample_rate, rec.center_freq
     freqs = sp.freq_axis(nfft, fs, fc)
     L = rec.n_samples
-    if persistence:
+    if overview is not None:
+        sp.pool_mode(overview_mode)
+        o_rows, o_cols = overview
+    if persistence or overview is not None:
         sp.nat.require_device()   # no CPU fallback, whatever the file length
     if L < nfft:   # mlab zero-pads a short input to one frame
         f, pxx = sp.welch_psd(rec.raw_slice() if rec.in_fmt == FMT_CI16 else rec.read_samples(), nfft, hop, window, fs, fc,
                               in_fmt=rec.in_fmt, in_scale=rec.in_scale, device=device)
         # no full frame in the capture: the persistence spectrum counts none (the PSD's single frame is zero-padded)
-        return RecordingSpectra(f, pxx, 1, sample_rate=fs, center_freq=fc,
-                                persistence=np.zeros((256, nfft), np.uint32) if persistence else None)
+        out = RecordingSpectra(f, pxx, 1, sample_rate=fs, center_freq=fc,
+                               persistence=np.zeros((256, nfft), np.uint32) if persistence else None)
+        if overview is not None:   # no full frame: an overview of no rows
+            K, B = overview_pooling(0, nfft, o_rows, o_cols)
+            out.overview_db = np.zeros((0, nfft // B), np.float32)
+            out.overview_wf = np.zeros((0, nfft // B), np.uint8)
+            out.overview_frames_per_row, out.overview_bins_per_col = K, B
+        return out
     pl = sp.get_plan(nfft, hop, window, rec.in_fmt, rec.in_scale, sp.DB_EPS_REFERENCE, device)
     F = (L - nfft) // hop + 1
     welch = np.zeros((1, nfft), np.float64)
@@ -261,14 +290,25 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
     rows = np.empty((F, nfft), np.uint8) if waterfall else None
     hist = np.zeros((hist_bins, hist_bins), np.uint32) if hist_r is not None else None
     counts = np.zeros((1, 256, nfft), np.uint32) if persistence else False
+    if overview is not None:
+        K, B = overview_pooling(F, nfft, o_rows, o_cols)
+        pool = (K, B, overview_mode)
+        acc = np.empty((1, -(-F // K), nfft // B), np.float64)
     h2d = d2h = 0
     first = True
     for f0, nf, raw in rec.frame_chunks(nfft, hop, max_chunk_samples):
         x = raw if rec.in_fmt == FMT_CI16 else raw.view(np.complex64)
+        # pooling and persistence cannot share a call: with both, the overview takes a call of its own
+        both = persistence and overview is not None
         r = pl.stft(x, welch=welch, maxhold=mh, wf_rows=(rows[f0:f0 + nf] if waterfall else False), vmin=vmin, vmax=vmax,
-                    persistence=counts, accumulate=not first)
+                    persistence=counts, accumulate=not first,
+                    **(dict(pool=pool, pool_acc=acc, pool_first_frame=f0) if overview is not None and not both else {}))
         h2d += r.h2d_bytes
         d2h += r.d2h_bytes
+        if both:
+            r = pl.stft(x, pool=pool, pool_acc=acc, pool_first_frame=f0, accumulate=not first)
+            h2d += r.h2d_bytes
+            d2h += r.d2h_bytes
         first = False
     if hist is not None:   # every sample once (no halo): the histogram is over the capture, not over frames
         step = max_chunk_samples
@@ -277,8 +317,13 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
             x = raw if rec.in_fmt == FMT_CI16 else raw.view(np.complex64)
             td.iq_hist2d(x, hist_r, hist_bins, in_fmt=rec.in_fmt, in_scale=rec.in_scale, out=hist, accumulate=True, device=device)
     pxx, _ = pl.welch_finalize(welch[0], F, fs, want_db=False)
-    return RecordingSpectra(freqs, pxx, F, mh[0] if maxhold else None, rows, hist, fs, fc, h2d, d2h,
-                            counts[0] if persistence else None)
+    out = RecordingSpectra(freqs, pxx, F, mh[0] if maxhold else None, rows, hist, fs, fc, h2d, d2h,
+                           counts[0] if persistence else None)
+    if overview is not None:
+        o_db, o_wf = pl.pool_finalize(acc, F, K, B, overview_mode, db=True, wf=True, vmin=vmin, vmax=vmax)
+        out.overview_db, out.overview_wf = o_db[0], o_wf[0]
+        out.overview_frames_per_row, out.overview_bins_per_col = K, B
+    return out
 
 
 def psd(path_or_rec, NFFT: int = 1024, noverlap: int = 0, max_samples: Optional[int] = None, device: int = 0):

@@ -49,6 +49,38 @@ def freq_axis(nfft: int, sample_rate: float, center_freq: float = 0.0) -> np.nda
     return np.fft.fftshift(np.fft.fftfreq(int(nfft), 1 / sample_rate)) + center_freq
 
 
+def pooled_freq_axis(nfft: int, bins_per_col: int, sample_rate: float, center_freq: float = 0.0) -> np.ndarray:
+    """Frequency of each column of a pooled spectrogram (``SpectralPlan.stft(pool=(K, B, mode))``): the mean of the
+    ``freq_axis`` frequencies of the B bins the column pools, float64 [nfft / B]."""
+    nfft, b = int(nfft), int(bins_per_col)
+    if b < 1 or nfft % b:
+        raise ValueError(f"bins_per_col {b} must be >= 1 and divide nfft {nfft}")
+    return freq_axis(nfft, sample_rate, center_freq).reshape(nfft // b, b).mean(axis=1)
+
+
+_POOL_MODES = {"mean": nat.POOL_MEAN, "max": nat.POOL_MAX}
+
+
+def pool_mode(mode) -> int:
+    """SPX_POOL_* of "mean" (average detector) or "max" (peak detector)."""
+    try:
+        return _POOL_MODES[mode]
+    except (KeyError, TypeError):
+        raise ValueError(f"unknown pool mode {mode!r} (expected 'mean' or 'max')") from None
+
+
+def _pool_shape(nfft: int, pool) -> tuple:
+    """(K, B, mode id) of a ``pool=(K, B, mode)`` argument, checked."""
+    try:
+        K, B, mode = pool
+    except (TypeError, ValueError):
+        raise ValueError(f"pool must be (frames_per_row, bins_per_col, 'mean' | 'max'), got {pool!r}") from None
+    K, B = int(K), int(B)
+    if K < 1 or B < 1 or nfft % B:
+        raise ValueError(f"pool: frames_per_row {K} must be >= 1, bins_per_col {B} >= 1 and a divisor of nfft {nfft}")
+    return K, B, pool_mode(mode)
+
+
 def _buffer_dtype_count(buf):
     """(numpy dtype, element count) of a numpy array, DeviceArray / DeviceView or torch tensor."""
     if isinstance(buf, np.ndarray):
@@ -80,6 +112,7 @@ class StftResult:
     h2d_bytes: int = 0
     d2h_bytes: int = 0
     persistence: Optional[object] = None  # uint32  [S, 256, N] frames per waterfall level and bin
+    pool_acc: Optional[object] = None     # float64 [S, G, N/B] pooled accumulator (finalise with pool_finalize)
 
 
 class SpectralPlan:
@@ -165,16 +198,32 @@ class SpectralPlan:
     def stft(self, x, *, n_streams: int = 1, db_rows=False, wf_rows=False, spectrum=False, welch=False,
              maxhold=False, vmin: float = -100.0, vmax: float = 0.0, accumulate: bool = False,
              stream: int = 0, n_samples: Optional[int] = None, peer_outputs: int = 0, persistence=False,
-             _time=None) -> StftResult:
+             pool=None, pool_acc=True, pool_first_frame: int = 0, _time=None) -> StftResult:
         """Windowed STFT of ``x`` (1 stream, or ``n_streams`` equal-length streams laid out back to
         back).  Each output flag is False (not wanted), True (allocate) or a caller buffer to fill
         (numpy for host input, DeviceArray / CUDA tensor for device input).
 
         ``persistence``: uint32 ``[n_streams, 256, nfft]``, for every bin the number of frames at each uint8 waterfall
         level of ``[vmin, vmax]`` (a persistence / density spectrum; every column sums to the frame count).  It is an
-        accumulator like ``welch`` and ``maxhold``.  It does not need ``wf_rows``: without them the rows stay on the GPU."""
+        accumulator like ``welch`` and ``maxhold``.  It does not need ``wf_rows``: without them the rows stay on the GPU.
+
+        ``pool=(K, B, "mean" | "max")``: a pooled spectrogram (display detectors).  Row g pools the frames
+        ``[g K, (g + 1) K)`` of global frame index (this call's frame 0 is ``pool_first_frame``), column c the bins
+        ``[c B, (c + 1) B)``; "mean" sums the power of the cell, "max" keeps its largest dB value.  ``pool_acc`` is the
+        float64 ``[n_streams, G, nfft / B]`` accumulator (True: allocate with G = ceil((pool_first_frame + F) / K)); it
+        is an accumulator like ``welch``, so calls on consecutive pieces of a capture pool into one image, and
+        ``pool_finalize`` turns it into dB and levels.  It does not need ``db_rows``: without them the rows stay on the
+        GPU."""
         if persistence is not False and persistence is not None and _time is not None:
             raise ValueError("persistence cannot be timed with _time (spx_stft_time runs spx_stft_exec)")
+        if pool is not None:
+            if _time is not None:
+                raise ValueError("pool cannot be timed with _time (spx_stft_time runs spx_stft_exec)")
+            if persistence is not False and persistence is not None:
+                raise ValueError("pool and persistence cannot be computed in one call")
+            pK, pB, pmode = _pool_shape(self.nfft, pool)
+            if int(pool_first_frame) < 0:
+                raise ValueError("pool_first_frame must be >= 0")
         if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
             x = self._host_input(x)
         in_ptr, mem = nat.as_ptr(x)
@@ -205,6 +254,27 @@ class SpectralPlan:
         o_we = out(welch, (n_streams, N), np.float64, "welch", accumulator=True)
         o_mh = out(maxhold, (n_streams, N), np.float32, "maxhold", accumulator=True)
         o_pe = out(persistence, (n_streams, 256, N), np.uint32, "persistence", accumulator=True)
+        o_pool = None
+        if pool is not None:
+            C_ = N // pB
+            if pool_acc is True:
+                G = -(-(int(pool_first_frame) + F) // pK)
+                # with accumulate=True a library-allocated accumulator adds to the mode's identity (0, or -inf for max)
+                if accumulate:
+                    ident = np.full((n_streams, G, C_), -np.inf if pmode == nat.POOL_MAX else 0.0)
+                    o_pool = ident if mem == MEM_HOST else DeviceArray.from_host(ident, self.device)
+                elif mem == MEM_HOST:
+                    o_pool = np.empty((n_streams, G, C_), np.float64)
+                else:
+                    o_pool = DeviceArray((n_streams, G, C_), np.float64, self.device)
+            else:
+                if pool_acc is False or pool_acc is None:
+                    raise ValueError("pool needs pool_acc (True or a buffer)")
+                _, cnt = _buffer_dtype_count(pool_acc)
+                G = cnt // max(1, n_streams * C_)
+                o_pool = out(pool_acc, (n_streams, G, C_), np.float64, "pool_acc", accumulator=True)
+            pa = nat.spx_pool_args(C.sizeof(nat.spx_pool_args), pmode, pK, pB, 0, int(pool_first_frame), G,
+                                   nat.as_ptr(o_pool)[0])
         a = nat.spx_stft_args()
         a.struct_size = C.sizeof(nat.spx_stft_args)
         a.mem = mem
@@ -228,10 +298,12 @@ class SpectralPlan:
             self.last_times_ms = [float(v) for v in ms]
         elif o_pe is not None:
             nat.check(nat.lib().spx_stft_exec_persistence(self._h, C.byref(a), nat.as_ptr(o_pe)[0]))
+        elif o_pool is not None:
+            nat.check(nat.lib().spx_stft_exec_pooled(self._h, C.byref(a), C.byref(pa)))
         else:
             nat.check(nat.lib().spx_stft_exec(self._h, C.byref(a)))
         return StftResult(int(a.n_frames_out), n_streams, o_db, o_wf, o_sp, o_we, o_mh,
-                          int(a.h2d_bytes_out), int(a.d2h_bytes_out), o_pe)
+                          int(a.h2d_bytes_out), int(a.d2h_bytes_out), o_pe, o_pool)
 
     def time_stft(self, x, *, warmup: int = 3, iters: int = 10, flush_l2: bool = False, **kw):
         """Device-resident timing of the exact launch ``stft`` would make: CUDA events on the launch
@@ -269,6 +341,28 @@ class SpectralPlan:
         nat.check(nat.lib().spx_welch_finalize_batch(self._h, mem, p, int(n_streams), int(n_frames), float(sample_rate),
                                                      nat.as_ptr(pxx)[0], nat.as_ptr(pdb)[0], stream or None))
         return pxx, pdb
+
+    def pool_finalize(self, pool_acc, n_frames_total: int, frames_per_row: int, bins_per_col: int, mode="mean",
+                      db: bool = True, wf: bool = False, vmin: float = -100.0, vmax: float = 0.0, n_streams: int = 1,
+                      stream: int = 0):
+        """Pooled dB (float32) and / or uint8 levels of ``[vmin, vmax]`` of an accumulator filled by
+        ``stft(pool=(frames_per_row, bins_per_col, mode))`` over ``n_frames_total`` frames, both shaped
+        ``[n_streams, G, nfft / B]`` with G = ceil(n_frames_total / K), in the accumulator's memory space.  Returns
+        ``(db, levels)``; an output not asked for is None.  The levels are those of the returned float32 dB."""
+        K, B, m = _pool_shape(self.nfft, (frames_per_row, bins_per_col, mode))
+        F = int(n_frames_total)
+        G = -(-F // K) if F > 0 else 0
+        shape = (int(n_streams), G, self.nfft // B)
+        _check_buffer(pool_acc, shape, np.float64, "pool_acc")
+        p, mem = nat.as_ptr(pool_acc)
+
+        def alloc(dtype):
+            return np.empty(shape, dtype) if mem == MEM_HOST else DeviceArray(shape, dtype, self.device)
+        o_db = alloc(np.float32) if db else None
+        o_wf = alloc(np.uint8) if wf else None
+        nat.check(nat.lib().spx_pool_finalize(self._h, mem, m, p, int(n_streams), G, F, K, B, nat.as_ptr(o_db)[0],
+                                              nat.as_ptr(o_wf)[0], float(vmin), float(vmax), stream or None))
+        return o_db, o_wf
 
 
 # ----------------------------------------------------------------------------- plan cache + convenience

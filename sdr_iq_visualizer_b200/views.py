@@ -93,6 +93,30 @@ def persistence_payload(counts, n_frames: int, vmin: float, vmax: float, freqs_m
     return {"z": z, "x": freqs_mhz, "y": y, "zmin": 0.0, "zmax": 1.0, "colorscale": scale, "db_range": (vmin, vmax)}
 
 
+def spectrogram_payload(db_or_levels, frames_per_row: int, hop: int, sample_rate: float, freqs_mhz=None,
+                        vmin: float = -100.0, vmax: float = 0.0) -> dict:
+    """Arguments of a ``go.Heatmap`` of a pooled spectrogram (``SpectralPlan.pool_finalize`` / ``process_recording(
+    overview=...)``, one stream's [G, C] float32 dB or uint8 levels, or [1, G, C]), in the style of
+    ``persistence_payload``: ``z`` as given (rows = pooled rows, oldest first), ``x`` the column frequencies
+    (``spectral.pooled_freq_axis`` in MHz), ``y`` each row's start time in seconds, g * K * hop / fs.  dB is shown over
+    [vmin, vmax], levels over [0, 255]."""
+    z = np.asarray(db_or_levels)
+    if z.ndim == 3:   # [S][G][C]: one stream only, so that no stream is dropped unseen
+        if z.shape[0] != 1:
+            raise ValueError(f"pooled rows: {z.shape[0]} streams; pass one stream's [G, C] rows")
+        z = z[0]
+    if z.ndim != 2:
+        raise ValueError(f"pooled rows: expected shape (G, C), got {z.shape}")
+    if int(frames_per_row) < 1 or int(hop) < 1 or not sample_rate > 0:
+        raise ValueError("frames_per_row and hop must be >= 1 and sample_rate > 0")
+    y = np.arange(z.shape[0], dtype=np.float64) * (int(frames_per_row) * int(hop) / float(sample_rate))
+    levels = z.dtype == np.uint8
+    lut = _spectral.viridis_lut()
+    scale = [[i / 255.0, "rgb(%d,%d,%d)" % tuple(lut[i])] for i in range(0, 256, 15)]
+    return {"z": z, "x": freqs_mhz, "y": y, "zmin": 0 if levels else vmin, "zmax": 255 if levels else vmax,
+            "colorscale": scale, "db_range": (vmin, vmax)}
+
+
 def constellation_density(samples, r: Optional[float] = None, bins: int = 256, in_fmt: int = _spectral.FMT_CF32,
                           in_scale: float = 1.0, device: int = 0) -> dict:
     """Exact I/Q density over ALL samples (kernel K4) instead of a random 2000-point scatter (:199-214).

@@ -262,6 +262,43 @@ SPX_API int spx_pool_finalize(spx_plan* plan, int32_t mem, int32_t mode, const d
                               int64_t n_rows, int64_t n_frames_total, int64_t frames_per_row, int32_t bins_per_col,
                               float* db_out, uint8_t* wf_out, float vmin, float vmax, void* stream);
 
+/* ---------------------------------------------------------------- digital down-converter (zoom)
+ * Mixes a band of interest to 0 Hz with a 64-bit NCO, low-pass filters it and keeps every decim-th output, so that the
+ * STFT path can look at a narrow band of a wide capture ("zoom").  For input x[n] (in_fmt samples times in_scale) whose
+ * sample n has global index first_sample + n:
+ *   phi(n) = ((first_sample + n) * phase_inc) mod 2^64              (exact integer arithmetic)
+ *   mix[n] = x[n] * exp(-2 pi i phi(n) / 2^64)                      (tuned shift = phase_inc * fs / 2^64)
+ *   y[m]   = sum_k h[k] mix[m D + T - 1 - k],  m = 0 .. M - 1,  M = (n_samples - T) / D + 1 (0 if n_samples < T)
+ * i.e. numpy's convolve(mix, h, 'valid')[::D].  The output rate is fs / D and its centre frequency fc + shift; with odd
+ * symmetric taps y[m] belongs to time (first_sample + m D + (T - 1) / 2) / fs.  Consecutive calls on pieces of a capture
+ * that overlap by T - D samples, each with the global first_sample of its piece, give the outputs of one call bit for bit:
+ * the arithmetic of y[m] depends only on global indices, the taps and the input.  Decimations beyond one stage (T > 8192)
+ * are two DDCs in cascade, the second with phase_inc 0. */
+typedef struct spx_ddc spx_ddc;
+
+typedef struct {
+    uint32_t struct_size;  /* sizeof(spx_ddc_config) */
+    int32_t device;
+    int32_t in_fmt;        /* SPX_FMT_* */
+    float in_scale;        /* multiplies every sample (0 = 1.0) */
+    int32_t decim;         /* D >= 1 (D > 2048 may return SPX_E_UNSUPPORTED: cascade two DDCs) */
+    int32_t n_taps;        /* T in [1, 8192] */
+    const double* taps;    /* host, h[0 .. T - 1]; rounded once to float32 at create */
+    int64_t phase_inc;     /* round(shift_hz / fs * 2^64) as two's complement */
+} spx_ddc_config;
+
+SPX_API int spx_ddc_create(spx_ddc** out, const spx_ddc_config* cfg);
+SPX_API int spx_ddc_destroy(spx_ddc* ddc);
+/* wait for everything the handle has enqueued on its own streams */
+SPX_API int spx_ddc_sync(spx_ddc* ddc);
+/* y of n_samples samples into out[M][2] (float32 I, Q); *n_out = M.  SPX_MEM_DEVICE: `in` / `out` are device pointers
+ * used on `stream` (NULL = the handle's stream), nothing is synchronised.  SPX_MEM_HOST: the input is staged through
+ * pieces of SPX_H2D_PIECE_BYTES (handle-creation environment variable, default 16 MiB) cut at output boundaries, the
+ * upload of one piece overlapping the kernel of the previous one; the call returns when `out` is written.  in and out
+ * must be 4-byte aligned.  SPX_E_INVALID for a bad mem, n_samples < 0, first_sample < 0, or NULL in / out when M > 0. */
+SPX_API int spx_ddc_exec(spx_ddc* ddc, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
+                         int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream);
+
 /* Measurement helper: runs spx_stft_exec (SPX_MEM_DEVICE buffers only) warmup+iters times on the
  * launch stream, each bracketed by CUDA events; optionally READS a 256 MiB buffer before every
  * iteration to flush the 126 MB L2 without leaving dirty lines behind.  ms_each[iters] receives the device time of

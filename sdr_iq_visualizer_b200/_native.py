@@ -62,6 +62,11 @@ class spx_pool_args(C.Structure):
 POOL_MEAN, POOL_MAX = 0, 1
 
 
+class spx_ddc_config(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("device", C.c_int32), ("in_fmt", C.c_int32), ("in_scale", C.c_float),
+                ("decim", C.c_int32), ("n_taps", C.c_int32), ("taps", C.c_void_p), ("phase_inc", C.c_int64)]
+
+
 class spx_features(C.Structure):
     _fields_ = [("n", C.c_int32), ("argmax", C.c_int32), ("peak_db", C.c_double), ("noise_floor_db", C.c_double),
                 ("snr_db", C.c_double), ("adaptive_thr", C.c_double), ("p20_lo", C.c_double), ("p20_hi", C.c_double),
@@ -124,6 +129,11 @@ _SIGNATURES = {
     "spx_stft_exec_pooled": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.POINTER(spx_pool_args)]),
     "spx_pool_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_int64,
                                     C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p]),
+    "spx_ddc_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(spx_ddc_config)]),
+    "spx_ddc_destroy": (C.c_int, [C.c_void_p]),
+    "spx_ddc_sync": (C.c_int, [C.c_void_p]),
+    "spx_ddc_exec": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.POINTER(C.c_int64),
+                               C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_void_p]),
     "spx_stft_time": (C.c_int, [C.c_void_p, C.POINTER(spx_stft_args), C.c_int32, C.c_int32, C.c_int32,
                                 C.POINTER(C.c_float)]),
     "spx_welch_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,

@@ -1,0 +1,454 @@
+// spx_ddc.cu -- digital down-converter: NCO mix + decimating FIR (DESIGN.md section 4, K9) and its C ABI (spx_ddc_*).
+//
+//   y[m] = sum_k h[k] mix[mD + T - 1 - k],   mix[n] = x[n] in_scale exp(-2 pi i ((first_sample + n) inc mod 2^64) / 2^64)
+//
+// A CTA owns a contiguous run of sub-tiles of SUB outputs.  Its mixed input lives in a shared-memory ring of
+// SUB D + T - 1 float2 samples: each sub-tile mixes the SUB D samples it adds (one NCO evaluation per sample, strategy
+// (a) of DESIGN.md K9), so a CTA mixes its T - 1 halo samples once, not once per sub-tile.  The reversed taps sit in shared
+// memory.  A warp computes R = 16 outputs m, m + s, ..., m + 15 s: lane l sums the taps j = l (mod 32) with a register
+// window that slides over the outputs (spx_ddc_device.cuh), so one shared load of a sample and one of a tap feed 32
+// FMAs.  A reduce-scatter over the lanes leaves output l / 2, component l % 2 in lane l; WR warps that split the tap
+// classes of the same outputs are added in a fixed order before the store.
+#include <stdlib.h>
+#include <string.h>
+
+#include <mutex>
+#include <new>
+#include <vector>
+
+#include "spx_ddc_device.cuh"
+#include "spx_internal.h"
+#include "spx_plan.h"
+
+namespace spx {
+
+constexpr int DDC_THREADS = 256;   // 8 warps
+constexpr int DDC_R = 16;          // outputs per warp: 2 R = 32 values, one per lane after the reduce-scatter
+constexpr int DDC_MAX_TAPS = 8192;
+constexpr size_t DDC_SMEM_TWO_PER_SM = 110u << 10;   // two CTAs per SM (228 KB, 1 KB reserved per CTA)
+
+struct DdcParams {
+    const void* in;
+    long long L;              // samples of the call
+    unsigned long long n0;    // global index of sample 0 (first_sample)
+    unsigned long long inc;   // phase increment
+    const float* taps;        // g[j] = h[T - 1 - j], float32
+    float* out;               // [M][2]
+    long long M;
+    long long n_sub;          // sub-tiles of the call
+    float scale;
+    int T, D, sub, ring, taps_pad;
+    int s, c, wr, wg;
+};
+
+template <int FMT>
+__device__ inline void ddc_load(const void* in, long long n, float* xr, float* xi) {
+    if (FMT == SPX_FMT_CI16) {
+        const short2 v = __ldg(reinterpret_cast<const short2*>(in) + n);
+        *xr = (float)v.x;
+        *xi = (float)v.y;
+    } else {
+        const float* f = reinterpret_cast<const float*>(in) + 2 * n;
+        *xr = __ldg(f);
+        *xi = __ldg(f + 1);
+    }
+}
+
+// mix CTA-relative samples [lo, hi) into the ring (slot = r mod ring); samples past the call's end are zero
+template <int FMT>
+__device__ inline void ddc_mix_range(const DdcParams& p, float2* ring, long long n_cta, long long lo, long long hi) {
+    long long r = lo + threadIdx.x;
+    int slot = (int)(r % p.ring);
+    constexpr int U = 4;
+    for (; r < hi; r += U * DDC_THREADS) {
+        float xr[U], xi[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const long long rr = r + u * DDC_THREADS, n = n_cta + rr;
+            xr[u] = 0.f;
+            xi[u] = 0.f;
+            if (rr < hi && n < p.L) ddc_load<FMT>(p.in, n, &xr[u], &xi[u]);
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const long long rr = r + u * DDC_THREADS;
+            if (rr < hi) {
+                const long long n = n_cta + rr;
+                float re, im;
+                ddc_mix(ddc_mul(xr[u], p.scale), ddc_mul(xi[u], p.scale), ddc_phase(p.n0 + (unsigned long long)n, p.inc), &re,
+                        &im);
+                ring[slot] = make_float2(re, im);
+            }
+            slot += DDC_THREADS;
+            if (slot >= p.ring) slot -= p.ring;
+        }
+    }
+}
+
+// one step t of a lane's sliding window: load element t + R - 1 into w[(K + R - 1) % R], then 2 R FMAs
+template <int K>
+__device__ __forceinline__ void ddc_step(float (&ar)[DDC_R], float (&ai)[DDC_R], float (&wre)[DDC_R], float (&wim)[DDC_R],
+                                         const float2* ring, int& slot, int step, int ring_n, float gv) {
+    const float2 v = ring[slot];
+    wre[(K + DDC_R - 1) % DDC_R] = v.x;
+    wim[(K + DDC_R - 1) % DDC_R] = v.y;
+    slot += step;
+    if (slot >= ring_n) slot -= ring_n;
+#pragma unroll
+    for (int i = 0; i < DDC_R; ++i) {
+        ar[i] = fmaf(gv, wre[(K + i) % DDC_R], ar[i]);
+        ai[i] = fmaf(gv, wim[(K + i) % DDC_R], ai[i]);
+    }
+}
+
+template <int... Ks>
+struct DdcSteps;
+template <>
+struct DdcSteps<> {
+    template <bool GUARD>
+    __device__ __forceinline__ static void run(float (&)[DDC_R], float (&)[DDC_R], float (&)[DDC_R], float (&)[DDC_R],
+                                               const float2*, int&, int, int, const float*, int, int) {}
+};
+template <int K, int... Ks>
+struct DdcSteps<K, Ks...> {
+    // taps t0 + K, t0 + K + 1, ... (GUARD: only those < n)
+    template <bool GUARD>
+    __device__ __forceinline__ static void run(float (&ar)[DDC_R], float (&ai)[DDC_R], float (&wre)[DDC_R],
+                                               float (&wim)[DDC_R], const float2* ring, int& slot, int step, int ring_n,
+                                               const float* gp, int t0, int n) {
+        if (GUARD && t0 + K >= n) return;
+        ddc_step<K>(ar, ai, wre, wim, ring, slot, step, ring_n, gp[(t0 + K) * step]);
+        DdcSteps<Ks...>::template run<GUARD>(ar, ai, wre, wim, ring, slot, step, ring_n, gp, t0, n);
+    }
+};
+using DdcAllSteps = DdcSteps<0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15>;
+static_assert(DDC_R == 16, "DdcAllSteps lists R steps");
+
+template <int FMT>
+__global__ void __launch_bounds__(DDC_THREADS, 2) ddc_kernel(const DdcParams p) {
+    extern __shared__ float4 ddc_smem[];
+    float* g = reinterpret_cast<float*>(ddc_smem);
+    float2* ring = reinterpret_cast<float2*>(g + p.taps_pad);
+    float* red = reinterpret_cast<float*>(ring + p.ring);   // [wr][sub][2]
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i < p.T; i += DDC_THREADS) g[i] = p.taps[i];
+    const long long sb0 = (long long)blockIdx.x * p.n_sub / gridDim.x;
+    const long long sb1 = (long long)(blockIdx.x + 1) * p.n_sub / gridDim.x;
+    const long long n_cta = sb0 * p.sub * (long long)p.D;   // call index of the CTA's sample 0
+    const int wr = warp % p.wr, wg = warp / p.wr;
+    const int groups = p.sub / DDC_R, step = 32 * p.c;
+    long long mixed = 0;
+    for (long long k = sb0; k <= sb1; ++k) {
+        const long long kk = k - sb0;
+        if (k < sb1) {
+            const long long hi = (kk + 1) * p.sub * (long long)p.D + p.T - 1;
+            ddc_mix_range<FMT>(p, ring, n_cta, mixed, hi);
+            mixed = hi;
+        }
+        if (k > sb0) {   // the outputs of the previous sub-tile: warp partials in order of wr
+            for (int idx = tid; idx < 2 * p.sub; idx += DDC_THREADS) {
+                const long long m = (k - 1) * p.sub + (idx >> 1);
+                if (m >= p.M) break;
+                float v = red[idx];
+                for (int w = 1; w < p.wr; ++w) v = __fadd_rn(v, red[w * 2 * p.sub + idx]);
+                p.out[2 * m + (idx & 1)] = v;
+            }
+        }
+        if (k == sb1) break;
+        __syncthreads();
+        for (int gi = wg; gi < groups; gi += p.wg) {
+            const int mm0 = (gi / p.s) * DDC_R * p.s + gi % p.s;
+            float ar[DDC_R], ai[DDC_R];
+#pragma unroll
+            for (int i = 0; i < DDC_R; ++i) ar[i] = ai[i] = 0.f;
+            for (int rho = wr; rho < p.c; rho += p.wr) {
+                const int n = ddc_lane_taps(p.T, p.c, lane, rho);
+                if (n == 0) continue;
+                const long long r0 = (kk * p.sub + mm0) * (long long)p.D + 32 * rho + lane;
+                int slot = (int)(r0 % p.ring);
+                const float* gp = g + 32 * rho + lane;
+                float wre[DDC_R], wim[DDC_R];
+#pragma unroll
+                for (int e = 0; e < DDC_R - 1; ++e) {
+                    const float2 v = ring[slot];
+                    wre[e] = v.x;
+                    wim[e] = v.y;
+                    slot += step;
+                    if (slot >= p.ring) slot -= p.ring;
+                }
+                int t0 = 0;
+                for (; t0 + DDC_R <= n; t0 += DDC_R)
+                    DdcAllSteps::run<false>(ar, ai, wre, wim, ring, slot, step, p.ring, gp, t0, n);
+                DdcAllSteps::run<true>(ar, ai, wre, wim, ring, slot, step, p.ring, gp, t0, n);
+            }
+            // reduce-scatter: value 2 i + comp of every lane, tree pairs (l, l ^ 16), (l, l ^ 8), ... -> lane 2 i + comp
+            float v[2 * DDC_R];
+#pragma unroll
+            for (int i = 0; i < DDC_R; ++i) {
+                v[2 * i] = ar[i];
+                v[2 * i + 1] = ai[i];
+            }
+#pragma unroll
+            for (int half = 16; half >= 1; half >>= 1) {
+                const bool up = (lane & half) != 0;
+#pragma unroll
+                for (int i = 0; i < half; ++i) {
+                    const float send = up ? v[i] : v[i + half];
+                    const float keep = up ? v[i + half] : v[i];
+                    v[i] = __fadd_rn(keep, __shfl_xor_sync(0xffffffffu, send, half));
+                }
+            }
+            red[(wr * p.sub + mm0 + (lane >> 1) * p.s) * 2 + (lane & 1)] = v[0];
+        }
+        __syncthreads();
+    }
+}
+
+// ------------------------------------------------------------------ launch geometry
+struct DdcLaunch {
+    DdcGeom G;
+    int sub, ring, taps_pad;
+    size_t smem;
+};
+
+static size_t ddc_smem_bytes(int T, int D, int wr, int sub, int* ring, int* taps_pad) {
+    *taps_pad = (T + 3) & ~3;
+    *ring = sub * D + T - 1;
+    return (size_t)*taps_pad * 4 + (size_t)*ring * 8 + (size_t)wr * sub * 8;
+}
+
+// SUB = R max(s, wg) k with the largest k that keeps two CTAs per SM (k = 1 and one CTA per SM when even that is too big)
+static int ddc_plan_launch(int T, int D, int max_smem, DdcLaunch* out) {
+    DdcLaunch L;
+    L.G = ddc_geom(D);
+    const int base = DDC_R * (L.G.s > L.G.wg ? L.G.s : L.G.wg);
+    int ring, tp;
+    if (ddc_smem_bytes(T, D, L.G.wr, base, &ring, &tp) > (size_t)max_smem)
+        return spx_set_error(SPX_E_UNSUPPORTED,
+                             "decim %d with %d taps needs more shared memory than one CTA has: decimate in two stages "
+                             "(a second DDC with shift 0 on the first one's output)", D, T);
+    int k = 1;
+    while ((long long)base * (k + 1) * D <= 16384 &&
+           ddc_smem_bytes(T, D, L.G.wr, base * (k + 1), &ring, &tp) <= DDC_SMEM_TWO_PER_SM)
+        ++k;
+    L.sub = base * k;
+    L.smem = ddc_smem_bytes(T, D, L.G.wr, L.sub, &L.ring, &L.taps_pad);
+    *out = L;
+    return SPX_OK;
+}
+
+}  // namespace spx
+
+using namespace spx;
+
+struct spx_ddc {
+    spx_ddc_config cfg{};
+    int sm_count = 0, max_smem = 0;
+    float* d_taps = nullptr;   // reversed, float32
+    DdcLaunch launch{};
+    cudaStream_t s_compute = nullptr, s_h2d = nullptr, s_d2h = nullptr;
+    std::vector<cudaEvent_t> events;
+    size_t piece_bytes = 16u << 20;   // H2D piece of the host path (SPX_H2D_PIECE_BYTES)
+    DevBuf st_in, st_out;
+    std::mutex mu;
+};
+
+namespace spx {
+
+static int ddc_event(spx_ddc* d, size_t i, cudaEvent_t* out) {
+    while (d->events.size() <= i) {
+        cudaEvent_t e;
+        SPX_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        d->events.push_back(e);
+    }
+    *out = d->events[i];
+    return SPX_OK;
+}
+
+static long long ddc_out_count(long long L, int T, int D) { return L < T ? 0 : (L - T) / D + 1; }
+
+// K9 over samples [0, L) of `in` (device), global index of sample 0 = n0, outputs -> out (device)
+static int ddc_launch(spx_ddc* d, const void* in, long long L, unsigned long long n0, float* out, cudaStream_t st) {
+    const int T = d->cfg.n_taps, D = d->cfg.decim;
+    const long long M = ddc_out_count(L, T, D);
+    if (M <= 0) return SPX_OK;
+    const DdcLaunch& G = d->launch;
+    DdcParams p;
+    p.in = in;
+    p.L = L;
+    p.n0 = n0;
+    p.inc = (unsigned long long)d->cfg.phase_inc;
+    p.taps = d->d_taps;
+    p.out = out;
+    p.M = M;
+    p.sub = G.sub;
+    p.n_sub = (M + G.sub - 1) / G.sub;
+    p.scale = d->cfg.in_scale;
+    p.T = T;
+    p.D = D;
+    p.ring = G.ring;
+    p.taps_pad = G.taps_pad;
+    p.s = G.G.s;
+    p.c = G.G.c;
+    p.wr = G.G.wr;
+    p.wg = G.G.wg;
+    const int per_sm = G.smem <= DDC_SMEM_TWO_PER_SM ? 2 : 1;
+    const long long cap = (long long)per_sm * (d->sm_count > 0 ? d->sm_count : 148);
+    const unsigned grid = (unsigned)(p.n_sub < cap ? p.n_sub : cap);
+    if (d->cfg.in_fmt == SPX_FMT_CI16)
+        ddc_kernel<SPX_FMT_CI16><<<grid, DDC_THREADS, G.smem, st>>>(p);
+    else
+        ddc_kernel<SPX_FMT_CF32><<<grid, DDC_THREADS, G.smem, st>>>(p);
+    SPX_CUDA(cudaGetLastError());
+    return SPX_OK;
+}
+
+// Host memory: pieces of about piece_bytes of input, cut at output boundaries with the T - D halo, uploaded on s_h2d into
+// two alternating buffers (the upload of piece k + 1 overlaps the kernel of piece k); each piece's outputs drain on s_d2h.
+static int ddc_exec_host(spx_ddc* d, const void* in, long long L, long long M, unsigned long long n0, float* out,
+                         int64_t* h2d_out, int64_t* d2h_out) {
+    const int T = d->cfg.n_taps, D = d->cfg.decim;
+    const size_t elt = d->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
+    long long per = ((long long)(d->piece_bytes / elt) - T) / D + 1;   // outputs per piece
+    if (per < 1) per = 1;
+    if (per > M) per = M;
+    const long long span = (per - 1) * D + T;   // input samples of a full piece
+    SPX_TRY(d->st_in.reserve(2 * (size_t)span * elt));
+    SPX_TRY(d->st_out.reserve((size_t)M * 8));
+    char* d_in[2] = {(char*)d->st_in.ptr, (char*)d->st_in.ptr + (size_t)span * elt};
+    float* d_out = (float*)d->st_out.ptr;
+    long long h2d = 0, d2h = 0;
+    size_t ev = 0;
+    cudaEvent_t e_done[2] = {nullptr, nullptr};
+    for (long long m0 = 0, k = 0; m0 < M; m0 += per, ++k) {
+        const long long nm = M - m0 < per ? M - m0 : per;
+        const long long a = m0 * D, n = (nm - 1) * D + T;
+        const int b = (int)(k & 1);
+        cudaEvent_t e_in, e_k;
+        SPX_TRY(ddc_event(d, ev++, &e_in));
+        SPX_TRY(ddc_event(d, ev++, &e_k));
+        if (e_done[b]) SPX_CUDA(cudaStreamWaitEvent(d->s_h2d, e_done[b], 0));   // the kernel that last read this buffer
+        SPX_CUDA(cudaMemcpyAsync(d_in[b], (const char*)in + (size_t)a * elt, (size_t)n * elt, cudaMemcpyHostToDevice, d->s_h2d));
+        h2d += n * (long long)elt;
+        SPX_CUDA(cudaEventRecord(e_in, d->s_h2d));
+        SPX_CUDA(cudaStreamWaitEvent(d->s_compute, e_in, 0));
+        SPX_TRY(ddc_launch(d, d_in[b], n, n0 + (unsigned long long)a, d_out + 2 * m0, d->s_compute));
+        SPX_CUDA(cudaEventRecord(e_k, d->s_compute));
+        e_done[b] = e_k;
+        SPX_CUDA(cudaStreamWaitEvent(d->s_d2h, e_k, 0));
+        SPX_CUDA(cudaMemcpyAsync(out + 2 * m0, d_out + 2 * m0, (size_t)nm * 8, cudaMemcpyDeviceToHost, d->s_d2h));
+        d2h += nm * 8;
+    }
+    SPX_CUDA(cudaStreamSynchronize(d->s_h2d));
+    SPX_CUDA(cudaStreamSynchronize(d->s_compute));
+    SPX_CUDA(cudaStreamSynchronize(d->s_d2h));
+    *h2d_out = h2d;
+    *d2h_out = d2h;
+    return SPX_OK;
+}
+
+}  // namespace spx
+
+extern "C" {
+
+int spx_ddc_create(spx_ddc** out, const spx_ddc_config* cfg) {
+    if (!out || !cfg) return spx_set_error(SPX_E_INVALID, "NULL argument");
+    *out = nullptr;
+    if (cfg->struct_size != sizeof(spx_ddc_config))
+        return spx_set_error(SPX_E_INVALID, "spx_ddc_config.struct_size %u != %zu", cfg->struct_size, sizeof(spx_ddc_config));
+    if (cfg->decim < 1) return spx_set_error(SPX_E_INVALID, "decim %d must be >= 1", cfg->decim);
+    if (cfg->n_taps < 1 || cfg->n_taps > DDC_MAX_TAPS)
+        return spx_set_error(SPX_E_INVALID,
+                             "n_taps %d must be in [1, %d]; for a larger decimation cascade two DDCs, the second with "
+                             "shift 0", cfg->n_taps, DDC_MAX_TAPS);
+    if (!cfg->taps) return spx_set_error(SPX_E_INVALID, "taps is NULL");
+    if (cfg->in_fmt != SPX_FMT_CF32 && cfg->in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt %d", cfg->in_fmt);
+    int ndev = 0;
+    SPX_TRY(spx_device_count(&ndev));
+    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
+    if (cfg->device < 0 || cfg->device >= ndev) return spx_set_error(SPX_E_INVALID, "device %d out of range (%d devices)", cfg->device, ndev);
+    SPX_CUDA(cudaSetDevice(cfg->device));
+    int max_smem = 0, sms = 0;
+    SPX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device));
+    SPX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device));
+    DdcLaunch launch;
+    SPX_TRY(ddc_plan_launch(cfg->n_taps, cfg->decim, max_smem, &launch));
+    spx_ddc* d = new (std::nothrow) spx_ddc();
+    if (!d) return spx_set_error(SPX_E_NOMEM, "out of host memory");
+    d->cfg = *cfg;
+    d->cfg.taps = nullptr;   // the handle keeps its own float32 copy
+    if (!(d->cfg.in_scale != 0.0f)) d->cfg.in_scale = 1.0f;
+    d->sm_count = sms;
+    d->max_smem = max_smem;
+    d->launch = launch;
+    if (const char* e = getenv("SPX_H2D_PIECE_BYTES")) { long long v = atoll(e); if (v >= 65536) d->piece_bytes = (size_t)v; }
+    int rc = SPX_OK;
+    do {
+        cudaError_t e;
+        std::vector<float> g((size_t)cfg->n_taps);
+        for (int j = 0; j < cfg->n_taps; ++j) g[(size_t)j] = (float)cfg->taps[cfg->n_taps - 1 - j];   // rounded once
+        if ((e = cudaMalloc(&d->d_taps, g.size() * sizeof(float))) != cudaSuccess) { rc = spx_set_error(SPX_E_NOMEM, "%s", cudaGetErrorString(e)); break; }
+        if ((e = cudaMemcpy(d->d_taps, g.data(), g.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
+        if ((e = cudaFuncSetAttribute(ddc_kernel<SPX_FMT_CF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)) != cudaSuccess ||
+            (e = cudaFuncSetAttribute(ddc_kernel<SPX_FMT_CI16>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
+        if ((e = cudaStreamCreateWithFlags(&d->s_compute, cudaStreamNonBlocking)) != cudaSuccess ||
+            (e = cudaStreamCreateWithFlags(&d->s_h2d, cudaStreamNonBlocking)) != cudaSuccess ||
+            (e = cudaStreamCreateWithFlags(&d->s_d2h, cudaStreamNonBlocking)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
+    } while (0);
+    if (rc != SPX_OK) {
+        spx_ddc_destroy(d);
+        return rc;
+    }
+    *out = d;
+    return SPX_OK;
+}
+
+int spx_ddc_destroy(spx_ddc* d) {
+    if (!d) return SPX_OK;
+    cudaSetDevice(d->cfg.device);
+    for (cudaStream_t s : {d->s_compute, d->s_h2d, d->s_d2h})
+        if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
+    for (cudaEvent_t e : d->events) cudaEventDestroy(e);
+    if (d->d_taps) cudaFree(d->d_taps);
+    d->st_in.release();
+    d->st_out.release();
+    delete d;
+    return SPX_OK;
+}
+
+int spx_ddc_sync(spx_ddc* d) {
+    if (!d) return spx_set_error(SPX_E_INVALID, "ddc is NULL");
+    std::lock_guard<std::mutex> g(d->mu);
+    SPX_CUDA(cudaSetDevice(d->cfg.device));
+    SPX_CUDA(cudaStreamSynchronize(d->s_h2d));
+    SPX_CUDA(cudaStreamSynchronize(d->s_compute));
+    SPX_CUDA(cudaStreamSynchronize(d->s_d2h));
+    return SPX_OK;
+}
+
+int spx_ddc_exec(spx_ddc* d, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
+                 int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream) {
+    if (!d) return spx_set_error(SPX_E_INVALID, "ddc is NULL");
+    if (mem != SPX_MEM_HOST && mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", mem);
+    if (n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
+    if (first_sample < 0) return spx_set_error(SPX_E_INVALID, "first_sample < 0");
+    const long long M = ddc_out_count(n_samples, d->cfg.n_taps, d->cfg.decim);
+    if (n_out) *n_out = M;
+    if (h2d_bytes_out) *h2d_bytes_out = 0;
+    if (d2h_bytes_out) *d2h_bytes_out = 0;
+    if (M == 0) return SPX_OK;
+    if (!out) return spx_set_error(SPX_E_INVALID, "out is NULL");
+    if (!in) return spx_set_error(SPX_E_INVALID, "in is NULL");
+    if (((uintptr_t)in & 3u) || ((uintptr_t)out & 3u)) return spx_set_error(SPX_E_INVALID, "in and out must be 4-byte aligned");
+    std::lock_guard<std::mutex> g(d->mu);
+    SPX_CUDA(cudaSetDevice(d->cfg.device));
+    if (mem == SPX_MEM_DEVICE)
+        return ddc_launch(d, in, n_samples, (unsigned long long)first_sample, out, stream ? (cudaStream_t)stream : d->s_compute);
+    int64_t h2d = 0, d2h = 0;
+    SPX_TRY(ddc_exec_host(d, in, n_samples, M, (unsigned long long)first_sample, out, &h2d, &d2h));
+    if (h2d_bytes_out) *h2d_bytes_out = h2d;
+    if (d2h_bytes_out) *d2h_bytes_out = d2h;
+    return SPX_OK;
+}
+
+}  // extern "C"

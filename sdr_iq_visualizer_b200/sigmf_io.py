@@ -231,6 +231,7 @@ class RecordingSpectra:
     overview_wf: Optional[np.ndarray] = None  # uint8 [G, N/B] its levels of [vmin, vmax]
     overview_frames_per_row: int = 0          # K
     overview_bins_per_col: int = 0            # B
+    zoom: Optional[tuple] = None              # (actual shift Hz, decim D, taps T) when the spectra are of a zoomed band
 
 
 def overview_pooling(n_frames: int, nfft: int, rows: int, cols: int) -> tuple:
@@ -249,7 +250,7 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
                       vmin: float = -120.0, vmax: float = 0.0, maxhold: bool = True, hist_r: Optional[float] = None,
                       hist_bins: int = 256, max_samples: Optional[int] = None, max_chunk_samples: int = 1 << 26,
                       device: int = 0, persistence: bool = False, overview: Optional[tuple] = None,
-                      overview_mode: str = "mean") -> RecordingSpectra:
+                      overview_mode: str = "mean", zoom: Optional[tuple] = None, zoom_taps=None) -> RecordingSpectra:
     """The offline path of process_sigmf_data.py on the GPU, for the whole file: Welch PSD with
     ``plt.psd(data, NFFT, Fs, Fc)`` semantics (Hann, ``noverlap = nfft - hop``, default no overlap), plus
     optional max-hold, uint8 waterfall rows and the I/Q density histogram.  ``max_samples`` restores
@@ -258,11 +259,18 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
     file's chunks without bringing the F x N rows to the host (unless ``waterfall`` asks for them too).
     ``overview=(rows, cols)``: a pooled spectrogram of about that many pixels (``overview_pooling`` picks K and B;
     ``overview_mode`` "mean" or "max" detector), accumulated on the GPU over the file's chunks in the same way; its dB
-    and levels of ``[vmin, vmax]`` are ``overview_db`` / ``overview_wf``."""
+    and levels of ``[vmin, vmax]`` are ``overview_db`` / ``overview_wf``.
+    ``zoom=(center_hz, decim)``: analyse the band around the absolute RF frequency ``center_hz`` instead of the whole
+    capture.  The file goes through a GPU down-converter (``ddc.DdcPlan``, default taps or ``zoom_taps``) chunk by chunk,
+    and every product above is computed on the decimated stream; the result describes that stream (``sample_rate`` fs / D,
+    ``center_freq`` fc + the tuned shift, ``freqs`` the zoomed axis, ``zoom`` = (shift, D, T))."""
     rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
     hop = int(hop or nfft)
     if max_samples is not None and max_samples < rec.n_samples:
         rec = SigMFRecording(rec.base, rec.meta, rec.datatype, rec.raw[: 2 * max_samples])
+    if zoom is not None:
+        return _process_zoomed(rec, zoom, zoom_taps, nfft, hop, window, waterfall, vmin, vmax, maxhold, hist_r,
+                               max_chunk_samples, device, persistence, overview, overview_mode)
     fs, fc = rec.sample_rate, rec.center_freq
     freqs = sp.freq_axis(nfft, fs, fc)
     L = rec.n_samples
@@ -323,6 +331,101 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
         o_db, o_wf = pl.pool_finalize(acc, F, K, B, overview_mode, db=True, wf=True, vmin=vmin, vmax=vmax)
         out.overview_db, out.overview_wf = o_db[0], o_wf[0]
         out.overview_frames_per_row, out.overview_bins_per_col = K, B
+    return out
+
+
+def _process_zoomed(rec, zoom, zoom_taps, nfft, hop, window, waterfall, vmin, vmax, maxhold, hist_r, max_chunk_samples,
+                    device, persistence, overview, overview_mode) -> RecordingSpectra:
+    """process_recording(zoom=...): each file chunk (``frame_chunks(T, D)``, halo T - D) is uploaded and down-converted
+    into a device buffer right after the unframed tail of the decimated stream; the STFT runs on that buffer and its last
+    unframed samples (fewer than nfft) are carried to the front of the other of two buffers for the next chunk."""
+    from . import ddc as ddc_mod
+    from ._native import DeviceArray, DeviceView
+    nat = sp.nat
+    if hist_r is not None:
+        raise ValueError("hist_r is not supported with zoom (the I/Q histogram is of the whole capture)")
+    center_hz, decim = zoom
+    fs, fc = rec.sample_rate, rec.center_freq
+    shift = float(center_hz) - fc
+    if abs(shift) > fs / 2:
+        raise ValueError(f"zoom centre {center_hz} Hz is {shift} Hz from the capture's centre {fc} Hz: |shift| must be "
+                         f"<= fs/2 = {fs / 2} Hz")
+    if overview is not None:
+        sp.pool_mode(overview_mode)
+        o_rows, o_cols = overview
+    nat.require_device()
+    dd = ddc_mod.DdcPlan(fs, shift, decim, zoom_taps, rec.in_fmt, rec.in_scale, device)
+    T, D = dd.n_taps, dd.decim
+    fs_z, fc_z = dd.out_rate, fc + dd.shift_hz
+    info = (dd.shift_hz, D, T)
+    M = dd.out_count(rec.n_samples)
+    if M < nfft:   # no full frame of the decimated stream: mlab zero-pads to one frame
+        y = dd.exec(rec.raw_slice() if rec.in_fmt == FMT_CI16 else rec.read_samples())
+        dd.close()
+        f, pxx = sp.welch_psd(y, nfft, hop, window, fs_z, fc_z, device=device)
+        out = RecordingSpectra(f, pxx, 1, sample_rate=fs_z, center_freq=fc_z,
+                               persistence=np.zeros((256, nfft), np.uint32) if persistence else None, zoom=info)
+        if overview is not None:
+            K, B = overview_pooling(0, nfft, o_rows, o_cols)
+            out.overview_db = np.zeros((0, nfft // B), np.float32)
+            out.overview_wf = np.zeros((0, nfft // B), np.uint8)
+            out.overview_frames_per_row, out.overview_bins_per_col = K, B
+        return out
+    pl = sp.get_plan(nfft, hop, window, FMT_CF32, 1.0, sp.DB_EPS_REFERENCE, device)
+    st = pl.stream
+    F = (M - nfft) // hop + 1
+    d_we = DeviceArray((1, nfft), np.float64, device)
+    d_mh = DeviceArray((1, nfft), np.float32, device) if maxhold else False
+    d_pc = DeviceArray((1, 256, nfft), np.uint32, device) if persistence else False
+    rows = np.empty((F, nfft), np.uint8) if waterfall else None
+    if overview is not None:
+        K, B = overview_pooling(F, nfft, o_rows, o_cols)
+        pool = (K, B, overview_mode)
+        d_acc = DeviceArray((1, -(-F // K), nfft // B), np.float64, device)
+    per = max(1, (max_chunk_samples - T) // D + 1)            # outputs per file chunk, at most
+    bufs = [DeviceArray((nfft - 1 + per,), np.complex64, device) for _ in range(2)]
+    d_raw = DeviceArray(((per - 1) * D + T,), np.complex64, device)   # the largest chunk, 8 bytes a sample
+    both = persistence and overview is not None   # pooling and persistence cannot share a call
+    carry = k = f0 = 0
+    for m0, nm, raw in rec.frame_chunks(T, D, max_chunk_samples):
+        buf, other = bufs[k & 1], bufs[(k + 1) & 1]
+        k += 1
+        raw = np.ascontiguousarray(raw)
+        nat.check(nat.lib().spx_stream_sync(device, st))   # the previous chunk's kernels are done with d_raw
+        nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
+        dd.exec(DeviceView(d_raw.ptr, raw.shape, raw.dtype, device),
+                out=DeviceView(buf.ptr + 8 * carry, (nm,), np.complex64, device), first_sample=m0 * D, stream=st)
+        n_avail = carry + nm
+        nf = pl.frame_count(n_avail)
+        if nf > 0:
+            x = DeviceView(buf.ptr, (n_avail,), np.complex64, device)
+            d_wf = DeviceArray((nf, nfft), np.uint8, device) if waterfall else False
+            pool_kw = dict(pool=pool, pool_acc=d_acc, pool_first_frame=f0) if overview is not None else {}
+            pl.stft(x, welch=d_we, maxhold=d_mh, wf_rows=d_wf, vmin=vmin, vmax=vmax, persistence=d_pc,
+                    accumulate=f0 > 0, **({} if both else pool_kw))
+            if both:
+                pl.stft(x, accumulate=f0 > 0, **pool_kw)
+            if waterfall:
+                pl.sync()
+                rows[f0:f0 + nf] = d_wf.to_host()
+            f0 += nf
+        consumed = nf * hop
+        carry = n_avail - consumed
+        if carry:
+            nat.check(nat.lib().spx_memcpy_d2d_async(device, other.ptr, buf.ptr + 8 * consumed, 8 * carry, st))
+    pxx, _ = pl.welch_finalize(d_we, F, fs_z, want_db=False)
+    out = RecordingSpectra(sp.freq_axis(nfft, fs_z, fc_z), None, F, sample_rate=fs_z, center_freq=fc_z, wf_rows=rows,
+                           zoom=info)
+    if overview is not None:
+        o_db, o_wf = pl.pool_finalize(d_acc, F, K, B, overview_mode, db=True, wf=True, vmin=vmin, vmax=vmax)
+    pl.sync()
+    out.pxx = pxx.to_host()
+    out.maxhold = d_mh.to_host()[0] if maxhold else None
+    out.persistence = d_pc.to_host()[0] if persistence else None
+    if overview is not None:
+        out.overview_db, out.overview_wf = o_db.to_host()[0], o_wf.to_host()[0]
+        out.overview_frames_per_row, out.overview_bins_per_col = K, B
+    dd.close()
     return out
 
 

@@ -69,6 +69,22 @@ int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out) {
     return SPX_OK;
 }
 
+// ------------------------------------------------------------------ plan-owned scratch across streams
+bool plan_has_scratch(const spx_plan* pl) { return pl->cfg.nfft > 8192 || pl->blu_m != 0; }
+
+int scratch_wait(spx_plan* pl, cudaStream_t st) {
+    if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
+    if (pl->scratch_stream_valid && pl->scratch_stream != st) SPX_CUDA(cudaStreamWaitEvent(st, pl->ev_scratch, 0));
+    return SPX_OK;
+}
+
+int scratch_record(spx_plan* pl, cudaStream_t st) {
+    SPX_CUDA(cudaEventRecord(pl->ev_scratch, st));
+    pl->scratch_stream = st;
+    pl->scratch_stream_valid = true;
+    return SPX_OK;
+}
+
 // ------------------------------------------------------------------ dispatch
 int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long long stream_stride, long long frames,
                        float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
@@ -223,11 +239,8 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
     // plan-owned scratch (four-step / K2v2 / Bluestein buffers, the row buffer): a device-resident call on a caller stream
     // may still be using it, so the kernels queued here on s_compute wait for that call first, as the device path does
     const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
-    const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || own_u8 || own_db;
-    if (owns_scratch) {
-        if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
-        if (pl->scratch_stream_valid && pl->scratch_stream != pl->s_compute) SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, pl->ev_scratch, 0));
-    }
+    const bool owns_scratch = plan_has_scratch(pl) || own_u8 || own_db;
+    if (owns_scratch) SPX_TRY(scratch_wait(pl, pl->s_compute));
 
     // accumulators: start from zero or from the caller's running values
     if (d_welch) {
@@ -383,11 +396,7 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
         SPX_CUDA(cudaMemcpyAsync(pc->acc, d_pool, pool_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
         d2h += (long long)pool_bytes;
     }
-    if (owns_scratch) {
-        SPX_CUDA(cudaEventRecord(pl->ev_scratch, pl->s_compute));
-        pl->scratch_stream = pl->s_compute;
-        pl->scratch_stream_valid = true;
-    }
+    if (owns_scratch) SPX_TRY(scratch_record(pl, pl->s_compute));
     SPX_CUDA(cudaStreamSynchronize(pl->s_h2d));
     SPX_CUDA(cudaStreamSynchronize(pl->s_h2d_alt));
     SPX_CUDA(cudaStreamSynchronize(pl->s_compute));
@@ -891,11 +900,8 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts, const Poo
         // first.
         const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
         const bool own_rows = own_u8 || own_db;
-        const bool owns_scratch = pl->cfg.nfft > 8192 || pl->blu_m != 0 || a->peer_outputs || own_rows;
-        if (owns_scratch) {
-            if (!pl->ev_scratch) SPX_CUDA(cudaEventCreateWithFlags(&pl->ev_scratch, cudaEventDisableTiming));
-            if (pl->scratch_stream_valid && pl->scratch_stream != st) SPX_CUDA(cudaStreamWaitEvent(st, pl->ev_scratch, 0));
-        }
+        const bool owns_scratch = plan_has_scratch(pl) || a->peer_outputs || own_rows;
+        if (owns_scratch) SPX_TRY(scratch_wait(pl, st));
         if (!a->accumulate) {
             if (a->welch_acc) SPX_CUDA(cudaMemsetAsync(a->welch_acc, 0, (size_t)S * N * sizeof(double), st));
             if (a->maxhold) SPX_CUDA(cudaMemsetAsync(a->maxhold, 0, (size_t)S * N * sizeof(float), st));
@@ -914,11 +920,7 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts, const Poo
                                      a->welch_acc, a->maxhold, a->vmin, a->vmax, st, a->peer_outputs ? 1 : 0);
         if (rc == SPX_OK && counts && !own_rows) rc = persist_launch(pl, a->wf_rows, S, F, counts, st);
         if (rc == SPX_OK && pc && !own_rows) rc = pool_launch(pl, a->db_rows, S, F, F, pc->first_frame, *pc, pc->acc, st);
-        if (rc == SPX_OK && owns_scratch) {
-            SPX_CUDA(cudaEventRecord(pl->ev_scratch, st));
-            pl->scratch_stream = st;
-            pl->scratch_stream_valid = true;
-        }
+        if (rc == SPX_OK && owns_scratch) rc = scratch_record(pl, st);
         return rc;
     }
     if (F == 0) {

@@ -64,6 +64,12 @@ struct spx_plan {
 
 namespace spx {
 int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out);
+// Plan-owned scratch (K2 halves, the K2v2 scratch and its counters, the Bluestein buffers) is shared by every call on the
+// plan, whatever stream it runs on.  A call that uses it brackets its kernels on `st`: scratch_wait makes `st` wait for
+// the last such call if that one ran on another stream, scratch_record marks `st` as the stream now using it.
+bool plan_has_scratch(const spx_plan* pl);
+int scratch_wait(spx_plan* pl, cudaStream_t st);
+int scratch_record(spx_plan* pl, cudaStream_t st);
 int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long long stream_stride, long long frames,
                        float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
                        float vmin, float vmax, cudaStream_t st, int sys_atomics = 0);

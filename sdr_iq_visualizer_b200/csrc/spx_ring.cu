@@ -210,6 +210,10 @@ extern "C" int spx_ring_commit(spx_ring* r, int64_t n_samples) {
     const long long F = spx_frame_count(avail, N, hop);
     if (s.d_welch) SPX_CUDA(cudaMemsetAsync(s.d_welch, 0, (size_t)N * sizeof(double), pl->s_compute));
     if (s.d_max) SPX_CUDA(cudaMemsetAsync(s.d_max, 0, (size_t)N * sizeof(float), pl->s_compute));
+    // a one-shot call on the same plan may still be using its scratch on a caller stream, and one enqueued after this
+    // commit must wait for the slot's kernels
+    const bool scratch = plan_has_scratch(pl);
+    if (scratch) SPX_TRY(scratch_wait(pl, pl->s_compute));
     SPX_TRY(stft_launch_device(pl, s.d_in, 1, 0, F, s.d_db, s.d_wf, nullptr, s.d_welch, s.d_max, r->cfg.vmin, r->cfg.vmax, pl->s_compute));
     SPX_CUDA(cudaEventRecord(s.e_stft, pl->s_compute));   // the rows are complete here: their copy does not wait for the measurements
     // classifier measurements of this slot's Welch block, right behind the STFT kernel on the same stream
@@ -219,6 +223,7 @@ extern "C" int spx_ring_commit(spx_ring* r, int64_t n_samples) {
         SPX_TRY(welch_finalize_launch(s.d_welch, N, inv, nullptr, s.d_pdb, pl->s_compute));
         SPX_TRY(spx_classify_features_dev(pl->cfg.device, s.d_pdb, 1, N, 1, N, s.d_feat, nullptr, 0, nullptr, pl->s_compute));
     }
+    if (scratch) SPX_TRY(scratch_record(pl, pl->s_compute));
     // carry the unconsumed tail into the head of the next slot's device buffer
     const long long consumed = F * hop;
     const long long new_carry = avail - consumed;

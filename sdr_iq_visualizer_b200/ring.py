@@ -9,7 +9,8 @@ per-buffer dicts (/root/reference/app/sdr/streamer.py:18,186-200).
     ...use blk...; ring.release() # slot can be reused
 
 Frames are continuous across slots; every slot is one Welch / max-hold block.  H2D / D2H byte counters
-are reported separately in ``stats()``.
+are reported separately in ``stats()``.  A commit is ordered with one-shot calls on the same plan that use its
+scratch (N > 8192 or Bluestein lengths), on whatever stream they run: a ring can share a cached plan with them.
 
 Ring depth: consecutive slots upload on two alternating streams.  A producer that keeps ``n_slots - 1`` commits in flight
 reaches the PCIe copy ceiling with ``n_slots >= 6`` (0.94 - 1.00 of it on config 2); with 4 slots only one upload is in

@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -86,30 +87,17 @@ int scratch_record(spx_plan* pl, cudaStream_t st) {
 }
 
 // ------------------------------------------------------------------ dispatch
+static size_t in_elt(const spx_plan* pl) { return pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8; }
+
 int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long long stream_stride, long long frames,
-                       float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
-                       float vmin, float vmax, cudaStream_t st, int sys_atomics) {
+                       const StftOut& out, cudaStream_t st) {
     if (frames <= 0 || n_streams <= 0) return SPX_OK;
-    if (pl->blu_m) {  // arbitrary length: Bluestein over the inner power-of-two plan, one stream at a time
-        const size_t elt = pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
-        const size_t N = (size_t)pl->cfg.nfft;
-        for (long long s = 0; s < n_streams; ++s) {
-            const size_t r0 = (size_t)(s * frames);
-            SPX_TRY(bluestein_launch_stream(pl, (const char*)in + (size_t)(s * stream_stride) * elt, frames, (long long)r0,
-                                            db_rows, wf_rows, spec_rows, welch_acc ? welch_acc + s * N : nullptr,
-                                            maxhold ? maxhold + s * N : nullptr, vmin, vmax, st, sys_atomics));
-        }
-        return SPX_OK;
-    }
-    if (pl->cfg.nfft >= 16384) {  // four-step path, one stream at a time
-        const size_t elt = pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
-        const size_t N = (size_t)pl->cfg.nfft;
-        for (long long s = 0; s < n_streams; ++s) {
-            const size_t r0 = (size_t)(s * frames);
-            SPX_TRY(bigfft_launch_stream(pl, (const char*)in + (size_t)(s * stream_stride) * elt, frames, (long long)r0,
-                                         db_rows, wf_rows, spec_rows, welch_acc ? welch_acc + s * N : nullptr,
-                                         maxhold ? maxhold + s * N : nullptr, vmin, vmax, st, sys_atomics));
-        }
+    // arbitrary length (Bluestein over the inner power-of-two plan) and the four-step path: one stream at a time
+    if (pl->blu_m || pl->cfg.nfft >= 16384) {
+        const auto launch_stream = pl->blu_m ? bluestein_launch_stream : bigfft_launch_stream;
+        for (long long s = 0; s < n_streams; ++s)
+            SPX_TRY(launch_stream(pl, (const char*)in + (size_t)(s * stream_stride) * in_elt(pl), frames, s * frames,
+                                  out.stream_at(s, pl->cfg.nfft), st));
         return SPX_OK;
     }
     StftLaunch L;
@@ -121,16 +109,16 @@ int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long l
     L.p.hop = pl->cfg.hop;
     L.p.win = pl->d_win;
     L.p.tw = pl->d_tw;
-    L.p.db_rows = db_rows;
-    L.p.wf_rows = wf_rows;
-    L.p.spec_rows = spec_rows;
-    L.p.welch_acc = welch_acc;
-    L.p.maxhold = maxhold;
+    L.p.db_rows = out.db;
+    L.p.wf_rows = out.wf;
+    L.p.spec_rows = out.spec;
+    L.p.welch_acc = out.welch;
+    L.p.maxhold = out.maxhold;
     L.p.db_eps = pl->cfg.db_eps;
-    L.p.db_pw_min = pl->cfg.db_eps * pl->cfg.db_eps * 1099511627776.0f;  // (2^20 eps)^2
-    L.p.sys_atomics = sys_atomics;
-    L.p.q_a = (float)(3.01029995663981195214 * 256.0 / ((double)vmax - (double)vmin));  // 10 log10(2) * scale
-    L.p.q_b = (float)(-(double)vmin * 256.0 / ((double)vmax - (double)vmin));
+    L.p.db_pw_min = db_pw_min(pl);
+    L.p.sys_atomics = out.sys_atomics;
+    L.p.q_a = out.q_a();
+    L.p.q_b = out.q_b();
     L.nfft = pl->cfg.nfft;
     L.in_fmt = pl->cfg.in_fmt;
     L.variant = pl->cfg.variant;
@@ -145,9 +133,7 @@ int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long l
     return spx_set_error(SPX_E_UNSUPPORTED, "nfft %d: large-N path not built yet", n);
 }
 
-static size_t in_elt(const spx_plan* pl) { return pl->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8; }
-
-// ------------------------------------------------------------------ row consumers without caller rows
+// ------------------------------------------------------------------ row consumers
 // The persistence spectrum consumes uint8 rows and the pooled spectrogram float dB rows.  Without caller rows of that kind
 // the STFT of frames [0, F) of every stream goes in batches through the plan's row buffer (SPX_PERSIST_ROWS_BYTES of
 // uint8 rows, or SPX_POOL_ROWS_BYTES of float rows), each batch followed by its consumer kernel on the same stream, so
@@ -159,144 +145,142 @@ static size_t in_elt(const spx_plan* pl) { return pl->cfg.in_fmt == SPX_FMT_CI16
 // batches run one stream at a time.
 enum RowKind { ROWS_U8, ROWS_DB };
 
+// The consumer of a call's rows besides the caller, if `acc` is set: the persistence counts [S][256][N] (uint32) of the
+// uint8 levels, or, when `pool` is set, the pooled accumulator [S][n_rows][N / B] (float64) of the float dB rows.  `acc`
+// is stream 0's accumulator, in the call's memory space or in device staging.
+struct RowSink {
+    char* acc = nullptr;
+    const PoolCall* pool = nullptr;
+    RowKind kind() const { return pool ? ROWS_DB : ROWS_U8; }
+    size_t stream_bytes(int N) const {
+        return pool ? (size_t)(pool->n_rows * (N / pool->bins_per_col)) * sizeof(double) : (size_t)256 * N * sizeof(uint32_t);
+    }
+    RowSink stream_at(long long s, int N) const {
+        RowSink k = *this;
+        if (acc) k.acc = acc + (size_t)s * stream_bytes(N);
+        return k;
+    }
+    // the rows of `out` this sink reads (null: none)
+    const void* rows_of(const StftOut& out) const { return pool ? (const void*)out.db : (const void*)out.wf; }
+    // over rows [S][F][N] of streams 0 .. S - 1 here, whose frame 0 is frame f0 of the call
+    int launch(const spx_plan* pl, const void* rows, long long S, long long F, long long f0, cudaStream_t st) const {
+        if (pool) return pool_launch(pl, (const float*)rows, S, F, pool->first_frame + f0, *pool, (double*)acc, st);
+        return persist_launch(pl, (const uint8_t*)rows, S, F, (uint32_t*)acc, st);
+    }
+};
+
+static size_t row_bytes(const spx_plan* pl, RowKind kind) { return (size_t)pl->cfg.nfft * (kind == ROWS_DB ? sizeof(float) : 1); }
+
 static long long row_batch_frames(const spx_plan* pl, RowKind kind, long long Sb, long long F) {
-    const size_t row = (size_t)pl->cfg.nfft * (kind == ROWS_DB ? sizeof(float) : 1);
-    long long fb = (long long)((kind == ROWS_DB ? pl->pool_rows_bytes : pl->persist_rows_bytes) / ((size_t)Sb * row));
+    long long fb = (long long)((kind == ROWS_DB ? pl->pool_rows_bytes : pl->persist_rows_bytes) / ((size_t)Sb * row_bytes(pl, kind)));
     if (fb < 1) fb = 1;
     return fb < F ? fb : F;
 }
 
-// consume(rows, s, Sb, f0, nf): rows [Sb][nf][N] of streams s .. s + Sb - 1, frames f0 .. f0 + nf - 1, in the buffer
-template <class Consume>
-static int row_batches(spx_plan* pl, RowKind kind, const char* in, long long S, long long stride, long long F,
-                       float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
-                       float vmin, float vmax, cudaStream_t st, Consume consume) {
+// The STFT of frames [0, F) of S streams into `out`, then `sink` over their rows: the caller's rows when `out` has rows
+// of the sink's kind, else batches through the row buffer.  f0: the call's index of frame 0 here.
+static int stft_then_sink(spx_plan* pl, const char* in, long long S, long long stride, long long F, long long f0,
+                          const StftOut& out, const RowSink& sink, cudaStream_t st) {
+    if (!sink.acc || sink.rows_of(out)) {
+        SPX_TRY(stft_launch_device(pl, in, S, stride, F, out, st));
+        return sink.acc ? sink.launch(pl, sink.rows_of(out), S, F, f0, st) : SPX_OK;
+    }
     const int N = pl->cfg.nfft, hop = pl->cfg.hop;
-    const size_t elt = in_elt(pl);
-    const long long Sb = S > 1 && (db_rows || wf_rows || spec_rows) ? 1 : S;
+    const RowKind kind = sink.kind();
+    const long long Sb = S > 1 && out.has_rows() ? 1 : S;
     const long long fb = row_batch_frames(pl, kind, Sb, F);
-    const size_t row = (size_t)N * (kind == ROWS_DB ? sizeof(float) : 1);
-    SPX_TRY(pl->st_rows.reserve((size_t)(Sb * fb) * row));   // a no-op when the host pipeline reserved it up front
+    SPX_TRY(pl->st_rows.reserve((size_t)(Sb * fb) * row_bytes(pl, kind)));   // a no-op when the host pipeline reserved it up front
     void* rows = pl->st_rows.ptr;
     for (long long s = 0; s < S; s += Sb) {
-        for (long long f0 = 0; f0 < F; f0 += fb) {
-            const long long nf = F - f0 < fb ? F - f0 : fb;
-            const size_t r0 = (size_t)(s * F + f0) * N;
-            SPX_TRY(stft_launch_device(pl, in + (size_t)(s * stride + f0 * hop) * elt, Sb, stride, nf,
-                                       kind == ROWS_DB ? (float*)rows : (db_rows ? db_rows + r0 : nullptr),
-                                       kind == ROWS_U8 ? (unsigned char*)rows : (wf_rows ? wf_rows + r0 : nullptr),
-                                       spec_rows ? spec_rows + r0 : nullptr, welch_acc ? welch_acc + s * N : nullptr,
-                                       maxhold ? maxhold + s * N : nullptr, vmin, vmax, st));
-            SPX_TRY(consume(rows, s, Sb, f0, nf));
+        for (long long b0 = 0; b0 < F; b0 += fb) {
+            const long long nf = F - b0 < fb ? F - b0 : fb;
+            StftOut o = out.rows_at((size_t)(s * F + b0), N).stream_at(s, N);
+            if (kind == ROWS_DB) o.db = (float*)rows;
+            else o.wf = (unsigned char*)rows;
+            SPX_TRY(stft_launch_device(pl, in + (size_t)(s * stride + b0 * hop) * in_elt(pl), Sb, stride, nf, o, st));
+            SPX_TRY(sink.stream_at(s, N).launch(pl, rows, Sb, nf, f0 + b0, st));
         }
     }
     return SPX_OK;
 }
 
-static int persist_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, float* db_rows,
-                           float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, uint32_t* counts,
-                           cudaStream_t st) {
+// The accumulators of a call in the caller's memory, in staging order: Welch sums, max-hold, the sink's.  Without
+// `accumulate` they start from zero, a pooled accumulator from the identity of pool->mode; `stage` is the device staging
+// of a host-memory call.
+struct CallAcc {
+    void* ptr;
+    size_t bytes;
+    const PoolCall* pool;
+    DevBuf* stage;
+};
+
+static std::vector<CallAcc> call_accs(spx_plan* pl, const spx_stft_args* a, const RowSink& sink) {
+    const size_t S = (size_t)a->n_streams;
     const int N = pl->cfg.nfft;
-    return row_batches(pl, ROWS_U8, in, S, stride, F, db_rows, nullptr, spec_rows, welch_acc, maxhold, vmin, vmax, st,
-                       [&](void* rows, long long s, long long Sb, long long, long long nf) {
-                           return persist_launch(pl, (const uint8_t*)rows, Sb, nf, counts + (size_t)s * 256 * N, st);
-                       });
+    std::vector<CallAcc> v;
+    if (a->welch_acc) v.push_back({a->welch_acc, S * N * sizeof(double), nullptr, &pl->st_welch});
+    if (a->maxhold) v.push_back({a->maxhold, S * N * sizeof(float), nullptr, &pl->st_max});
+    if (sink.acc) v.push_back({sink.acc, S * sink.stream_bytes(N), sink.pool, &pl->st_sink});
+    return v;
 }
 
-// acc: the accumulator of stream 0 of these streams; frame0: the global index of frame 0 of `in`
-static int pool_batches(spx_plan* pl, const char* in, long long S, long long stride, long long F, unsigned char* wf_rows,
-                        float2* spec_rows, double* welch_acc, float* maxhold, float vmin, float vmax, const PoolCall& pc,
-                        double* acc, long long frame0, cudaStream_t st) {
-    const long long cells = pc.n_rows * (pl->cfg.nfft / pc.bins_per_col);
-    return row_batches(pl, ROWS_DB, in, S, stride, F, nullptr, wf_rows, spec_rows, welch_acc, maxhold, vmin, vmax, st,
-                       [&](void* rows, long long s, long long Sb, long long f0, long long nf) {
-                           return pool_launch(pl, (const float*)rows, Sb, nf, nf, frame0 + f0, pc, acc + (size_t)s * cells,
-                                              st);
-                       });
+static int reset_on_device(const CallAcc& c, void* acc, cudaStream_t st) {
+    if (c.pool) return pool_fill_launch((double*)acc, (long long)(c.bytes / sizeof(double)), c.pool->mode, st);
+    SPX_CUDA(cudaMemsetAsync(acc, 0, c.bytes, st));
+    return SPX_OK;
 }
 
 // ------------------------------------------------------------------ host-memory pipeline
-static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t* counts, const PoolCall* pc) {
+static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, const RowSink& sink) {
     const int N = pl->cfg.nfft, hop = pl->cfg.hop;
     const size_t elt = in_elt(pl);
     const long long S = a->n_streams, L = a->n_samples;
     const long long stride_host = S > 1 ? a->stream_stride : 0;
     const size_t rows = (size_t)(S * F);
+    const std::vector<CallAcc> accs = call_accs(pl, a, sink);
     SPX_TRY(pl->st_in.reserve((size_t)(S * L) * elt));
     if (a->db_rows) SPX_TRY(pl->st_db.reserve(rows * N * sizeof(float)));
     if (a->wf_rows) SPX_TRY(pl->st_wf.reserve(rows * N));
     if (a->spec_rows) SPX_TRY(pl->st_spec.reserve(rows * N * sizeof(float2)));
-    if (a->welch_acc) SPX_TRY(pl->st_welch.reserve((size_t)S * N * sizeof(double)));
-    if (a->maxhold) SPX_TRY(pl->st_max.reserve((size_t)S * N * sizeof(float)));
+    for (const CallAcc& c : accs) SPX_TRY(c.stage->reserve(c.bytes));
     char* d_in = (char*)pl->st_in.ptr;
-    float* d_db = a->db_rows ? (float*)pl->st_db.ptr : nullptr;
-    unsigned char* d_wf = a->wf_rows ? (unsigned char*)pl->st_wf.ptr : nullptr;
-    float2* d_spec = a->spec_rows ? (float2*)pl->st_spec.ptr : nullptr;
-    double* d_welch = a->welch_acc ? (double*)pl->st_welch.ptr : nullptr;
-    float* d_max = a->maxhold ? (float*)pl->st_max.ptr : nullptr;
+    StftOut d_out;   // the outputs in device staging
+    d_out.db = a->db_rows ? (float*)pl->st_db.ptr : nullptr;
+    d_out.wf = a->wf_rows ? (unsigned char*)pl->st_wf.ptr : nullptr;
+    d_out.spec = a->spec_rows ? (float2*)pl->st_spec.ptr : nullptr;
+    d_out.welch = a->welch_acc ? (double*)pl->st_welch.ptr : nullptr;
+    d_out.maxhold = a->maxhold ? (float*)pl->st_max.ptr : nullptr;
+    d_out.vmin = a->vmin;
+    d_out.vmax = a->vmax;
+    RowSink d_sink = sink;
+    if (sink.acc) d_sink.acc = (char*)pl->st_sink.ptr;
     long long h2d = 0, d2h = 0;
 
     // plan-owned scratch (four-step / K2v2 / Bluestein buffers, the row buffer): a device-resident call on a caller stream
     // may still be using it, so the kernels queued here on s_compute wait for that call first, as the device path does
-    const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
-    const bool owns_scratch = plan_has_scratch(pl) || own_u8 || own_db;
+    const bool own_rows = sink.acc && !sink.rows_of(d_out);
+    const bool owns_scratch = plan_has_scratch(pl) || own_rows;
     if (owns_scratch) SPX_TRY(scratch_wait(pl, pl->s_compute));
 
-    // accumulators: start from zero or from the caller's running values
-    if (d_welch) {
+    // accumulators: start from the caller's running values or from their reset value
+    for (const CallAcc& c : accs) {
         if (a->accumulate) {
-            SPX_CUDA(cudaMemcpyAsync(d_welch, a->welch_acc, (size_t)S * N * sizeof(double), cudaMemcpyHostToDevice, pl->s_compute));
-            h2d += S * N * (long long)sizeof(double);
+            SPX_CUDA(cudaMemcpyAsync(c.stage->ptr, c.ptr, c.bytes, cudaMemcpyHostToDevice, pl->s_compute));
+            h2d += (long long)c.bytes;
         } else {
-            SPX_CUDA(cudaMemsetAsync(d_welch, 0, (size_t)S * N * sizeof(double), pl->s_compute));
-        }
-    }
-    if (d_max) {
-        if (a->accumulate) {
-            SPX_CUDA(cudaMemcpyAsync(d_max, a->maxhold, (size_t)S * N * sizeof(float), cudaMemcpyHostToDevice, pl->s_compute));
-            h2d += S * N * (long long)sizeof(float);
-        } else {
-            SPX_CUDA(cudaMemsetAsync(d_max, 0, (size_t)S * N * sizeof(float), pl->s_compute));
-        }
-    }
-    // persistence counts: from the caller's running values only when accumulating
-    const size_t count_bytes = (size_t)S * 256 * N * sizeof(uint32_t);
-    uint32_t* d_counts = nullptr;
-    if (counts) {
-        SPX_TRY(pl->st_counts.reserve(count_bytes));
-        d_counts = (uint32_t*)pl->st_counts.ptr;
-        if (a->accumulate) {
-            SPX_CUDA(cudaMemcpyAsync(d_counts, counts, count_bytes, cudaMemcpyHostToDevice, pl->s_compute));
-            h2d += (long long)count_bytes;
-        } else {
-            SPX_CUDA(cudaMemsetAsync(d_counts, 0, count_bytes, pl->s_compute));
-        }
-    }
-    // pooled accumulator: the same rule, the mode's identity when not accumulating
-    const long long pool_cells = pc ? pc->n_rows * (N / pc->bins_per_col) : 0;
-    const size_t pool_bytes = (size_t)(S * pool_cells) * sizeof(double);
-    double* d_pool = nullptr;
-    if (pc) {
-        SPX_TRY(pl->st_pool.reserve(pool_bytes));
-        d_pool = (double*)pl->st_pool.ptr;
-        if (a->accumulate) {
-            SPX_CUDA(cudaMemcpyAsync(d_pool, pc->acc, pool_bytes, cudaMemcpyHostToDevice, pl->s_compute));
-            h2d += (long long)pool_bytes;
-        } else {
-            SPX_TRY(pool_fill_launch(d_pool, S * pool_cells, pc->mode, pl->s_compute));
+            SPX_TRY(reset_on_device(c, c.stage->ptr, pl->s_compute));
         }
     }
 
     // piece size: big enough to amortise launches, small enough to overlap (about 8-16 MiB)
     long long piece = (long long)(pl->piece_bytes / elt);
     if (piece < (long long)N * 4) piece = (long long)N * 4;
-    // counts / pooling without rows: one row buffer for every piece, sized for the largest (a piece spans at most `piece`
-    // samples, so at most piece / hop + 1 frames), reserved here -- growing it between pieces would free device memory,
-    // which synchronises the device in the middle of the pipeline
-    if (own_u8 || own_db) {
+    // a sink without rows: one row buffer for every piece, sized for the largest (a piece spans at most `piece` samples, so
+    // at most piece / hop + 1 frames), reserved here -- growing it between pieces would free device memory, which
+    // synchronises the device in the middle of the pipeline
+    if (own_rows) {
         const long long most = piece / hop + 2 < F ? piece / hop + 2 : F;
-        const RowKind kind = own_db ? ROWS_DB : ROWS_U8;
-        SPX_TRY(pl->st_rows.reserve((size_t)row_batch_frames(pl, kind, 1, most) * N * (own_db ? sizeof(float) : 1)));
+        SPX_TRY(pl->st_rows.reserve((size_t)row_batch_frames(pl, sink.kind(), 1, most) * row_bytes(pl, sink.kind())));
     }
     struct Piece { long long s, f_lo, f_hi; };
     std::vector<Piece> pieces;
@@ -331,28 +315,10 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
             SPX_TRY(plan_event(pl, ev++, &e_k));
             SPX_CUDA(cudaEventRecord(e_in, pl->s_h2d));
             SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, e_in, 0));
-            const size_t r0 = (size_t)(s * F + f_lo);
             NvtxRange r_k("spx STFT kernel piece");
-            if (own_u8) {   // counts without rows: the piece's rows go through the plan's row buffer
-                SPX_TRY(persist_batches(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, d_db ? d_db + r0 * N : nullptr,
-                                        d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
-                                        d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, d_counts + (size_t)s * 256 * N,
-                                        pl->s_compute));
-            } else if (own_db) {   // pooling without dB rows: likewise, float rows
-                SPX_TRY(pool_batches(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, d_wf ? d_wf + r0 * N : nullptr,
-                                     d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
-                                     d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, *pc, d_pool + (size_t)(s * pool_cells),
-                                     pc->first_frame + f_lo, pl->s_compute));
-            } else {
-                SPX_TRY(stft_launch_device(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo,
-                                           d_db ? d_db + r0 * N : nullptr, d_wf ? d_wf + r0 * N : nullptr,
-                                           d_spec ? d_spec + r0 * N : nullptr, d_welch ? d_welch + s * N : nullptr,
-                                           d_max ? d_max + s * N : nullptr, a->vmin, a->vmax, pl->s_compute));
-                if (d_counts) SPX_TRY(persist_launch(pl, d_wf + r0 * N, 1, f_hi - f_lo, d_counts + (size_t)s * 256 * N, pl->s_compute));
-                if (d_pool)
-                    SPX_TRY(pool_launch(pl, d_db + r0 * N, 1, f_hi - f_lo, f_hi - f_lo, pc->first_frame + f_lo, *pc,
-                                        d_pool + (size_t)(s * pool_cells), pl->s_compute));
-            }
+            SPX_TRY(stft_then_sink(pl, dd + (size_t)(f_lo * hop) * elt, 1, 0, f_hi - f_lo, f_lo,
+                                   d_out.rows_at((size_t)(s * F + f_lo), N).stream_at(s, N), d_sink.stream_at(s, N),
+                                   pl->s_compute));
             SPX_CUDA(cudaEventRecord(e_k, pl->s_compute));
             pieces.push_back({s, f_lo, f_hi});
             f_lo = f_hi;
@@ -364,37 +330,25 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, uint32_t*
     for (const Piece& pc : pieces) {
         cudaEvent_t e_k = pl->events[evi];
         evi += 2;
-        if (!(d_db || d_wf || d_spec)) continue;
+        if (!d_out.has_rows()) continue;
         SPX_CUDA(cudaStreamWaitEvent(pl->s_d2h, e_k, 0));
         const size_t r0 = (size_t)(pc.s * F + pc.f_lo), nr = (size_t)(pc.f_hi - pc.f_lo);
-        if (d_db) {
-            SPX_CUDA(cudaMemcpyAsync(a->db_rows + r0 * N, d_db + r0 * N, nr * N * sizeof(float), cudaMemcpyDeviceToHost, pl->s_d2h));
+        if (d_out.db) {
+            SPX_CUDA(cudaMemcpyAsync(a->db_rows + r0 * N, d_out.db + r0 * N, nr * N * sizeof(float), cudaMemcpyDeviceToHost, pl->s_d2h));
             d2h += (long long)(nr * N * sizeof(float));
         }
-        if (d_wf) {
-            SPX_CUDA(cudaMemcpyAsync(a->wf_rows + r0 * N, d_wf + r0 * N, nr * N, cudaMemcpyDeviceToHost, pl->s_d2h));
+        if (d_out.wf) {
+            SPX_CUDA(cudaMemcpyAsync(a->wf_rows + r0 * N, d_out.wf + r0 * N, nr * N, cudaMemcpyDeviceToHost, pl->s_d2h));
             d2h += (long long)(nr * N);
         }
-        if (d_spec) {
-            SPX_CUDA(cudaMemcpyAsync(a->spec_rows + r0 * N * 2, d_spec + r0 * N, nr * N * sizeof(float2), cudaMemcpyDeviceToHost, pl->s_d2h));
+        if (d_out.spec) {
+            SPX_CUDA(cudaMemcpyAsync(a->spec_rows + r0 * N * 2, d_out.spec + r0 * N, nr * N * sizeof(float2), cudaMemcpyDeviceToHost, pl->s_d2h));
             d2h += (long long)(nr * N * sizeof(float2));
         }
     }
-    if (d_welch) {
-        SPX_CUDA(cudaMemcpyAsync(a->welch_acc, d_welch, (size_t)S * N * sizeof(double), cudaMemcpyDeviceToHost, pl->s_compute));
-        d2h += S * N * (long long)sizeof(double);
-    }
-    if (d_max) {
-        SPX_CUDA(cudaMemcpyAsync(a->maxhold, d_max, (size_t)S * N * sizeof(float), cudaMemcpyDeviceToHost, pl->s_compute));
-        d2h += S * N * (long long)sizeof(float);
-    }
-    if (d_counts) {
-        SPX_CUDA(cudaMemcpyAsync(counts, d_counts, count_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
-        d2h += (long long)count_bytes;
-    }
-    if (d_pool) {
-        SPX_CUDA(cudaMemcpyAsync(pc->acc, d_pool, pool_bytes, cudaMemcpyDeviceToHost, pl->s_compute));
-        d2h += (long long)pool_bytes;
+    for (const CallAcc& c : accs) {
+        SPX_CUDA(cudaMemcpyAsync(c.ptr, c.stage->ptr, c.bytes, cudaMemcpyDeviceToHost, pl->s_compute));
+        d2h += (long long)c.bytes;
     }
     if (owns_scratch) SPX_TRY(scratch_record(pl, pl->s_compute));
     SPX_CUDA(cudaStreamSynchronize(pl->s_h2d));
@@ -464,6 +418,7 @@ static int stft_exec_device_peer(spx_plan* pl, spx_stft_args* a, long long F, cu
         SPX_TRY(plan_event(pl, (size_t)i, &e_k[i]));
         SPX_TRY(plan_event(pl, (size_t)(2 + i), &e_c[i]));
     }
+    const StftOut local{nullptr, a->wf_rows, nullptr, w_local, m_local, a->vmin, a->vmax};
     long long idx = 0;
     for (long long s = 0; s < S; ++s) {
         const char* in_s = (const char*)a->in + (size_t)(s * a->stream_stride) * elt;
@@ -472,10 +427,9 @@ static int stft_exec_device_peer(spx_plan* pl, spx_stft_args* a, long long F, cu
             const int b = (int)(idx & 1);
             const bool staged = a->wf_rows && !rows_local;
             if (idx >= 2 && staged) SPX_CUDA(cudaStreamWaitEvent(st, e_c[b], 0));   // the copy that last used this buffer is done
-            unsigned char* rows_dst = staged ? stage[b] : (a->wf_rows ? a->wf_rows + (size_t)(s * F + f_lo) * N : nullptr);
-            SPX_TRY(stft_launch_device(pl, in_s + (size_t)(f_lo * hop) * elt, 1, 0, nf, nullptr, rows_dst, nullptr,
-                                       w_local ? w_local + s * N : nullptr, m_local ? m_local + s * N : nullptr,
-                                       a->vmin, a->vmax, st, 0));
+            StftOut o = local.rows_at((size_t)(s * F + f_lo), N).stream_at(s, N);
+            if (staged) o.wf = stage[b];
+            SPX_TRY(stft_launch_device(pl, in_s + (size_t)(f_lo * hop) * elt, 1, 0, nf, o, st));
             if (!staged) continue;
             SPX_CUDA(cudaEventRecord(e_k[b], st));
             SPX_CUDA(cudaStreamWaitEvent(pl->s_d2h, e_k[b], 0));
@@ -756,7 +710,7 @@ int spx_plan_destroy(spx_plan* pl) {
     pl->st_big.release();
     pl->st_in.release(); pl->st_db.release(); pl->st_wf.release(); pl->st_spec.release();
     pl->st_welch.release(); pl->st_max.release(); pl->st_misc.release(); pl->st_flush.release();
-    pl->st_counts.release(); pl->st_pool.release(); pl->st_rows.release();
+    pl->st_sink.release(); pl->st_rows.release();
     delete pl;
     return SPX_OK;
 }
@@ -864,22 +818,23 @@ int spx_plan_window_sums(spx_plan* pl, double* sum_w2, double* sum_w) {
     return SPX_OK;
 }
 
-// spx_stft_exec, plus the persistence counts [S][256][N] of the call's uint8 levels when `counts` is not NULL, or the
-// pooled accumulator when `pc` is not NULL (never both)
-static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts, const PoolCall* pc) {
+// spx_stft_exec, plus `sink` over the call's rows when sink.acc is not NULL
+static int stft_exec(spx_plan* pl, spx_stft_args* a, const RowSink& sink) {
     if (!pl || !a) return spx_set_error(SPX_E_INVALID, "NULL argument");
     if (a->struct_size != sizeof(spx_stft_args))
         return spx_set_error(SPX_E_INVALID, "spx_stft_args.struct_size %u != %zu", a->struct_size, sizeof(spx_stft_args));
-    if (counts && a->peer_outputs) return spx_set_error(SPX_E_UNSUPPORTED, "persistence with peer_outputs is not supported");
-    if (pc && a->peer_outputs) return spx_set_error(SPX_E_UNSUPPORTED, "pooling with peer_outputs is not supported");
+    if (sink.acc && a->peer_outputs)
+        return spx_set_error(SPX_E_UNSUPPORTED, "%s with peer_outputs is not supported", sink.pool ? "pooling" : "persistence");
     if (a->n_streams < 1) return spx_set_error(SPX_E_INVALID, "n_streams must be >= 1");
     if (a->n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
     if (a->mem != SPX_MEM_HOST && a->mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", a->mem);
     if ((a->wf_rows != nullptr) && !(a->vmax > a->vmin)) return spx_set_error(SPX_E_INVALID, "wf_rows needs vmax > vmin");
-    if (counts && !(a->vmax > a->vmin)) return spx_set_error(SPX_E_INVALID, "persistence needs vmax > vmin");
+    if (sink.acc && sink.kind() == ROWS_U8 && !(a->vmax > a->vmin))
+        return spx_set_error(SPX_E_INVALID, "persistence needs vmax > vmin");
     if (a->n_streams > 1 && a->stream_stride < a->n_samples && a->mem == SPX_MEM_HOST)
         return spx_set_error(SPX_E_INVALID, "stream_stride < n_samples");
     const long long F = spx_frame_count(a->n_samples, pl->cfg.nfft, pl->cfg.hop);
+    const PoolCall* pc = sink.pool;
     if (pc && F > 0 && pool_row_of(pc->first_frame + F - 1, pc->frames_per_row) >= pc->n_rows)
         return spx_set_error(SPX_E_INVALID, "frames %lld .. %lld fall outside the %lld pooled rows of %lld frames",
                              pc->first_frame, pc->first_frame + F - 1, pc->n_rows, pc->frames_per_row);
@@ -888,59 +843,40 @@ static int stft_exec(spx_plan* pl, spx_stft_args* a, uint32_t* counts, const Poo
     a->d2h_bytes_out = 0;
     std::lock_guard<std::mutex> g(pl->mu);
     SPX_CUDA(cudaSetDevice(pl->cfg.device));
-    const int N = pl->cfg.nfft;
-    const long long S = a->n_streams;
-    const size_t count_bytes = (size_t)S * 256 * N * sizeof(uint32_t);
-    const long long pool_cells = pc ? pc->n_rows * (N / pc->bins_per_col) : 0;
     if (a->in == nullptr && F > 0) return spx_set_error(SPX_E_INVALID, "in is NULL");
     if (a->mem == SPX_MEM_DEVICE) {
         cudaStream_t st = a->stream ? (cudaStream_t)a->stream : pl->s_compute;
+        const StftOut out{a->db_rows, a->wf_rows, reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold,
+                          a->vmin, a->vmax, a->peer_outputs ? 1 : 0};
         // Plan-owned scratch (four-step / K2v2 scratch and counters, Bluestein buffers, peer staging, the row buffer) is
         // shared by every call on this plan: a call on another stream than the previous one waits for that one's kernels
         // first.
-        const bool own_u8 = counts && !a->wf_rows, own_db = pc && !a->db_rows;
-        const bool own_rows = own_u8 || own_db;
-        const bool owns_scratch = plan_has_scratch(pl) || a->peer_outputs || own_rows;
+        const bool owns_scratch = plan_has_scratch(pl) || a->peer_outputs || (sink.acc && !sink.rows_of(out));
         if (owns_scratch) SPX_TRY(scratch_wait(pl, st));
-        if (!a->accumulate) {
-            if (a->welch_acc) SPX_CUDA(cudaMemsetAsync(a->welch_acc, 0, (size_t)S * N * sizeof(double), st));
-            if (a->maxhold) SPX_CUDA(cudaMemsetAsync(a->maxhold, 0, (size_t)S * N * sizeof(float), st));
-            if (counts) SPX_CUDA(cudaMemsetAsync(counts, 0, count_bytes, st));
-            if (pc) SPX_TRY(pool_fill_launch(pc->acc, S * pool_cells, pc->mode, st));
-        }
+        if (!a->accumulate)
+            for (const CallAcc& c : call_accs(pl, a, sink)) SPX_TRY(reset_on_device(c, c.ptr, st));
         int rc;
-        if (own_db) rc = pool_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->wf_rows,
-                                      reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold, a->vmin, a->vmax, *pc,
-                                      pc->acc, pc->first_frame, st);
-        else if (own_u8) rc = persist_batches(pl, (const char*)a->in, S, a->stream_stride, F, a->db_rows,
-                                           reinterpret_cast<float2*>(a->spec_rows), a->welch_acc, a->maxhold, a->vmin, a->vmax,
-                                           counts, st);
-        else if (a->peer_outputs && !a->db_rows && !a->spec_rows && F > 0) rc = stft_exec_device_peer(pl, a, F, st);
-        else rc = stft_launch_device(pl, a->in, S, a->stream_stride, F, a->db_rows, a->wf_rows, reinterpret_cast<float2*>(a->spec_rows),
-                                     a->welch_acc, a->maxhold, a->vmin, a->vmax, st, a->peer_outputs ? 1 : 0);
-        if (rc == SPX_OK && counts && !own_rows) rc = persist_launch(pl, a->wf_rows, S, F, counts, st);
-        if (rc == SPX_OK && pc && !own_rows) rc = pool_launch(pl, a->db_rows, S, F, F, pc->first_frame, *pc, pc->acc, st);
+        if (a->peer_outputs && !a->db_rows && !a->spec_rows && F > 0) rc = stft_exec_device_peer(pl, a, F, st);
+        else rc = stft_then_sink(pl, (const char*)a->in, a->n_streams, a->stream_stride, F, 0, out, sink, st);
         if (rc == SPX_OK && owns_scratch) rc = scratch_record(pl, st);
         return rc;
     }
-    if (F == 0) {
-        if (!a->accumulate) {
-            if (a->welch_acc) memset(a->welch_acc, 0, (size_t)S * N * sizeof(double));
-            if (a->maxhold) memset(a->maxhold, 0, (size_t)S * N * sizeof(float));
-            if (counts) memset(counts, 0, count_bytes);
-            const double id = pc && pc->mode == SPX_POOL_MAX ? -INFINITY : 0.0;
-            for (long long i = 0; i < S * pool_cells; ++i) pc->acc[i] = id;
-        }
+    if (F == 0) {   // nothing to run: the accumulators are reset in host memory
+        if (!a->accumulate)
+            for (const CallAcc& c : call_accs(pl, a, sink)) {
+                if (c.pool) std::fill_n((double*)c.ptr, c.bytes / sizeof(double), c.pool->mode == SPX_POOL_MAX ? -INFINITY : 0.0);
+                else memset(c.ptr, 0, c.bytes);
+            }
         return SPX_OK;
     }
-    return stft_exec_host(pl, a, F, counts, pc);
+    return stft_exec_host(pl, a, F, sink);
 }
 
-int spx_stft_exec(spx_plan* pl, spx_stft_args* a) { return stft_exec(pl, a, nullptr, nullptr); }
+int spx_stft_exec(spx_plan* pl, spx_stft_args* a) { return stft_exec(pl, a, RowSink{}); }
 
 int spx_stft_exec_persistence(spx_plan* pl, spx_stft_args* a, uint32_t* counts) {
     if (!counts) return spx_set_error(SPX_E_INVALID, "counts is NULL");
-    return stft_exec(pl, a, counts, nullptr);
+    return stft_exec(pl, a, RowSink{(char*)counts, nullptr});
 }
 
 // K, B and the mode of a pooled call or its finalisation
@@ -959,8 +895,8 @@ int spx_stft_exec_pooled(spx_plan* pl, spx_stft_args* a, spx_pool_args* p) {
     SPX_TRY(check_pool_shape(pl, p->mode, p->frames_per_row, p->bins_per_col));
     if (p->first_frame < 0 || p->n_rows < 0) return spx_set_error(SPX_E_INVALID, "first_frame and n_rows must be >= 0");
     if (!p->acc) return spx_set_error(SPX_E_INVALID, "acc is NULL");
-    const PoolCall pc{p->mode, p->frames_per_row, p->bins_per_col, p->first_frame, p->n_rows, p->acc};
-    return stft_exec(pl, a, nullptr, &pc);
+    const PoolCall pc{p->mode, p->frames_per_row, p->bins_per_col, p->first_frame, p->n_rows};
+    return stft_exec(pl, a, RowSink{(char*)p->acc, &pc});
 }
 
 int spx_pool_finalize(spx_plan* pl, int32_t mem, int32_t mode, const double* acc, int32_t n_streams, int64_t n_rows,

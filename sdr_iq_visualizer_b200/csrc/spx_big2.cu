@@ -250,18 +250,17 @@ int big2_plan_init(spx_plan* pl) {
 
 // K2v2 handles: cf32 or ci16 input, N = 65536, hop a multiple of 256 samples, 16-byte aligned stream start, outputs among
 // {uint8 rows, Welch sum, max-hold}.  Everything else goes through the two-kernel path of spx_bigfft.cu.
-bool big2_eligible(const spx_plan* pl, const void* in, const float* db_rows, const float2* spec_rows) {
+bool big2_eligible(const spx_plan* pl, const void* in, const StftOut& out) {
     if (pl->cfg.nfft != BIG2_N || pl->d_big2 == nullptr) return false;
     if (pl->cfg.variant == 1) return false;                    // variant 1 = the round-1 two-kernel path, kept for comparison
-    if (db_rows != nullptr || spec_rows != nullptr) return false;
+    if (out.db != nullptr || out.spec != nullptr) return false;
     if (pl->cfg.hop % 256 != 0 || ((uintptr_t)in & 15u) != 0) return false;
     return tmap_encoder() != nullptr;
 }
 
-int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, unsigned char* wf_rows, double* welch_acc,
-                       float* maxhold, float vmin, float vmax, cudaStream_t st, int sys_atomics) {
+int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out, cudaStream_t st) {
     if (frames <= 0) return SPX_OK;
-    const bool acc = welch_acc != nullptr || maxhold != nullptr;
+    const bool acc = out.welch != nullptr || out.maxhold != nullptr;
     const bool ci16 = pl->cfg.in_fmt == SPX_FMT_CI16;
     auto k_acc = ci16 ? big2_kernel<true, FMT_CI16> : big2_kernel<true, FMT_CF32>;
     auto k_rows = ci16 ? big2_kernel<false, FMT_CI16> : big2_kernel<false, FMT_CF32>;
@@ -298,14 +297,14 @@ int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long
     p.done = (int*)((char*)pl->st_big.ptr + scratch_bytes);
     p.frames = frames;
     p.row0 = row0;
-    p.wf_rows = wf_rows;
-    p.welch_acc = welch_acc;
-    p.maxhold = maxhold;
+    p.wf_rows = out.wf;
+    p.welch_acc = out.welch;
+    p.maxhold = out.maxhold;
     p.db_eps = pl->cfg.db_eps;
-    p.db_pw_min = pl->cfg.db_eps * pl->cfg.db_eps * 1099511627776.0f;
-    p.q_a = (float)(3.01029995663981195214 * 256.0 / ((double)vmax - (double)vmin));
-    p.q_b = (float)(-(double)vmin * 256.0 / ((double)vmax - (double)vmin));
-    p.sys_atomics = sys_atomics;
+    p.db_pw_min = db_pw_min(pl);
+    p.q_a = out.q_a();
+    p.q_b = out.q_b();
+    p.sys_atomics = out.sys_atomics;
     p.in_row0 = 0;
     p.hop_rows = pl->cfg.hop / 256;
     p.lanes = (int)lanes;

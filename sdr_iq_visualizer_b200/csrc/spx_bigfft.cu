@@ -482,12 +482,10 @@ static int big_launch_pair_t(spx_plan* pl, BigParams& p, cudaStream_t st, bool a
 }
 
 // one stream, frames [0, frames): batches of frames through the L2-sized scratch
-int bigfft_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,
-                         unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold, float vmin,
-                         float vmax, cudaStream_t st, int sys_atomics) {
+int bigfft_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out, cudaStream_t st) {
     const int n = pl->cfg.nfft;
-    if (big2_eligible(pl, in, db_rows, spec_rows))   // config-5 shape: one persistent kernel, scratch stays in L2
-        return big2_launch_stream(pl, in, frames, row0, wf_rows, welch_acc, maxhold, vmin, vmax, st, sys_atomics);
+    if (big2_eligible(pl, in, out))   // config-5 shape: one persistent kernel, scratch stays in L2
+        return big2_launch_stream(pl, in, frames, row0, out, st);
     const size_t frame_bytes = (size_t)n * sizeof(float2);
     // two halves of the scratch: the column kernel of batch k+1 (aux stream) runs next to the row kernel of batch k, so
     // the tail wave of one kernel is filled by the other instead of leaving SMs idle
@@ -509,16 +507,16 @@ int bigfft_launch_stream(spx_plan* pl, const void* in, long long frames, long lo
     p.tw2 = pl->d_tw2;
     p.wn_fine = pl->d_wn_fine;
     p.wn_coarse = pl->d_wn_coarse;
-    p.db_rows = db_rows;
-    p.wf_rows = wf_rows;
-    p.spec_rows = spec_rows;
-    p.welch_acc = welch_acc;
-    p.maxhold = maxhold;
+    p.db_rows = out.db;
+    p.wf_rows = out.wf;
+    p.spec_rows = out.spec;
+    p.welch_acc = out.welch;
+    p.maxhold = out.maxhold;
     p.db_eps = pl->cfg.db_eps;
-    p.db_pw_min = pl->cfg.db_eps * pl->cfg.db_eps * 1099511627776.0f;
-    p.q_a = (float)(3.01029995663981195214 * 256.0 / ((double)vmax - (double)vmin));
-    p.q_b = (float)(-(double)vmin * 256.0 / ((double)vmax - (double)vmin));
-    p.sys_atomics = sys_atomics;
+    p.db_pw_min = db_pw_min(pl);
+    p.q_a = out.q_a();
+    p.q_b = out.q_b();
+    p.sys_atomics = out.sys_atomics;
     if (two) {   // everything already queued on st (accumulator memsets, the previous call) comes first
         SPX_CUDA(cudaEventRecord(pl->ev_big[0], st));
         SPX_CUDA(cudaStreamWaitEvent(pl->s_big_aux, pl->ev_big[0], 0));

@@ -166,9 +166,8 @@ int bluestein_plan_init(spx_plan* pl) {
     return SPX_OK;
 }
 
-int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,
-                            unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold, float vmin,
-                            float vmax, cudaStream_t st, int sys_atomics) {
+int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out,
+                            cudaStream_t st) {
     const int n = pl->cfg.nfft, m = pl->blu_m;
     const size_t frame_bytes = (size_t)m * sizeof(float2);
     long long fb = (long long)((128u << 20) / frame_bytes);
@@ -186,17 +185,19 @@ int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long
     p.bspec = pl->d_blu + 2 * n;
     p.buf_a = (float2*)pl->st_big.ptr;
     p.buf_b = p.buf_a + (size_t)fb * m;
-    p.db_rows = db_rows;
-    p.wf_rows = wf_rows;
-    p.spec_rows = spec_rows;
-    p.welch_acc = welch_acc;
-    p.maxhold = maxhold;
+    p.db_rows = out.db;
+    p.wf_rows = out.wf;
+    p.spec_rows = out.spec;
+    p.welch_acc = out.welch;
+    p.maxhold = out.maxhold;
     p.db_eps = pl->cfg.db_eps;
-    p.q_a = (float)(3.01029995663981195214 * 256.0 / ((double)vmax - (double)vmin));
-    p.q_b = (float)(-(double)vmin * 256.0 / ((double)vmax - (double)vmin));
-    p.sys_atomics = sys_atomics;
-    const bool acc = welch_acc != nullptr || maxhold != nullptr;
+    p.q_a = out.q_a();
+    p.q_b = out.q_b();
+    p.sys_atomics = out.sys_atomics;
+    const bool acc = out.welch != nullptr || out.maxhold != nullptr;
     const int sms = pl->sm_count;
+    StftOut inner;   // the inner power-of-two transform: spectrum rows in buf_b
+    inner.spec = p.buf_b;
     for (long long f0 = 0; f0 < frames; f0 += fb) {
         p.frames = (int)(frames - f0 < fb ? frames - f0 : fb);
         p.sample0 = f0 * pl->cfg.hop;
@@ -206,10 +207,10 @@ int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long
         if (pl->cfg.in_fmt == SPX_FMT_CF32) blu_pre_kernel<FMT_CF32><<<g1, 256, 0, st>>>(p);
         else blu_pre_kernel<FMT_CI16><<<g1, 256, 0, st>>>(p);
         SPX_CUDA(cudaGetLastError());
-        SPX_TRY(stft_launch_device(pl->blu_inner, p.buf_a, 1, 0, p.frames, nullptr, nullptr, p.buf_b, nullptr, nullptr, 0.f, 1.f, st, 0));
+        SPX_TRY(stft_launch_device(pl->blu_inner, p.buf_a, 1, 0, p.frames, inner, st));
         blu_mul_kernel<<<g1, 256, 0, st>>>(p);
         SPX_CUDA(cudaGetLastError());
-        SPX_TRY(stft_launch_device(pl->blu_inner, p.buf_a, 1, 0, p.frames, nullptr, nullptr, p.buf_b, nullptr, nullptr, 0.f, 1.f, st, 0));
+        SPX_TRY(stft_launch_device(pl->blu_inner, p.buf_a, 1, 0, p.frames, inner, st));
         const int bx = (n + 255) / 256;
         int chunks = (sms * 8 + bx - 1) / bx;
         if (chunks > p.frames) chunks = p.frames;

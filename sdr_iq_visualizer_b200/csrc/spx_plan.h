@@ -37,9 +37,9 @@ struct spx_plan {
     size_t pool_rows_bytes = 256u << 20;    // float dB row buffer of a pooled call without caller dB rows (measured, DESIGN.md K8)
     // staging for SPX_MEM_HOST execution (grow-only)
     spx::DevBuf st_in, st_db, st_wf, st_spec, st_welch, st_max, st_misc, st_flush;
-    // persistence spectrum / pooled spectrogram: counts and accumulator staging of the host path, and the plan-owned row
-    // buffer (uint8 levels or float dB rows; device path without caller rows; host path without caller rows, one piece)
-    spx::DevBuf st_counts, st_pool, st_rows;
+    // persistence spectrum / pooled spectrogram: counts or pooled accumulator staging of the host path, and the plan-owned
+    // row buffer (uint8 levels or float dB rows; device path without caller rows; host path without caller rows, one piece)
+    spx::DevBuf st_sink, st_rows;
     // large-N (four-step) path, nfft >= 16384
     int big_n1 = 0, big_n2 = 0;
     float2* d_big_tw = nullptr;  // one allocation holding the four tables below
@@ -70,37 +70,66 @@ int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out);
 bool plan_has_scratch(const spx_plan* pl);
 int scratch_wait(spx_plan* pl, cudaStream_t st);
 int scratch_record(spx_plan* pl, cudaStream_t st);
+
+// Outputs of an STFT launch, in device memory: rows [r][N] (dB, uint8 levels, spectrum) and accumulators [s][N] (Welch
+// sums, max-hold).  A null member is not produced.  vmin / vmax set the uint8 levels; sys_atomics makes the accumulator
+// flushes system-scope (accumulators on another GPU).
+struct StftOut {
+    float* db = nullptr;
+    unsigned char* wf = nullptr;
+    float2* spec = nullptr;
+    double* welch = nullptr;
+    float* maxhold = nullptr;
+    float vmin = 0.f, vmax = 1.f;
+    int sys_atomics = 0;
+    bool has_rows() const { return db || wf || spec; }
+    // the rows from row r0 on, or the accumulators of stream s, of rows of N bins; null members stay null
+    StftOut rows_at(size_t r0, size_t N) const {
+        StftOut o = *this;
+        if (db) o.db = db + r0 * N;
+        if (wf) o.wf = wf + r0 * N;
+        if (spec) o.spec = spec + r0 * N;
+        return o;
+    }
+    StftOut stream_at(long long s, size_t N) const {
+        StftOut o = *this;
+        if (welch) o.welch = welch + (size_t)s * N;
+        if (maxhold) o.maxhold = maxhold + (size_t)s * N;
+        return o;
+    }
+    // the row epilogue's uint8 level = q_a * log2(power) + q_b
+    float q_a() const { return (float)(3.01029995663981195214 * 256.0 / ((double)vmax - (double)vmin)); }  // 10 log10(2) * scale
+    float q_b() const { return (float)(-(double)vmin * 256.0 / ((double)vmax - (double)vmin)); }
+};
+// the row epilogue's power floor, (2^20 eps)^2
+inline float db_pw_min(const spx_plan* pl) { return pl->cfg.db_eps * pl->cfg.db_eps * 1099511627776.0f; }
+
 int stft_launch_device(spx_plan* pl, const void* in, long long n_streams, long long stream_stride, long long frames,
-                       float* db_rows, unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold,
-                       float vmin, float vmax, cudaStream_t st, int sys_atomics = 0);
+                       const StftOut& out, cudaStream_t st);
 int bigfft_plan_init(spx_plan* pl);
-int bigfft_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,
-                         unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold, float vmin,
-                         float vmax, cudaStream_t st, int sys_atomics = 0);
+int bigfft_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out, cudaStream_t st);
 int peer_reduce_launch(const double* w_local, const float* m_local, double* w_peer, float* m_peer, long long n, cudaStream_t st);
 int big2_plan_init(spx_plan* pl);
-bool big2_eligible(const spx_plan* pl, const void* in, const float* db_rows, const float2* spec_rows);
-int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, unsigned char* wf_rows, double* welch_acc,
-                       float* maxhold, float vmin, float vmax, cudaStream_t st, int sys_atomics);
+bool big2_eligible(const spx_plan* pl, const void* in, const StftOut& out);
+int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out, cudaStream_t st);
 int persist_launch(const spx_plan* pl, const uint8_t* rows, long long n_streams, long long frames, uint32_t* counts,
                    cudaStream_t st);
-// a pooled call (spx_pool_args, checked); acc is [S][n_rows][nfft / bins_per_col] in the call's memory space
+// a pooled call (spx_pool_args, checked)
 struct PoolCall {
     int mode;
     long long frames_per_row;
     int bins_per_col;
     long long first_frame, n_rows;
-    double* acc;
 };
-int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long long rows_per_stream, long long frames,
-                long long frame0, const PoolCall& pc, double* acc, cudaStream_t st);
+// rows [n_streams][frames][nfft] into acc [n_streams][n_rows][nfft / bins_per_col]; frame0: global index of frame 0
+int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long long frames, long long frame0,
+                const PoolCall& pc, double* acc, cudaStream_t st);
 int pool_fill_launch(double* acc, long long n, int mode, cudaStream_t st);
 int pool_finalize_launch(const spx_plan* pl, const double* acc, long long n_streams, long long G, long long F_total,
                          long long K, int B, int mode, float vmin, float vmax, float* db_out, uint8_t* wf_out,
                          cudaStream_t st);
 int welch_finalize_launch(const double* acc, int n, double inv_norm, double* pxx, double* pxx_db, cudaStream_t st);
 int bluestein_plan_init(spx_plan* pl);
-int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, float* db_rows,
-                            unsigned char* wf_rows, float2* spec_rows, double* welch_acc, float* maxhold, float vmin,
-                            float vmax, cudaStream_t st, int sys_atomics = 0);
+int bluestein_launch_stream(spx_plan* pl, const void* in, long long frames, long long row0, const StftOut& out,
+                            cudaStream_t st);
 }  // namespace spx

@@ -161,8 +161,8 @@ int pool_finalize_launch(const spx_plan* pl, const double* acc, long long n_stre
 
 // Frames per chunk: enough chunks for about 2048 threads per SM (two waves of the four CTAs an SM holds), at least
 // POOL_MIN_ROWS rows each.
-int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long long rows_per_stream, long long frames,
-                long long frame0, const PoolCall& pc, double* acc, cudaStream_t st) {
+int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long long frames, long long frame0,
+                const PoolCall& pc, double* acc, cudaStream_t st) {
     if (frames <= 0 || n_streams <= 0) return SPX_OK;
     const int N = pl->cfg.nfft, B = pc.bins_per_col;
     const int threads = (N + 3) / 4 >= POOL_THREADS ? POOL_THREADS : (((N + 3) / 4 + 31) / 32) * 32;
@@ -187,13 +187,13 @@ int pool_launch(const spx_plan* pl, const float* rows, long long n_streams, long
     for (long long g0 = 0; g0 < n_streams; g0 += group) {
         const long long ng = n_streams - g0 < group ? n_streams - g0 : group;
         dim3 grid((unsigned)strips, (unsigned)(ng * chunks));
-        const float* r = rows + (size_t)(g0 * rows_per_stream) * N;
+        const float* r = rows + (size_t)(g0 * frames) * N;
         double* a = acc + (size_t)(g0 * pc.n_rows) * C;
         if (pc.mode == SPX_POOL_MAX)
-            pool_kernel<true><<<grid, threads, 0, st>>>(r, rows_per_stream, frames, N, B, pc.frames_per_row, frame0, per,
+            pool_kernel<true><<<grid, threads, 0, st>>>(r, frames, frames, N, B, pc.frames_per_row, frame0, per,
                                                         (int)chunks, vec, lanes, pl->cfg.db_eps, a, pc.n_rows);
         else
-            pool_kernel<false><<<grid, threads, 0, st>>>(r, rows_per_stream, frames, N, B, pc.frames_per_row, frame0, per,
+            pool_kernel<false><<<grid, threads, 0, st>>>(r, frames, frames, N, B, pc.frames_per_row, frame0, per,
                                                          (int)chunks, vec, lanes, pl->cfg.db_eps, a, pc.n_rows);
         SPX_CUDA(cudaGetLastError());
     }

@@ -214,7 +214,8 @@ extern "C" int spx_ring_commit(spx_ring* r, int64_t n_samples) {
     // commit must wait for the slot's kernels
     const bool scratch = plan_has_scratch(pl);
     if (scratch) SPX_TRY(scratch_wait(pl, pl->s_compute));
-    SPX_TRY(stft_launch_device(pl, s.d_in, 1, 0, F, s.d_db, s.d_wf, nullptr, s.d_welch, s.d_max, r->cfg.vmin, r->cfg.vmax, pl->s_compute));
+    SPX_TRY(stft_launch_device(pl, s.d_in, 1, 0, F, StftOut{s.d_db, s.d_wf, nullptr, s.d_welch, s.d_max, r->cfg.vmin, r->cfg.vmax},
+                               pl->s_compute));
     SPX_CUDA(cudaEventRecord(s.e_stft, pl->s_compute));   // the rows are complete here: their copy does not wait for the measurements
     // classifier measurements of this slot's Welch block, right behind the STFT kernel on the same stream
     const bool feats = s.d_feat != nullptr && F > 0;

@@ -173,7 +173,15 @@ typedef struct {
     int32_t in_fmt;   /* SPX_FMT_* */
     float in_scale;   /* multiplies every sample: 1.0 stream path, 2^-15 SigMF ci16_le */
     float db_eps;     /* dB rows are 20*log10(|X| + db_eps); reference 1e-12 (streamer.py:121) */
-    int32_t variant;  /* kernel tuning variant, 0 = default */
+    int32_t variant;  /* kernel selection; spx_plan_create rejects any other value with SPX_E_INVALID.  The non-zero
+                       * values force a path the default also takes for some inputs, as a reference to test against;
+                       * for lengths they do not concern they behave like 0.
+                       *   0: the default (fastest measured kernel per shape)
+                       *   1: N = 65536: the two-kernel four-step path instead of the single-kernel one
+                       *  12: N = 1024 / 2048 / 4096: K1, the kernel the default uses for frames that are not 128-byte
+                       *      aligned, for every input
+                       *  22: N = 1024 / 2048 / 4096, aligned frames: the generic K1v2 kernel, without strip staging,
+                       *      L2 prefetch or the kernels specialised to one set of row outputs */
     int32_t reserved;
 } spx_plan_config;
 

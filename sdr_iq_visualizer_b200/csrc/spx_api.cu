@@ -629,6 +629,8 @@ int spx_plan_create(spx_plan** out, const spx_plan_config* cfg) {
     if (cfg->hop < 1 || cfg->hop > cfg->nfft) return spx_set_error(SPX_E_INVALID, "hop %d must be in [1, nfft]", cfg->hop);
     if (cfg->window < 0 || cfg->window > 2) return spx_set_error(SPX_E_INVALID, "unknown window %d", cfg->window);
     if (cfg->in_fmt != SPX_FMT_CF32 && cfg->in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt %d", cfg->in_fmt);
+    if (cfg->variant != 0 && cfg->variant != 1 && cfg->variant != 12 && cfg->variant != 22)
+        return spx_set_error(SPX_E_INVALID, "unknown variant %d: accepted values are 0, 1, 12 and 22 (see spx.h)", cfg->variant);
     int ndev = 0;
     SPX_TRY(spx_device_count(&ndev));
     if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");

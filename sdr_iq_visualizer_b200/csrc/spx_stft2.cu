@@ -42,47 +42,28 @@ static int launch_fmt_outs(StftLaunch& L) {
 }
 
 int launch_stft2(StftLaunch& L) {
-    if (L.variant == 23) {   // strip staging of overlapping frames (experiment; N = 4096, hop = N/2 or N/4), else the default
-        int rc = SPX_OK;
-        if (launch_stft2_strip<2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L, &rc)) return rc;
-        return launch_stft2_n<4096, 2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L);
+    // FMA-form DFTs + uint8 index on the FMA / ALU pipes instead of F2I (XU)
+    constexpr int T0 = TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA;
+    if (L.variant == 22) {   // the generic T0 kernel alone: the reference the strip kernel is tested against
+        switch (L.nfft) {
+            case 1024: return launch_stft2_n<1024, 2, T0>(L);
+            case 2048: return launch_stft2_n<2048, 2, T0>(L);
+            case 4096: return launch_stft2_n<4096, 2, T0>(L);
+        }
     }
-    if (L.variant == 0 && L.nfft == 4096 && L.in_fmt == FMT_CF32 && L.p.hop == 1024) {
+    if (L.nfft == 4096 && L.in_fmt == FMT_CF32 && L.p.hop == 1024) {
         // measured (profiles/r02_strip_staging_sweep.jsonl): strip staging wins 3 % on cf32 at 75 % overlap (the frame is
         // 32 KB, three quarters of it already in shared memory), is neutral for ci16 and at 50 % overlap -- used only here
-        int rc = SPX_OK;
-        if (launch_stft2_strip<2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L, &rc)) return rc;
+        return launch_stft2_strip<T0>(L);
     }
-    if (L.variant == 0) {
-        constexpr int T0 = TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA;
-        // L2 prefetch of the next frame (compile-time as well): cf32, N = 4096 without overlap only (+ 5 %,
-        // profiles/r02_l2_prefetch_sweep.txt; neutral for int16, - 1 % with overlap, - 3 % for N = 2048 / 1024 with their 2 / 4
-        // frames in flight per CTA)
-        if (L.nfft == 4096 && L.in_fmt == FMT_CF32 && L.p.hop >= 4096) return launch_outs<4096, FMT_CF32, T0 | TUNE_L2PF>(L);
-        switch (L.nfft) {
-            case 1024: return launch_fmt_outs<1024, T0>(L);
-            case 2048: return launch_fmt_outs<2048, T0>(L);
-            case 4096: return launch_fmt_outs<4096, T0>(L);
-        }
-    }
-    if (L.variant == 22 || L.variant == 0) {   // default: FMA-form DFTs + uint8 index on the FMA / ALU pipes instead of F2I (XU)
-        switch (L.nfft) {
-            case 1024: return launch_stft2_n<1024, 2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L);
-            case 2048: return launch_stft2_n<2048, 2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L);
-            case 4096: return launch_stft2_n<4096, 2, TUNE_I2FP | TUNE_FMADFT | TUNE_QFMA>(L);
-        }
-    }
-    if (L.variant == 21) {   // radix-16 DFTs in fused-multiply-add form (dft16_fma)
-        switch (L.nfft) {
-            case 1024: return launch_stft2_n<1024, 2, TUNE_I2FP | TUNE_FMADFT>(L);
-            case 2048: return launch_stft2_n<2048, 2, TUNE_I2FP | TUNE_FMADFT>(L);
-            case 4096: return launch_stft2_n<4096, 2, TUNE_I2FP | TUNE_FMADFT>(L);
-        }
-    }
+    // L2 prefetch of the next frame (compile-time as well): cf32, N = 4096 without overlap only (+ 5 %,
+    // profiles/r02_l2_prefetch_sweep.txt; neutral for int16, - 1 % with overlap, - 3 % for N = 2048 / 1024 with their 2 / 4
+    // frames in flight per CTA)
+    if (L.nfft == 4096 && L.in_fmt == FMT_CF32 && L.p.hop >= 4096) return launch_outs<4096, FMT_CF32, T0 | TUNE_L2PF>(L);
     switch (L.nfft) {
-        case 1024: return launch_stft2_n<1024, 2, TUNE_I2FP>(L);
-        case 2048: return launch_stft2_n<2048, 2, TUNE_I2FP>(L);
-        case 4096: return launch_stft2_n<4096, 2, TUNE_I2FP>(L);
+        case 1024: return launch_fmt_outs<1024, T0>(L);
+        case 2048: return launch_fmt_outs<2048, T0>(L);
+        case 4096: return launch_fmt_outs<4096, T0>(L);
         default: return spx_set_error(SPX_E_UNSUPPORTED, "K1v2 handles nfft 1024 / 2048 / 4096, not %d", L.nfft);
     }
 }

@@ -128,7 +128,7 @@ __global__ void __launch_bounds__(256, OCC) stft2_kernel(const StftParams p, con
     }
 }
 
-// ------------------------------------------------------------------ strip-staging variant (experiment, variant 23)
+// ------------------------------------------------------------------ strip staging of overlapping frames
 // N = 4096, hop = N / R: only the newest hop block of a frame crosses L2 -> shared memory (north_star: "TMA /
 // shared-memory staging of overlapping frames").  Same arithmetic and data flow as stft2_kernel otherwise.
 template <int FMT, bool ACC, int R, int OCC, int TUNE>
@@ -324,20 +324,11 @@ int launch_stft2_strip_inst(StftLaunch& L) {
     return SPX_OK;
 }
 
-// variant 23: strip staging, N = 4096 and hop = N/2 or N/4 only (false: not applicable, the caller takes the default kernel)
-template <int OCC, int TUNE>
-bool launch_stft2_strip(StftLaunch& L, int* rc) {
-    if (L.nfft != 4096 || (L.p.hop != 1024 && L.p.hop != 2048)) return false;
+// strip staging as the default uses it: cf32, N = 4096, hop = N/4 (the caller checks the shape)
+template <int TUNE>
+int launch_stft2_strip(StftLaunch& L) {
     const bool acc = L.p.welch_acc != nullptr || L.p.maxhold != nullptr;
-    const bool cf = L.in_fmt == FMT_CF32;
-    if (L.p.hop == 1024) {
-        *rc = cf ? (acc ? launch_stft2_strip_inst<FMT_CF32, true, 4, OCC, TUNE>(L) : launch_stft2_strip_inst<FMT_CF32, false, 4, OCC, TUNE>(L))
-                 : (acc ? launch_stft2_strip_inst<FMT_CI16, true, 4, OCC, TUNE>(L) : launch_stft2_strip_inst<FMT_CI16, false, 4, OCC, TUNE>(L));
-    } else {
-        *rc = cf ? (acc ? launch_stft2_strip_inst<FMT_CF32, true, 2, OCC, TUNE>(L) : launch_stft2_strip_inst<FMT_CF32, false, 2, OCC, TUNE>(L))
-                 : (acc ? launch_stft2_strip_inst<FMT_CI16, true, 2, OCC, TUNE>(L) : launch_stft2_strip_inst<FMT_CI16, false, 2, OCC, TUNE>(L));
-    }
-    return true;
+    return acc ? launch_stft2_strip_inst<FMT_CF32, true, 4, 2, TUNE>(L) : launch_stft2_strip_inst<FMT_CF32, false, 4, 2, TUNE>(L);
 }
 
 template <int N, int OCC, int TUNE>

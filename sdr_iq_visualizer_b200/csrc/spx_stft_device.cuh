@@ -13,7 +13,7 @@
 namespace spx {
 
 enum { FMT_CF32 = 0, FMT_CI16 = 1 };
-enum { TW_LDG = 0, TW_REG = 1, TW_SMEM = 2, TW_HYB = 3 };  // HYB: pass 1 from a small smem table, later passes from register bases
+enum { TW_LDG = 0, TW_REG = 1, TW_SMEM = 2 };
 
 struct StftParams {
     const void* in;              // cf32 (float2) or ci16 (short2) samples
@@ -413,8 +413,8 @@ SPX_HD void stft_phase(float2* v, int tid, const StftParams& p, long long sample
     } else {
         const float2* src = ((S - 1) & 1) ? bufB : bufA;
         pass_load_smem<N, S>(v, tid, src);
-        if constexpr (TWM == TW_REG || (TWM == TW_HYB && S > 1)) pass_twiddle_regs<N, S>(v, twr);
-        else pass_twiddle_table<N, S, TWM == TW_SMEM || TWM == TW_HYB>(v, tid, tw);
+        if constexpr (TWM == TW_REG) pass_twiddle_regs<N, S>(v, twr);
+        else pass_twiddle_table<N, S, TWM == TW_SMEM>(v, tid, tw);
     }
     pass_dft<N, S>(v);
     if constexpr (S == P - 1) {

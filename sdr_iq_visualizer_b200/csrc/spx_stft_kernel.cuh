@@ -91,10 +91,10 @@ __global__ void __launch_bounds__(StftCfg<N>::THREADS, OCC) stft_kernel(const St
             win_half = wsm;
         }
     }
-    constexpr int TW_SMEM_F2 = TWM == TW_SMEM ? C::TW_F2 : (TWM == TW_HYB ? plan_tw_offset(N, 2) : 0);
-    if constexpr (TW_SMEM_F2 > 0 && P > 1) {
+    constexpr bool TW_IN_SMEM = TWM == TW_SMEM && P > 1;
+    if constexpr (TW_IN_SMEM) {
         float2* tws = smem + C::FPC * C::slot_f2(STAGE, FMT) + C::win_f2(STAGE);
-        for (int i = threadIdx.x; i < TW_SMEM_F2; i += C::THREADS) tws[i] = __ldg(p.tw + i);
+        for (int i = threadIdx.x; i < C::TW_F2; i += C::THREADS) tws[i] = __ldg(p.tw + i);
         tw = tws;
     }
     const unsigned bar_u32 = smem_u32(&mbar[STAGE ? slot : 0]);
@@ -103,11 +103,11 @@ __global__ void __launch_bounds__(StftCfg<N>::THREADS, OCC) stft_kernel(const St
         if (tid == 0) mbar_init(bar_u32, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if constexpr (STAGE || (TW_SMEM_F2 > 0 && P > 1)) __syncthreads();
+    if constexpr (STAGE || TW_IN_SMEM) __syncthreads();
 
     TwRegs<N> twr;
-    if constexpr ((TWM == TW_REG || TWM == TW_HYB) && P > 1) {
-        if constexpr (P > 1 && TWM == TW_REG) tw_regs_load_pass<N, 1>(twr, tid, p.tw);
+    if constexpr (TWM == TW_REG && P > 1) {
+        tw_regs_load_pass<N, 1>(twr, tid, p.tw);
         if constexpr (P > 2) tw_regs_load_pass<N, 2>(twr, tid, p.tw);
         if constexpr (P > 3) tw_regs_load_pass<N, 3>(twr, tid, p.tw);
     }
@@ -178,117 +178,12 @@ __global__ void __launch_bounds__(StftCfg<N>::THREADS, OCC) stft_kernel(const St
     }
 }
 
-// ------------------------------------------------------------------ software-pipelined variant (rows only)
-// K1 is limited by how well the FMA pipe stays busy while warps sit in their shared-memory exchange phases (two
-// barrier-coupled CTAs per SM).  For three-pass plans without accumulators there are registers to spare, so this
-// variant overlaps frame f+1's first pass (staged input -> window -> radix-16 DFT, no dependence on frame f) with the
-// latency of frame f's first exchange: the exchange barriers are split-phase mbarriers (arrive, independent work,
-// wait) instead of bar.sync.
-__device__ __forceinline__ FrameCursor next_frame(const FrameCursor& c, const StftParams& p, unsigned n_workers) {
-    FrameCursor n = c;
-    if (c.fi + 1 < c.nf) n.fi = c.fi + 1;
-    else n.seek(p, c.chunk + n_workers);
-    return n;
-}
-
-template <int N, int FMT, int OCC, int TUNE>
-__global__ void __launch_bounds__(StftCfg<N>::THREADS, OCC) stft_kernel_pipe(const StftParams p) {
-    using C = StftCfg<N>;
-    static_assert(C::P == 3 && C::FPC == 1, "pipelined variant: three passes, one frame per CTA");
-    constexpr unsigned FRAME_BYTES = (unsigned)N * (FMT == FMT_CF32 ? 8u : 4u);
-    constexpr int ELT = FMT == FMT_CF32 ? 8 : 4;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ unsigned long long mbar[3];   // 0: TMA of the staged frame, 1 / 2: the two exchanges
-    float2* smem = reinterpret_cast<float2*>(smem_raw);
-    const int tid = threadIdx.x;
-    void* stage = (void*)smem;
-    float2* bufA = smem + (FMT == FMT_CF32 ? N : N / 2);
-    float2* bufB = bufA + padded_size(N);
-    const float* win_half = nullptr;
-    if (p.win != nullptr) {
-        float* wsm = reinterpret_cast<float*>(smem + C::slot_f2(true, FMT));
-        for (int i = tid; i < N / 2; i += C::THREADS) wsm[i] = __ldg(p.win + i);
-        win_half = wsm;
-    }
-    const unsigned bar_tma = smem_u32(&mbar[0]), bar_e0 = smem_u32(&mbar[1]), bar_e1 = smem_u32(&mbar[2]);
-    const unsigned stage_u32 = smem_u32(smem);
-    if (tid == 0) {
-        mbar_init(bar_tma, 1);
-        mbar_init(bar_e0, C::THREADS / 32);   // one arrival per warp (elected lane after __syncwarp)
-        mbar_init(bar_e1, C::THREADS / 32);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-
-    TwRegs<N> twr;
-    tw_regs_load_pass<N, 1>(twr, tid, p.tw);
-    tw_regs_load_pass<N, 2>(twr, tid, p.tw);
-    StftAcc<false> acc;
-    acc.reset();
-
-    const unsigned n_workers = gridDim.x;
-    const char* in_bytes = reinterpret_cast<const char*>(p.in);
-    FrameCursor cur;
-    cur.seek(p, blockIdx.x);
-    if (!cur.valid) return;
-    auto issue_tma = [&](const FrameCursor& c) {
-        if (tid == 0) {
-            mbar_expect_tx(bar_tma, FRAME_BYTES);
-            bulk_g2s(stage_u32, in_bytes + c.sample0(p) * ELT, FRAME_BYTES, bar_tma);
-        }
-    };
-    issue_tma(cur);
-    FrameCursor nxt = next_frame(cur, p, n_workers);
-    unsigned p_tma = 0, p_ex = 0;
-    float2 v[16], w[16];
-    mbar_wait(bar_tma, p_tma);
-    p_tma ^= 1u;
-    load_frame_staged<N, FMT, TUNE>(v, stage, win_half, tid);
-    pass_dft<N, 0>(v);
-    __syncthreads();                       // every thread has read the staged frame
-    if (nxt.valid) issue_tma(nxt);
-    while (true) {
-        const long long row = cur.row();
-        const bool has_next = nxt.valid;
-        pass_store_smem<N, 0>(v, tid, bufA);
-        __syncwarp();
-        if ((tid & 31) == 0) mbar_arrive(bar_e0);
-        if (has_next) {                    // independent of the exchange in flight: first pass of the next frame
-            mbar_wait(bar_tma, p_tma);
-            p_tma ^= 1u;
-            load_frame_staged<N, FMT, TUNE>(w, stage, win_half, tid);
-            pass_dft<N, 0>(w);
-        }
-        mbar_wait(bar_e0, p_ex);
-        pass_load_smem<N, 1>(v, tid, bufA);
-        pass_twiddle_regs<N, 1>(v, twr);
-        pass_dft<N, 1>(v);
-        pass_store_smem<N, 1>(v, tid, bufB);
-        __syncwarp();
-        if ((tid & 31) == 0) mbar_arrive(bar_e1);
-        FrameCursor nx2 = nxt;
-        if (has_next) nx2 = next_frame(nxt, p, n_workers);
-        mbar_wait(bar_e1, p_ex);
-        p_ex ^= 1u;
-        if (has_next && nx2.valid) issue_tma(nx2);   // every thread has read the staged next frame (it arrived at e1)
-        pass_load_smem<N, 2>(v, tid, bufB);
-        pass_twiddle_regs<N, 2>(v, twr);
-        pass_dft<N, 2>(v);
-        epilogue<N, false>(v, tid, p, row, acc);
-        if (!has_next) break;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) v[i] = w[i];
-        cur = nxt;
-        nxt = nx2;
-    }
-}
-
 // ------------------------------------------------------------------ host side
 struct StftLaunch {
     StftParams p;          // chunking fields are filled in by the launcher
     int nfft;
     int in_fmt;
-    int variant;           // tuning variant (0 = default)
+    int variant;           // spx_plan_config.variant: 0, or 12 / 22 to force K1 / the generic K1v2 kernel
     int sm_count;
     long long total_frames;  // n_streams * F
     cudaStream_t stream;
@@ -300,7 +195,6 @@ int launch_stft_inst(StftLaunch& L) {
     auto kern = stft_kernel<N, FMT, ACC, TWM, OCC, STAGE, TUNE>;
     size_t smem = (size_t)(C::FPC * C::slot_f2(STAGE, FMT) + C::win_f2(STAGE)) * sizeof(float2);
     if (TWM == TW_SMEM) smem += (size_t)C::TW_F2 * sizeof(float2);
-    if (TWM == TW_HYB) smem += (size_t)plan_tw_offset(N, 2) * sizeof(float2);
     static int occ_cache[64] = {0};  // per instantiation, per device (benign race: same value)
     int dev = 0;
     SPX_CUDA(cudaGetDevice(&dev));
@@ -328,37 +222,6 @@ int launch_stft_inst(StftLaunch& L) {
     long long grid = (L.p.total_chunks + C::FPC - 1) / C::FPC;
     const long long grid_max = (long long)L.sm_count * occ;
     if (grid > grid_max) grid = grid_max;
-    if (grid < 1) grid = 1;
-    kern<<<(unsigned)grid, C::THREADS, smem, L.stream>>>(L.p);
-    SPX_CUDA(cudaGetLastError());
-    return SPX_OK;
-}
-
-template <int N, int FMT, int OCC, int TUNE>
-int launch_stft_pipe_inst(StftLaunch& L) {
-    using C = StftCfg<N>;
-    auto kern = stft_kernel_pipe<N, FMT, OCC, TUNE>;
-    const size_t smem = (size_t)(C::slot_f2(true, FMT) + C::win_f2(true)) * sizeof(float2);
-    static int occ_cache[64] = {0};
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    int occ = occ_cache[dev & 63];
-    if (occ == 0) {
-        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, C::THREADS, smem));
-        if (occ < 1) return spx_set_error(SPX_E_CUDA, "pipelined stft kernel does not fit on an SM");
-        occ_cache[dev & 63] = occ;
-    }
-    const long long workers_max = (long long)L.sm_count * occ;
-    const long long F = L.p.frames_per_stream;
-    long long per_worker = (L.total_frames + workers_max - 1) / workers_max;
-    long long fpc = per_worker < 1 ? 1 : per_worker;
-    if (fpc > F) fpc = F;
-    const long long cps = (F + fpc - 1) / fpc;
-    L.p.frames_per_chunk = (int)fpc;
-    L.p.chunks_per_stream = (int)cps;
-    L.p.total_chunks = cps * L.p.n_streams;
-    long long grid = L.p.total_chunks < workers_max ? L.p.total_chunks : workers_max;
     if (grid < 1) grid = 1;
     kern<<<(unsigned)grid, C::THREADS, smem, L.stream>>>(L.p);
     SPX_CUDA(cudaGetLastError());
@@ -397,7 +260,7 @@ int launch_stft_n(StftLaunch& L) {
 // one translation unit per size group instantiates these
 int launch_stft_small(StftLaunch& L);   // N = 16 .. 512
 int launch_stft_1k2k(StftLaunch& L);    // N = 1024, 2048
-int launch_stft_4k(StftLaunch& L);      // N = 4096 (+ tuning variants)
+int launch_stft_4k(StftLaunch& L);      // N = 4096
 int launch_stft_8k(StftLaunch& L);      // N = 8192
 
 }  // namespace spx

@@ -148,6 +148,15 @@ static int emul2_n(int fmt, bool acc, StftParams& p) {
     if (fmt == FMT_CF32) return acc ? emul_stft2<N, FMT_CF32, true, TUNE>(p) : emul_stft2<N, FMT_CF32, false, TUNE>(p);
     return acc ? emul_stft2<N, FMT_CI16, true, TUNE>(p) : emul_stft2<N, FMT_CI16, false, TUNE>(p);
 }
+template <int TUNE>
+static int emul2_nfft(int nfft, int fmt, bool acc, StftParams& p) {
+    switch (nfft) {
+        case 1024: return emul2_n<1024, TUNE>(fmt, acc, p);
+        case 2048: return emul2_n<2048, TUNE>(fmt, acc, p);
+        case 4096: return emul2_n<4096, TUNE>(fmt, acc, p);
+        default: return -4;
+    }
+}
 
 extern "C" int spx_emul_stft(int nfft, int in_fmt, int tw_mode, const void* in, long long n_samples, int n_streams,
                              long long stream_stride, int hop, const float* win, float db_eps, float vmin, float vmax,
@@ -175,14 +184,10 @@ extern "C" int spx_emul_stft(int nfft, int in_fmt, int tw_mode, const void* in, 
     p.chunks_per_stream = (int)((p.frames_per_stream + frames_per_chunk - 1) / frames_per_chunk);
     p.total_chunks = (long long)p.chunks_per_stream * n_streams;
     const bool acc = welch_acc != nullptr || maxhold != nullptr;
-    if (tw_mode & 0x20) {   // K1v2 phases
-        const bool fma = (tw_mode & 0x40) != 0;
-        switch (nfft) {
-            case 1024: return fma ? emul2_n<1024, TUNE_FMADFT | TUNE_QFMA>(in_fmt, acc, p) : emul2_n<1024, 0>(in_fmt, acc, p);
-            case 2048: return fma ? emul2_n<2048, TUNE_FMADFT | TUNE_QFMA>(in_fmt, acc, p) : emul2_n<2048, 0>(in_fmt, acc, p);
-            case 4096: return fma ? emul2_n<4096, TUNE_FMADFT | TUNE_QFMA>(in_fmt, acc, p) : emul2_n<4096, 0>(in_fmt, acc, p);
-            default: return -4;
-        }
+    if (tw_mode & 0x20) {   // K1v2 phases; 0x40: FMA-form DFTs + FMA-pipe colormap index, 0x80: FMA-form DFTs + F2I index
+        if (tw_mode & 0x40) return emul2_nfft<TUNE_FMADFT | TUNE_QFMA>(nfft, in_fmt, acc, p);
+        if (tw_mode & 0x80) return emul2_nfft<TUNE_FMADFT>(nfft, in_fmt, acc, p);
+        return emul2_nfft<0>(nfft, in_fmt, acc, p);
     }
     g_staged = (tw_mode & 0x10) != 0;
     tw_mode &= 0xf;

@@ -45,6 +45,27 @@ def test_no_cpu_fallback_without_gpu():
     assert classifier.classify_signal_advanced(np.array([]), np.array([]))["label"] == "No Data"
 
 
+def test_plan_create_accepts_only_the_documented_variants():
+    """spx_plan_config.variant is 0, 1, 12 or 22 for every nfft; any other value is refused with SPX_E_INVALID before a
+    device is looked for, so the check holds with or without a GPU."""
+    import ctypes as C
+    from sdr_iq_visualizer_b200 import _native as nat
+    has_gpu = nat.device_count() > 0
+    for nfft in (256, 1000, 4096, 65536):
+        for variant in (0, 1, 12, 22, -1, 2, 5, 11, 20, 21, 23):
+            cfg = nat.spx_plan_config(C.sizeof(nat.spx_plan_config), 0, nfft, nfft // 4, nat.WINDOW_HANN, nat.FMT_CI16,
+                                      1.0, 1e-12, variant, 0)
+            h = C.c_void_p()
+            rc = nat.lib().spx_plan_create(C.byref(h), C.byref(cfg))
+            if variant in (0, 1, 12, 22):
+                assert rc == (nat.OK if has_gpu else nat.E_NODEVICE), (nfft, variant, nat.last_error())
+                if h.value:
+                    nat.check(nat.lib().spx_plan_destroy(h))
+            else:
+                assert rc == nat.E_INVALID and h.value is None, (nfft, variant)
+                assert f"unknown variant {variant}: accepted values are 0, 1, 12 and 22" in nat.last_error()
+
+
 def test_product_never_imports_oracle():
     pkg = os.path.join(ROOT, "sdr_iq_visualizer_b200")
     for base in (pkg, os.path.join(ROOT, "app")):

@@ -194,13 +194,16 @@ def test_emul_k1v2_parity(emul, nfft, hop, kind, fmt):
 @pytest.mark.parametrize("nfft,hop,kind,fmt", [(4096, 1024, "hann", 1), (4096, 4096, "rect", 0), (2048, 1024, "hann", 0), (1024, 512, "blackman", 0)])
 def test_emul_k1v2_fma_form_dft(emul, nfft, hop, kind, fmt):
     """dft16_fma (no stand-alone W_16 multiplies, 144 instead of 160 operations): same parity bar, and its error against
-    the float64 oracle is no worse than the plain radix-16 butterfly's."""
+    the float64 oracle is no worse than the plain radix-16 butterfly's.  The colormap index on the FMA pipe (TUNE_QFMA)
+    is bit for bit the F2I one."""
     L = nfft + hop * 9 + 3
     xc = sref.synth_iq(L, seed=nfft + hop + 1)
     x = sref.to_ci16(xc) if fmt else xc.astype(np.complex64)
     vmin, vmax = (0.0, 130.0) if fmt else (-60.0, 60.0)
     o = run_emul(emul, x, nfft, hop, kind, fmt=fmt, tw_mode=K2 | 0x40, vmin=vmin, vmax=vmax)
     ref = run_emul(emul, x, nfft, hop, kind, fmt=fmt, tw_mode=K2, vmin=vmin, vmax=vmax)
+    f2i = run_emul(emul, x, nfft, hop, kind, fmt=fmt, tw_mode=K2 | 0x80, vmin=vmin, vmax=vmax)
+    np.testing.assert_array_equal(o["wf"], f2i["wf"])
     X = oracle_power(x, nfft, hop, o["win64"], fmt=fmt)
     P = X.real**2 + X.imag**2
     err = lambda r: np.sqrt((np.abs(r["spec"][..., 0] + 1j * r["spec"][..., 1] - X) ** 2).mean() / P.mean())

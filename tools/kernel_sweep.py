@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""GPU micro-benchmark of the fused STFT kernel: variants x shapes, device-resident, CUDA events.
+"""GPU micro-benchmark of the fused STFT kernels over shapes, device-resident, CUDA events.
 Run on the B200 box:  python tools/kernel_sweep.py [--quick]   (prints one JSON line per case)."""
 import argparse
 import json
@@ -58,18 +58,15 @@ def run_case(name, nfft, hop, window, fmt, L, outs, variant=0, iters=10, flush=F
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--quick", action="store_true")
-    ap.add_argument("--variants", default="0,1,2,3,4")
     ap.add_argument("--only4k", action="store_true")
     args = ap.parse_args()
     print(json.dumps(nat.device_info(0)))
     L = 1 << 24 if args.quick else 61_440_000
-    variants = [int(v) for v in args.variants.split(",")]
-    for v in variants:
-        run_case("C2 ci16 75% u8+acc", 4096, 1024, "hann", sp.FMT_CI16, L, ["u8", "acc"], v)
-        run_case("headline cf32 hop=N f32", 4096, 4096, "hann", sp.FMT_CF32, L, ["db"], v)
-        run_case("cf32 hop=N u8", 4096, 4096, "hann", sp.FMT_CF32, L, ["u8"], v)
-        run_case("cf32 hop=N acc only", 4096, 4096, "hann", sp.FMT_CF32, L, ["acc"], v)
-        run_case("cf32 50% f32", 4096, 2048, "hann", sp.FMT_CF32, L, ["db"], v)
+    run_case("C2 ci16 75% u8+acc", 4096, 1024, "hann", sp.FMT_CI16, L, ["u8", "acc"])
+    run_case("headline cf32 hop=N f32", 4096, 4096, "hann", sp.FMT_CF32, L, ["db"])
+    run_case("cf32 hop=N u8", 4096, 4096, "hann", sp.FMT_CF32, L, ["u8"])
+    run_case("cf32 hop=N acc only", 4096, 4096, "hann", sp.FMT_CF32, L, ["acc"])
+    run_case("cf32 50% f32", 4096, 2048, "hann", sp.FMT_CF32, L, ["db"])
     if args.only4k:
         return
     for n in (65536, 16384, 1 << 18):

@@ -1,5 +1,6 @@
 #!/usr/bin/env python3
-"""K1 (variant 0) vs K1v2 (variants 20, 21) on the shapes that matter, device-resident, CUDA events (B200 box)."""
+"""K1 (variant 12) vs the default K1v2 (variant 0) on the shapes that matter, device-resident, CUDA events (B200 box):
+python tools/sweep_k1v2.py [12,0]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import kernel_sweep as ks

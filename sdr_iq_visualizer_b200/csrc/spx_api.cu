@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <map>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -58,6 +59,59 @@ void DevBuf::release() {
     if (ptr) cudaFree(ptr);
     ptr = nullptr;
     cap = 0;
+}
+
+struct KernelOnDevice {
+    const void* kern;
+    int dev;
+    bool operator<(const KernelOnDevice& o) const { return kern != o.kern ? kern < o.kern : dev < o.dev; }
+};
+
+int kernel_setup(const void* kern, int threads, size_t smem, int* occ) {
+    static std::mutex mu;
+    static std::map<KernelOnDevice, int> occ_of;   // blocks per SM
+    int dev = 0;
+    SPX_CUDA(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> g(mu);
+    const KernelOnDevice key{kern, dev};
+    auto it = occ_of.find(key);
+    if (it == occ_of.end()) {
+        int o = 0;
+        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kern, threads, smem));
+        it = occ_of.emplace(key, o).first;
+    }
+    if (occ) *occ = it->second;
+    return SPX_OK;
+}
+
+int DeviceCtx::carve(std::initializer_list<size_t> bytes, void** part) {
+    size_t total = 0;
+    for (size_t b : bytes) total += (b + 255) & ~(size_t)255;
+    SPX_TRY(stage.reserve(total));
+    char* p = (char*)stage.ptr;
+    for (size_t b : bytes) {
+        *part++ = p;
+        p += (b + 255) & ~(size_t)255;
+    }
+    return SPX_OK;
+}
+
+int device_ctx(int device, DeviceCtx** out) {
+    static DeviceCtx ctx[64];
+    int ndev = 0;
+    SPX_TRY(spx_device_count(&ndev));
+    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
+    if (device < 0 || device >= ndev || device >= 64) return spx_set_error(SPX_E_INVALID, "bad device %d", device);
+    SPX_CUDA(cudaSetDevice(device));
+    DeviceCtx& c = ctx[device];
+    std::lock_guard<std::mutex> g(c.mu);
+    if (!c.st) {
+        SPX_CUDA(cudaDeviceGetAttribute(&c.sm_count, cudaDevAttrMultiProcessorCount, device));
+        SPX_CUDA(cudaStreamCreateWithFlags(&c.st, cudaStreamNonBlocking));
+    }
+    *out = &c;
+    return SPX_OK;
 }
 
 int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out) {

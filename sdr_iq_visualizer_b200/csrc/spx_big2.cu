@@ -264,21 +264,12 @@ int big2_launch_stream(spx_plan* pl, const void* in, long long frames, long long
     const bool ci16 = pl->cfg.in_fmt == SPX_FMT_CI16;
     auto k_acc = ci16 ? big2_kernel<true, FMT_CI16> : big2_kernel<true, FMT_CF32>;
     auto k_rows = ci16 ? big2_kernel<false, FMT_CI16> : big2_kernel<false, FMT_CF32>;
-    static int occ_cache2[2][64] = {{0}};
-    int* occ_cache = occ_cache2[ci16 ? 1 : 0];
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    if (occ_cache[dev & 63] == 0) {
-        int o1 = 0, o2 = 0;
-        SPX_CUDA(cudaFuncSetAttribute(k_acc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BIG2_SMEM));
-        SPX_CUDA(cudaFuncSetAttribute(k_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BIG2_SMEM));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o1, k_acc, 256, BIG2_SMEM));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o2, k_rows, 256, BIG2_SMEM));
-        const int o = o1 < o2 ? o1 : o2;
-        if (o < 1) return spx_set_error(SPX_E_CUDA, "big2 kernel does not fit on an SM");
-        occ_cache[dev & 63] = o;
-    }
-    long long lanes = (long long)pl->sm_count * occ_cache[dev & 63] / 16;
+    int o1 = 0, o2 = 0;
+    SPX_TRY(kernel_setup((const void*)k_acc, 256, BIG2_SMEM, &o1));
+    SPX_TRY(kernel_setup((const void*)k_rows, 256, BIG2_SMEM, &o2));
+    const int o = o1 < o2 ? o1 : o2;
+    if (o < 1) return spx_set_error(SPX_E_CUDA, "big2 kernel does not fit on an SM");
+    long long lanes = (long long)pl->sm_count * o / 16;
     if (lanes < 1) return spx_set_error(SPX_E_CUDA, "big2 kernel: fewer than 16 resident CTAs");
     if (lanes > frames) lanes = frames;
     int lag = BIG2_LAG_DEFAULT;

@@ -433,28 +433,16 @@ static int big_launch_pair_t(spx_plan* pl, BigParams& p, cudaStream_t st, bool a
     auto ka_i = big_cols_kernel<N1, N2, FMT_CI16, TMA_A>;
     auto kb_a = big_rows_kernel<N1, N2, true, true>;    // the scratch rows are always 16-byte aligned
     auto kb_n = big_rows_kernel<N1, N2, false, true>;
-    static int occ_a[64][2] = {{0}}, occ_b[64][2] = {{0}};   // per device, benign race (same values)
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    dev &= 63;
-    if (occ_a[dev][0] == 0) {
-        SPX_CUDA(cudaFuncSetAttribute(ka_c, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem_a(8)));
-        SPX_CUDA(cudaFuncSetAttribute(ka_i, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::smem_a(4)));
-        SPX_CUDA(cudaFuncSetAttribute(kb_a, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        SPX_CUDA(cudaFuncSetAttribute(kb_n, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        int o[4] = {0, 0, 0, 0};
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o[0], ka_c, C::THREADS_A, C::smem_a(8)));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o[1], ka_i, C::THREADS_A, C::smem_a(4)));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o[2], kb_a, C::THREADS_B, smem_b));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o[3], kb_n, C::THREADS_B, smem_b));
-        for (int i = 0; i < 4; ++i)
-            if (o[i] < 1) return spx_set_error(SPX_E_CUDA, "large-N kernel does not fit on an SM (N1=%d N2=%d)", N1, N2);
-        occ_a[dev][1] = o[1]; occ_b[dev][0] = o[2]; occ_b[dev][1] = o[3];
-        occ_a[dev][0] = o[0];
-    }
+    int occ_cols[2] = {0, 0}, occ_rows[2] = {0, 0};   // kernel A: cf32, ci16 input; kernel B: with, without accumulators
+    SPX_TRY(kernel_setup((const void*)ka_c, C::THREADS_A, C::smem_a(8), &occ_cols[0]));
+    SPX_TRY(kernel_setup((const void*)ka_i, C::THREADS_A, C::smem_a(4), &occ_cols[1]));
+    SPX_TRY(kernel_setup((const void*)kb_a, C::THREADS_B, smem_b, &occ_rows[0]));
+    SPX_TRY(kernel_setup((const void*)kb_n, C::THREADS_B, smem_b, &occ_rows[1]));
+    if (occ_cols[0] < 1 || occ_cols[1] < 1 || occ_rows[0] < 1 || occ_rows[1] < 1)
+        return spx_set_error(SPX_E_CUDA, "large-N kernel does not fit on an SM (N1=%d N2=%d)", N1, N2);
     // kernel A: grid = column groups x frame lanes (a multiple of the group count: a CTA keeps its columns)
     constexpr int GROUPS_A = N2 / C::G;
-    const int resident_a = pl->sm_count * occ_a[dev][cf32 ? 0 : 1];
+    const int resident_a = pl->sm_count * occ_cols[cf32 ? 0 : 1];
     int lanes = resident_a / GROUPS_A;
     if (lanes < 1) lanes = 1;
     if (lanes > p.frames) lanes = p.frames;
@@ -468,7 +456,7 @@ static int big_launch_pair_t(spx_plan* pl, BigParams& p, cudaStream_t st, bool a
     }
     // kernel B: (row groups) x (frame chunks) work items, one resident wave; accumulators flush once per item
     const int groups = N1 / C::FPC;
-    const int resident_b = pl->sm_count * occ_b[dev][acc ? 0 : 1];
+    const int resident_b = pl->sm_count * occ_rows[acc ? 0 : 1];
     int chunks = (resident_b + groups - 1) / groups;
     if (chunks > p.frames) chunks = p.frames;
     if (chunks < 1) chunks = 1;

@@ -365,13 +365,21 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
     }
 }
 
-// per-device scratch for host-memory calls
-struct FeatScratch {
-    std::mutex mu;
-    DevBuf in, out, peaks;
-    cudaStream_t st = nullptr;
-};
-static FeatScratch g_feat[64];
+// features_kernel over `batch` spectra of n bins, `stride` apart, in float32 (dtype 0) or float64 (dtype 1, checked by the
+// caller); NULL user_opts: the reference's options
+static int features_launch(const void* in, int dtype, int n, int batch, long long stride, spx_features* out, int* peaks,
+                           int peaks_cap, const spx_feature_opts* user_opts, cudaStream_t st) {
+    spx_feature_opts opts;
+    memset(&opts, 0, sizeof(opts));
+    opts.drop_db[0] = 3.0; opts.drop_db[1] = 10.0; opts.drop_db[2] = 20.0;
+    if (user_opts) opts = *user_opts;
+    if (dtype)
+        features_kernel<double><<<batch, FT, 0, st>>>((const double*)in, n, stride, out, peaks, peaks_cap, opts);
+    else
+        features_kernel<float><<<batch, FT, 0, st>>>((const float*)in, n, stride, out, peaks, peaks_cap, opts);
+    SPX_CUDA(cudaGetLastError());
+    return SPX_OK;
+}
 
 }  // namespace spx
 
@@ -381,10 +389,6 @@ extern "C" int spx_classify_features(int32_t device, int32_t mem, const void* po
                                      int32_t batch, int64_t stride, spx_features* out, int32_t* peaks,
                                      int32_t peaks_cap, const spx_feature_opts* user_opts, void* stream) {
     if (!out) return spx_set_error(SPX_E_INVALID, "out is NULL");
-    spx_feature_opts opts;
-    memset(&opts, 0, sizeof(opts));
-    opts.drop_db[0] = 3.0; opts.drop_db[1] = 10.0; opts.drop_db[2] = 20.0;
-    if (user_opts) opts = *user_opts;
     if (batch < 0 || n < 0) return spx_set_error(SPX_E_INVALID, "negative size");
     if (dtype != 0 && dtype != 1) return spx_set_error(SPX_E_INVALID, "dtype must be 0 (float32) or 1 (float64)");
     if (batch == 0) return SPX_OK;
@@ -395,38 +399,29 @@ extern "C" int spx_classify_features(int32_t device, int32_t mem, const void* po
     if (!power_db) return spx_set_error(SPX_E_INVALID, "power_db is NULL");
     if (batch > 1 && stride < n) return spx_set_error(SPX_E_INVALID, "stride < n");
     if (peaks && peaks_cap < 1) peaks = nullptr;
-    int ndev = 0;
-    SPX_TRY(spx_device_count(&ndev));
-    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (device < 0 || device >= ndev || device >= 64) return spx_set_error(SPX_E_INVALID, "bad device %d", device);
-    SPX_CUDA(cudaSetDevice(device));
-    FeatScratch& S = g_feat[device];
-    std::lock_guard<std::mutex> g(S.mu);
-    if (!S.st) SPX_CUDA(cudaStreamCreateWithFlags(&S.st, cudaStreamNonBlocking));
-    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : S.st;
-    const size_t esz = dtype ? 8 : 4;
+    DeviceCtx* ctx;
+    SPX_TRY(device_ctx(device, &ctx));
+    std::lock_guard<std::mutex> g(ctx->mu);
+    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : ctx->st;
     const void* d_in = power_db;
     long long d_stride = stride;
+    size_t in_bytes = 0;
     if (mem == SPX_MEM_HOST) {
         if (batch == 1) d_stride = n;
-        const size_t bytes = ((size_t)(batch - 1) * (size_t)d_stride + (size_t)n) * esz;
-        SPX_TRY(S.in.reserve(bytes));
-        SPX_CUDA(cudaMemcpyAsync(S.in.ptr, power_db, bytes, cudaMemcpyHostToDevice, st));
-        d_in = S.in.ptr;
+        in_bytes = ((size_t)(batch - 1) * (size_t)d_stride + (size_t)n) * (dtype ? 8 : 4);
     }
-    SPX_TRY(S.out.reserve(sizeof(spx_features) * (size_t)batch));
-    int* d_pk = nullptr;
-    if (peaks) {
-        SPX_TRY(S.peaks.reserve(sizeof(int) * (size_t)batch * (size_t)peaks_cap));
-        d_pk = (int*)S.peaks.ptr;
+    const size_t out_bytes = sizeof(spx_features) * (size_t)batch;
+    const size_t pk_bytes = peaks ? sizeof(int) * (size_t)batch * (size_t)peaks_cap : 0;
+    void* part[3];   // staged input (host memory only), results, peaks
+    SPX_TRY(ctx->carve({in_bytes, out_bytes, pk_bytes}, part));
+    if (mem == SPX_MEM_HOST) {
+        SPX_CUDA(cudaMemcpyAsync(part[0], power_db, in_bytes, cudaMemcpyHostToDevice, st));
+        d_in = part[0];
     }
-    if (dtype)
-        features_kernel<double><<<batch, FT, 0, st>>>((const double*)d_in, n, d_stride, (spx_features*)S.out.ptr, d_pk, peaks_cap, opts);
-    else
-        features_kernel<float><<<batch, FT, 0, st>>>((const float*)d_in, n, d_stride, (spx_features*)S.out.ptr, d_pk, peaks_cap, opts);
-    SPX_CUDA(cudaGetLastError());
-    SPX_CUDA(cudaMemcpyAsync(out, S.out.ptr, sizeof(spx_features) * (size_t)batch, cudaMemcpyDeviceToHost, st));
-    if (peaks) SPX_CUDA(cudaMemcpyAsync(peaks, d_pk, sizeof(int) * (size_t)batch * (size_t)peaks_cap, cudaMemcpyDeviceToHost, st));
+    int* d_pk = peaks ? (int*)part[2] : nullptr;
+    SPX_TRY(features_launch(d_in, dtype, n, batch, d_stride, (spx_features*)part[1], d_pk, peaks_cap, user_opts, st));
+    SPX_CUDA(cudaMemcpyAsync(out, part[1], out_bytes, cudaMemcpyDeviceToHost, st));
+    if (peaks) SPX_CUDA(cudaMemcpyAsync(peaks, d_pk, pk_bytes, cudaMemcpyDeviceToHost, st));
     SPX_CUDA(cudaStreamSynchronize(st));
     return SPX_OK;
 }
@@ -438,17 +433,7 @@ extern "C" int spx_classify_features_dev(int32_t device, const void* power_db_de
     if (batch < 1 || n < 1) return spx_set_error(SPX_E_INVALID, "batch and n must be positive");
     if (dtype != 0 && dtype != 1) return spx_set_error(SPX_E_INVALID, "dtype must be 0 (float32) or 1 (float64)");
     if (batch > 1 && stride < n) return spx_set_error(SPX_E_INVALID, "stride < n");
-    spx_feature_opts opts;
-    memset(&opts, 0, sizeof(opts));
-    opts.drop_db[0] = 3.0; opts.drop_db[1] = 10.0; opts.drop_db[2] = 20.0;
-    if (user_opts) opts = *user_opts;
     if (peaks_dev && peaks_cap < 1) peaks_dev = nullptr;
     SPX_CUDA(cudaSetDevice(device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (dtype)
-        features_kernel<double><<<batch, FT, 0, st>>>((const double*)power_db_dev, n, stride, out_dev, peaks_dev, peaks_cap, opts);
-    else
-        features_kernel<float><<<batch, FT, 0, st>>>((const float*)power_db_dev, n, stride, out_dev, peaks_dev, peaks_cap, opts);
-    SPX_CUDA(cudaGetLastError());
-    return SPX_OK;
+    return features_launch(power_db_dev, dtype, n, batch, stride, out_dev, peaks_dev, peaks_cap, user_opts, (cudaStream_t)stream);
 }

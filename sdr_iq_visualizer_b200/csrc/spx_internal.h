@@ -33,4 +33,8 @@ struct NvtxRange {
         if (_rc != SPX_OK) return _rc; \
     } while (0)
 
+// Blocks of `kern` resident per SM at `threads` threads and `smem` bytes of dynamic shared memory on the current
+// device (occ may be NULL); the first call per kernel and device raises the kernel's dynamic shared-memory limit to smem.
+int kernel_setup(const void* kern, int threads, size_t smem, int* occ);
+
 }  // namespace spx

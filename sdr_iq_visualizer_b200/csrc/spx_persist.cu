@@ -97,7 +97,7 @@ int persist_launch(const spx_plan* pl, const uint8_t* rows, long long n_streams,
     if (frames <= 0 || n_streams <= 0) return SPX_OK;
     const int N = pl->cfg.nfft;
     const int smem = 256 * PERSIST_W * (int)sizeof(uint32_t);
-    SPX_CUDA(cudaFuncSetAttribute(persist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    SPX_TRY(kernel_setup((const void*)persist_kernel, PERSIST_THREADS, smem, nullptr));
     const long long strips = (N + PERSIST_W - 1) / PERSIST_W;
     const int vec = (N % 4 == 0 && ((uintptr_t)rows & 3u) == 0) ? 1 : 0;
     // gridDim.y = streams x chunks <= 65535: streams go in groups when there are more

@@ -1,7 +1,9 @@
-// spx_plan.h -- the opaque plan object behind include/spx.h (host-side only).
+// spx_plan.h -- the opaque plan object behind include/spx.h, and the per-device state of the plan-less calls (host-side only).
 #pragma once
 #include <cuda_runtime.h>
 
+#include <initializer_list>
+#include <map>
 #include <mutex>
 #include <vector>
 
@@ -15,6 +17,23 @@ struct DevBuf {
     int reserve(size_t bytes);  // grow-only
     void release();
 };
+
+// What the plan-less one-shot calls (spx_classify_features, spx_iq_hist2d, spx_frame_stats, spx_stream_frame_f64) keep per
+// device.  Each call holds `mu` while it uses the context, so the calls on one device serialise.
+struct DeviceCtx {
+    std::mutex mu;
+    cudaStream_t st = nullptr;   // non-blocking: every host-memory call, and the device-memory calls of the histogram, frame
+                                 // stats and features without a caller stream (spx_stream_frame_f64 keeps the caller's)
+    int sm_count = 0;
+    DevBuf stage;                // device staging of host-memory calls (grow-only)
+    cudaMemPool_t hist_pool = nullptr;   // spx_iq_hist2d's per-CTA tables (stream-ordered: calls on other streams may overlap)
+    std::map<int, double2*> tw64;        // spx_stream_frame_f64: n -> device table of n/2 float64 twiddles
+    // Reserves `stage` for parts of these sizes, each at a 256-byte aligned offset, and points part[i] at part i.
+    int carve(std::initializer_list<size_t> bytes, void** part);
+};
+
+// The context of `device` (0 <= device < min(device count, 64)), made current, with its stream and SM count set up.
+int device_ctx(int device, DeviceCtx** out);
 
 }  // namespace spx
 

@@ -232,16 +232,9 @@ template <int N, int FMT, bool ACC, int OCC, int TUNE>
 int launch_stft2_inst(StftLaunch& L) {
     using C = Stft2Cfg<N, FMT>;
     auto kern = stft2_kernel<N, FMT, ACC, OCC, TUNE>;
-    static int occ_cache[64] = {0};
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    int occ = occ_cache[dev & 63];
-    if (occ == 0) {
-        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, C::THREADS, C::SMEM));
-        if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft2 kernel does not fit on an SM");
-        occ_cache[dev & 63] = occ;
-    }
+    int occ = 0;
+    SPX_TRY(kernel_setup((const void*)kern, C::THREADS, C::SMEM, &occ));
+    if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft2 kernel does not fit on an SM");
     // chunking exactly as K1: <= 256 frames per chunk, chunks never cross a stream
     const long long workers_max = (long long)L.sm_count * occ * C::FPC;
     const long long F = L.p.frames_per_stream;
@@ -282,16 +275,9 @@ int launch_stft2_strip_inst(StftLaunch& L) {
     constexpr int N = 4096;
     using C = Stft2Cfg<N, FMT>;
     auto kern = stft2_strip_kernel<FMT, ACC, R, OCC, TUNE>;
-    static int occ_cache[64] = {0};
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    int occ = occ_cache[dev & 63];
-    if (occ == 0) {
-        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, C::SMEM));
-        if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft2 strip kernel does not fit on an SM");
-        occ_cache[dev & 63] = occ;
-    }
+    int occ = 0;
+    SPX_TRY(kernel_setup((const void*)kern, 256, C::SMEM, &occ));
+    if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft2 strip kernel does not fit on an SM");
     // long chunks (the strip only pays inside a chunk): one chunk per worker and stream where possible, <= 256 frames
     const long long workers_max = (long long)L.sm_count * occ;
     const long long F = L.p.frames_per_stream;

@@ -195,16 +195,9 @@ int launch_stft_inst(StftLaunch& L) {
     auto kern = stft_kernel<N, FMT, ACC, TWM, OCC, STAGE, TUNE>;
     size_t smem = (size_t)(C::FPC * C::slot_f2(STAGE, FMT) + C::win_f2(STAGE)) * sizeof(float2);
     if (TWM == TW_SMEM) smem += (size_t)C::TW_F2 * sizeof(float2);
-    static int occ_cache[64] = {0};  // per instantiation, per device (benign race: same value)
-    int dev = 0;
-    SPX_CUDA(cudaGetDevice(&dev));
-    int occ = occ_cache[dev & 63];
-    if (occ == 0) {
-        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, C::THREADS, smem));
-        if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft kernel does not fit on an SM");
-        occ_cache[dev & 63] = occ;
-    }
+    int occ = 0;
+    SPX_TRY(kernel_setup((const void*)kern, C::THREADS, smem, &occ));
+    if (occ < 1) return spx_set_error(SPX_E_CUDA, "stft kernel does not fit on an SM");
     const long long workers_max = (long long)L.sm_count * occ * C::FPC;
     // chunking: <= 256 frames per chunk, chunks never cross a stream
     const long long F = L.p.frames_per_stream;

@@ -10,11 +10,10 @@
 #include <math.h>
 #include <string.h>
 
-#include <map>
 #include <mutex>
 #include <vector>
 
-#include "spx_internal.h"
+#include "spx_plan.h"
 
 namespace spx {
 
@@ -60,17 +59,10 @@ __global__ void __launch_bounds__(512) stream_frame_f64_kernel(const void* __res
     }
 }
 
-struct StreamCache {
-    std::mutex mu;
-    std::map<long long, double2*> tw;   // (device << 32 | n) -> device table of n/2 twiddles
-    std::map<int, void*> scratch;       // device -> 512 KiB of staging for host-memory calls
-};
-static StreamCache g_stream;
-
-static int stream_twiddles(int device, int n, double2** out) {
-    const long long key = ((long long)device << 32) | (unsigned)n;
-    auto it = g_stream.tw.find(key);
-    if (it != g_stream.tw.end()) { *out = it->second; return SPX_OK; }
+// the device table of n/2 float64 twiddles exp(-2 pi i k / n) of ctx's device
+static int stream_twiddles(DeviceCtx* ctx, int n, double2** out) {
+    auto it = ctx->tw64.find(n);
+    if (it != ctx->tw64.end()) { *out = it->second; return SPX_OK; }
     std::vector<double2> h((size_t)(n / 2 > 0 ? n / 2 : 1));
     const double two_pi = 6.283185307179586476925286766559;
     for (int k = 0; k < n / 2; ++k) {
@@ -83,7 +75,7 @@ static int stream_twiddles(int device, int n, double2** out) {
     double2* d = nullptr;
     SPX_CUDA(cudaMalloc(&d, h.size() * sizeof(double2)));
     SPX_CUDA(cudaMemcpy(d, h.data(), h.size() * sizeof(double2), cudaMemcpyHostToDevice));
-    g_stream.tw[key] = d;
+    ctx->tw64[n] = d;
     *out = d;
     return SPX_OK;
 }
@@ -98,40 +90,31 @@ extern "C" int spx_stream_frame_f64(int device, int mem, const void* samples, in
     if (n < 2 || n > 8192 || (n & (n - 1)) != 0) return spx_set_error(SPX_E_UNSUPPORTED, "spx_stream_frame_f64: n must be a power of two in [2, 8192], got %d", n);
     if (wf_row && !(vmax > vmin)) return spx_set_error(SPX_E_INVALID, "wf_row needs vmax > vmin");
     if (mem != SPX_MEM_HOST && mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", mem);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    }
-    SPX_CUDA(cudaSetDevice(device));
-    std::lock_guard<std::mutex> g(g_stream.mu);
+    DeviceCtx* ctx;
+    SPX_TRY(device_ctx(device, &ctx));
+    std::lock_guard<std::mutex> g(ctx->mu);
     double2* tw = nullptr;
-    SPX_TRY(stream_twiddles(device, n, &tw));
+    SPX_TRY(stream_twiddles(ctx, n, &tw));
     int log2n = 0;
     while ((1 << log2n) < n) ++log2n;
-    cudaStream_t st = (cudaStream_t)stream;
+    cudaStream_t st = mem == SPX_MEM_HOST ? ctx->st : (cudaStream_t)stream;
     const size_t in_bytes = (size_t)n * (in_is_c128 ? 16 : 8);
     const void* d_in = samples;
     double* d_db = power_db_out;
     double2* d_spec = reinterpret_cast<double2*>(spec_out);
     unsigned char* d_wf = wf_row;
     if (mem == SPX_MEM_HOST) {
-        void*& scr = g_stream.scratch[device];
-        if (!scr) SPX_CUDA(cudaMalloc(&scr, 512u << 10));
-        char* base = (char*)scr;                       // [in 128 KiB][dB 64 KiB][spec 128 KiB][u8 8 KiB]
-        SPX_CUDA(cudaMemcpyAsync(base, samples, in_bytes, cudaMemcpyHostToDevice, st));
-        d_in = base;
-        d_db = power_db_out ? (double*)(base + (128u << 10)) : nullptr;
-        d_spec = spec_out ? (double2*)(base + (192u << 10)) : nullptr;
-        d_wf = wf_row ? (unsigned char*)(base + (320u << 10)) : nullptr;
+        void* part[4];
+        SPX_TRY(ctx->carve({in_bytes, (size_t)n * sizeof(double), (size_t)n * sizeof(double2), (size_t)n}, part));
+        SPX_CUDA(cudaMemcpyAsync(part[0], samples, in_bytes, cudaMemcpyHostToDevice, st));
+        d_in = part[0];
+        d_db = power_db_out ? (double*)part[1] : nullptr;
+        d_spec = spec_out ? (double2*)part[2] : nullptr;
+        d_wf = wf_row ? (unsigned char*)part[3] : nullptr;
     }
     const size_t smem = (size_t)n * sizeof(double2);
     auto kern = in_is_c128 ? stream_frame_f64_kernel<true> : stream_frame_f64_kernel<false>;
-    static bool attr_set[2] = {false, false};
-    if (!attr_set[in_is_c128 ? 1 : 0]) {
-        SPX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 8192 * (int)sizeof(double2)));
-        attr_set[in_is_c128 ? 1 : 0] = true;
-    }
+    SPX_TRY(kernel_setup((const void*)kern, 512, 8192 * sizeof(double2), nullptr));
     const double q_scale = wf_row ? 256.0 / (vmax - vmin) : 0.0;
     kern<<<1, n >= 1024 ? 512 : (n >= 64 ? n / 2 : 32), smem, st>>>(d_in, n, log2n, tw, eps, d_db, d_spec, d_wf, vmin, q_scale);
     SPX_CUDA(cudaGetLastError());

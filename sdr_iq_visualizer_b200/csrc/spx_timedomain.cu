@@ -433,24 +433,6 @@ static HistConst hist_constants(const HistGrid& g, int in_fmt, double scale) {
     return hc;
 }
 
-struct TdScratch {
-    std::mutex mu;
-    DevBuf in, a, b;
-    cudaStream_t st = nullptr;
-    cudaMemPool_t pool = nullptr;   // stream-ordered scratch for the private histogram tables (calls on different streams may overlap)
-};
-static TdScratch g_td[64];
-
-static int td_begin(int device, TdScratch** out) {
-    int ndev = 0;
-    SPX_TRY(spx_device_count(&ndev));
-    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (device < 0 || device >= ndev || device >= 64) return spx_set_error(SPX_E_INVALID, "bad device %d", device);
-    SPX_CUDA(cudaSetDevice(device));
-    *out = &g_td[device];
-    return SPX_OK;
-}
-
 }  // namespace spx
 
 using namespace spx;
@@ -461,11 +443,10 @@ extern "C" int spx_iq_hist2d(int32_t device, int32_t mem, const void* in, int32_
     if (bins < 1 || bins > 4096 || !(r > 0.0)) return spx_set_error(SPX_E_INVALID, "need 1 <= bins <= 4096 and R > 0");
     if (in_fmt != SPX_FMT_CF32 && in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt");
     if (n < 0 || (n > 0 && !in)) return spx_set_error(SPX_E_INVALID, "bad input");
-    TdScratch* S;
-    SPX_TRY(td_begin(device, &S));
-    std::lock_guard<std::mutex> lk(S->mu);
-    if (!S->st) SPX_CUDA(cudaStreamCreateWithFlags(&S->st, cudaStreamNonBlocking));
-    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : S->st;
+    DeviceCtx* ctx;
+    SPX_TRY(device_ctx(device, &ctx));
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : ctx->st;
     HistGrid g;
     g.start = -r;
     g.stop = r;
@@ -476,27 +457,24 @@ extern "C" int spx_iq_hist2d(int32_t device, int32_t mem, const void* in, int32_
     const void* d_in = in;
     unsigned int* d_hist = hist;
     if (mem == SPX_MEM_HOST) {
-        SPX_TRY(S->in.reserve((size_t)n * esz));
-        SPX_TRY(S->a.reserve(hbytes));
-        if (n) SPX_CUDA(cudaMemcpyAsync(S->in.ptr, in, (size_t)n * esz, cudaMemcpyHostToDevice, st));
-        d_in = S->in.ptr;
-        d_hist = (unsigned int*)S->a.ptr;
+        void* part[2];
+        SPX_TRY(ctx->carve({(size_t)n * esz, hbytes}, part));
+        if (n) SPX_CUDA(cudaMemcpyAsync(part[0], in, (size_t)n * esz, cudaMemcpyHostToDevice, st));
+        d_in = part[0];
+        d_hist = (unsigned int*)part[1];
         if (accumulate) SPX_CUDA(cudaMemcpyAsync(d_hist, hist, hbytes, cudaMemcpyHostToDevice, st));
     }
     bool zeroed = accumulate != 0;
     if (n > 0) {
-        int sm = 148;
-        cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device);
+        const int sm = ctx->sm_count;
         const int vec_ok = ((uintptr_t)d_in & 15u) == 0 ? 1 : 0;
         const size_t words = (size_t)((bins * bins + 1) / 2);
         const size_t smem = ((words + 3) & ~(size_t)3) * sizeof(unsigned int) + (size_t)(bins + 2) * sizeof(float);
         if (smem <= 200u * 1024u && in_scale > 0.0 && in_scale < 1e30) {
             // shared-memory privatised counting: one CTA per SM, each with a contiguous share of the input (a multiple of 8
             // samples, at least one epoch so that small inputs do not spread over CTAs that each dump a table)
-            auto k_c = hist2d_smem_kernel<SPX_FMT_CF32>;
-            auto k_i = hist2d_smem_kernel<SPX_FMT_CI16>;
-            SPX_CUDA(cudaFuncSetAttribute(k_c, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SPX_CUDA(cudaFuncSetAttribute(k_i, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            auto kern = in_fmt == SPX_FMT_CF32 ? hist2d_smem_kernel<SPX_FMT_CF32> : hist2d_smem_kernel<SPX_FMT_CI16>;
+            SPX_TRY(kernel_setup((const void*)kern, 1024, 200 * 1024, nullptr));
             long long span = ((n + sm - 1) / sm + 7) & ~7ll;
             if (span < 32760) span = 32760;
             const long long blocks = (n + span - 1) / span;
@@ -504,17 +482,17 @@ extern "C" int spx_iq_hist2d(int32_t device, int32_t mem, const void* in, int32_
             unsigned int* tabs = nullptr;
             const int tab_stride = (int)((words + 3) & ~(size_t)3);
             if (blocks > 4) {
-                if (!S->pool) {
+                if (!ctx->hist_pool) {
                     cudaMemPoolProps props;
                     memset(&props, 0, sizeof(props));
                     props.allocType = cudaMemAllocationTypePinned;
                     props.location.type = cudaMemLocationTypeDevice;
                     props.location.id = device;
-                    SPX_CUDA(cudaMemPoolCreate(&S->pool, &props));
+                    SPX_CUDA(cudaMemPoolCreate(&ctx->hist_pool, &props));
                     unsigned long long keep = ~0ull;   // freed blocks stay in the pool: the next call reuses them
-                    SPX_CUDA(cudaMemPoolSetAttribute(S->pool, cudaMemPoolAttrReleaseThreshold, &keep));
+                    SPX_CUDA(cudaMemPoolSetAttribute(ctx->hist_pool, cudaMemPoolAttrReleaseThreshold, &keep));
                 }
-                SPX_CUDA(cudaMallocFromPoolAsync((void**)&tabs, (size_t)blocks * tab_stride * sizeof(unsigned int), S->pool, st));
+                SPX_CUDA(cudaMallocFromPoolAsync((void**)&tabs, (size_t)blocks * tab_stride * sizeof(unsigned int), ctx->hist_pool, st));
             }
             cudaLaunchAttribute pdl[1];
             pdl[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -530,7 +508,7 @@ extern "C" int spx_iq_hist2d(int32_t device, int32_t mem, const void* in, int32_
             cfg.gridDim = dim3((unsigned)blocks);
             cfg.blockDim = dim3(1024);
             cfg.dynamicSmemBytes = smem;
-            SPX_CUDA(cudaLaunchKernelEx(&cfg, in_fmt == SPX_FMT_CF32 ? k_c : k_i, d_in, (long long)n, in_scale, g, d_hist, vec_ok, span, tabs, tab_stride, hc));
+            SPX_CUDA(cudaLaunchKernelEx(&cfg, kern, d_in, (long long)n, in_scale, g, d_hist, vec_ok, span, tabs, tab_stride, hc));
             if (tabs) {
                 cfg.gridDim = dim3((unsigned)((words + 63) / 64));
                 cfg.blockDim = dim3(256);
@@ -567,24 +545,22 @@ extern "C" int spx_frame_stats(int32_t device, int32_t mem, const void* in, int3
     if (n_frames_out) *n_frames_out = F;
     if (F == 0) return SPX_OK;
     if (!in || !mean_pow || !peak_pow) return spx_set_error(SPX_E_INVALID, "NULL buffer");
-    TdScratch* S;
-    SPX_TRY(td_begin(device, &S));
-    std::lock_guard<std::mutex> lk(S->mu);
-    if (!S->st) SPX_CUDA(cudaStreamCreateWithFlags(&S->st, cudaStreamNonBlocking));
-    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : S->st;
+    DeviceCtx* ctx;
+    SPX_TRY(device_ctx(device, &ctx));
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    cudaStream_t st = (mem == SPX_MEM_DEVICE && stream) ? (cudaStream_t)stream : ctx->st;
     const size_t esz = in_fmt == SPX_FMT_CI16 ? 4 : 8;
     const void* d_in = in;
     float *d_mean = mean_pow, *d_peak = peak_pow;
     if (mem == SPX_MEM_HOST) {
-        SPX_TRY(S->in.reserve((size_t)n * esz));
-        SPX_TRY(S->b.reserve((size_t)F * 2 * sizeof(float)));
-        SPX_CUDA(cudaMemcpyAsync(S->in.ptr, in, (size_t)n * esz, cudaMemcpyHostToDevice, st));
-        d_in = S->in.ptr;
-        d_mean = (float*)S->b.ptr;
+        void* part[2];
+        SPX_TRY(ctx->carve({(size_t)n * esz, (size_t)F * 2 * sizeof(float)}, part));
+        SPX_CUDA(cudaMemcpyAsync(part[0], in, (size_t)n * esz, cudaMemcpyHostToDevice, st));
+        d_in = part[0];
+        d_mean = (float*)part[1];
         d_peak = d_mean + F;
     }
-    int sm = 148;
-    cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device);
+    const int sm = ctx->sm_count;
     long long blocks = F < (long long)sm * 8 ? F : (long long)sm * 8;
     if (in_fmt == SPX_FMT_CF32)
         frame_stats_kernel<SPX_FMT_CF32><<<(unsigned)blocks, 256, 0, st>>>(d_in, F, frame_len, hop, in_scale, d_mean, d_peak);

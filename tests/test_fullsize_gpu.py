@@ -80,7 +80,7 @@ def test_config4_full_size_streams_and_features():
     assert F == 16383
     r = pl.stft(d_in, n_streams=S, welch=True, maxhold=True, n_samples=Ls)
     pxx, pdb = pl.welch_finalize(r.welch_acc, F, 61.44e6, n_streams=S)
-    feats = features.measure_batch(pdb, n=N, batch=S)
+    feats = features.measure_batch(pdb, n=N, batch=S, stream=pl.stream)   # after the finalize on the plan's stream
     pxx_h = pxx.to_host().reshape(S, N)
     counts = np.bincount(np.arange(F) % period, minlength=period).astype(np.float64)
     w = sref.window("hann", N)

@@ -156,3 +156,36 @@ def test_hist2d_fuzz_against_numpy():
     r = subprocess.run([sys.executable, os.path.join(root, "tools", "fuzz_hist2d.py"), "120", "7"], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     assert "0 mismatches" in r.stdout
+
+
+def test_plan_less_calls_on_every_device_and_bad_index(td):
+    """The plan-less one-shot calls (histogram, frame stats, float64 stream frame, classifier measurements) keep their
+    stream, staging and kernel set-up per device: on every device, after a first call on device 0, each returns exactly
+    device 0's result, and a device index equal to the device count is rejected as an invalid argument."""
+    from sdr_iq_visualizer_b200 import _native as nat, features, spectral
+    n_dev = nat.device_count()
+    x = sref.synth_iq(1 << 20, seed=17).astype(np.complex64)
+    frame = x[:8192].astype(np.complex128)
+
+    def run(dev):
+        _, pdb = spectral.stream_frame(frame, 2.5e6, 9.15e8, device=dev)
+        return (pdb, td.iq_hist2d(x, 4.0, 256, device=dev), td.frame_stats(x, 4096, 4096, device=dev),
+                features.measure(pdb, device=dev))
+
+    for call in (lambda: spectral.stream_frame(frame, 2.5e6, 9.15e8, device=n_dev),
+                 lambda: td.iq_hist2d(x, 4.0, 256, device=n_dev),
+                 lambda: td.frame_stats(x, 4096, 4096, device=n_dev),
+                 lambda: features.measure(np.zeros(8192), device=n_dev)):
+        with pytest.raises(nat.SpectralError) as e:
+            call()
+        assert e.value.code == nat.E_INVALID
+    if n_dev < 2:
+        pytest.skip("needs two GPUs")
+    ref = run(0)
+    for dev in range(n_dev):
+        got = run(dev)
+        np.testing.assert_array_equal(got[0], ref[0])
+        np.testing.assert_array_equal(got[1], ref[1])
+        np.testing.assert_array_equal(got[2][0], ref[2][0])
+        np.testing.assert_array_equal(got[2][1], ref[2][1])
+        assert got[3] == ref[3], dev

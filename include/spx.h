@@ -307,6 +307,49 @@ SPX_API int spx_ddc_sync(spx_ddc* ddc);
 SPX_API int spx_ddc_exec(spx_ddc* ddc, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
                          int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream);
 
+/* ---------------------------------------------------------------- polyphase channelizer (channel scan)
+ * Splits a wideband capture into M baseband channels in one pass: all M down-conversions of the DDC above at once.  With
+ * the DDC's names (x = in_fmt samples times in_scale, sample n has global index first_sample + n, real taps h[0 .. T-1]),
+ * channel j = 0 .. M-1 in fftshift order, offset c = j - M/2, is the DDC with phase_inc_j = c 2^64 / M (mod 2^64), taps h
+ * and decimation D:
+ *   y_j[m] = sum_k h[k] x[mD + T-1-k] exp(-2 pi i c (first_sample + mD + T-1-k) / M),   m = 0 .. n_out - 1
+ *   n_out  = (n_samples - T) / D + 1   (0 if n_samples < T), as spx_ddc_exec
+ * Channel j is centred at fc + c fs / M and runs at fs / D; a tone at its centre comes out at 0 Hz.  It is computed as a
+ * fold of the taps by global sample class (first_sample + n) mod M followed by one M-point FFT per output step, and the
+ * arithmetic of y_j[m] depends only on global indices, the taps and the input: calls on pieces of a capture that overlap
+ * by T - D samples, each with the global first_sample of its piece, give the outputs of one call bit for bit.
+ * Supported: M a power of two in [16, 4096]; D = M (critically sampled) or M / 2 (2x oversampled); T in [1, 32 M]. */
+typedef struct spx_chan spx_chan;
+
+typedef struct {
+    uint32_t struct_size;  /* sizeof(spx_chan_config) */
+    int32_t device;
+    int32_t in_fmt;        /* SPX_FMT_* */
+    float in_scale;        /* multiplies every sample (0 = 1.0) */
+    int32_t n_channels;    /* M: power of two in [16, 4096] */
+    int32_t decim;         /* D: M or M / 2 */
+    int32_t n_taps;        /* T in [1, 32 M] */
+    const double* taps;    /* host, h[0 .. T - 1]; rounded once to float32 at create */
+} spx_chan_config;
+
+/* SPX_E_INVALID: NULL out / cfg, a wrong struct_size, M not a power of two in [16, 4096], D not M or M / 2, T outside
+ * [1, 32 M], NULL taps, an unknown in_fmt, a device index out of range.  SPX_E_NODEVICE: no CUDA device (no CPU
+ * fallback). */
+SPX_API int spx_chan_create(spx_chan** out, const spx_chan_config* cfg);
+SPX_API int spx_chan_destroy(spx_chan* chan);
+/* wait for everything the handle has enqueued on its own streams; SPX_E_INVALID for NULL */
+SPX_API int spx_chan_sync(spx_chan* chan);
+/* The channels of n_samples samples into out[M][out_stride] (complex64 as float32 I, Q; channel-major, columns
+ * n_out .. out_stride - 1 are left as they are); *n_out = n_out.  SPX_MEM_DEVICE: `in` / `out` are device pointers used
+ * on `stream` (NULL = the handle's stream), nothing is synchronised.  SPX_MEM_HOST: the input is staged through pieces
+ * of SPX_H2D_PIECE_BYTES (handle-creation environment variable, default 16 MiB) cut at output boundaries with the T - D
+ * halo; each piece's [M][per] block is copied into the host rows as it finishes, and the call returns when `out` is
+ * written.  SPX_E_INVALID for a NULL handle, a bad mem, n_samples < 0, first_sample < 0, and, when n_out > 0,
+ * out_stride < n_out, NULL in or out, `in` not 4-byte or `out` not 8-byte aligned.  n_out = 0 launches nothing. */
+SPX_API int spx_chan_exec(spx_chan* chan, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample,
+                          float* out, int64_t out_stride, int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out,
+                          void* stream);
+
 /* Measurement helper: runs spx_stft_exec (SPX_MEM_DEVICE buffers only) warmup+iters times on the
  * launch stream, each bracketed by CUDA events; optionally READS a 256 MiB buffer before every
  * iteration to flush the 126 MB L2 without leaving dirty lines behind.  ms_each[iters] receives the device time of

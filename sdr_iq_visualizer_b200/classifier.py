@@ -38,14 +38,19 @@ def _spacing_std(freqs, peaks) -> float:
     return float(np.std(np.diff(pf)))
 
 
-def measure(freqs, power_db) -> dict:
-    """GPU measurements + the Hz quantities derived from the caller's frequency axis (un-rounded)."""
-    m = _features.measure(power_db)
+def add_hz(freqs, m: dict) -> dict:
+    """Adds to a ``features.measure_batch`` result (with its peak list) the Hz quantities derived from the caller's
+    frequency axis, un-rounded: occupied bandwidths bw3 / bw10 / bw20 and the peak-spacing sigma.  Returns ``m``."""
     m["bw3"] = _span(freqs, m["first_3db"], m["last_3db"])
     m["bw10"] = _span(freqs, m["first_10db"], m["last_10db"])
     m["bw20"] = _span(freqs, m["first_20db"], m["last_20db"])
     m["peak_spacing_std_hz"] = _spacing_std(freqs, m["peaks"])   # the list is complete (features.measure_batch raises otherwise)
     return m
+
+
+def measure(freqs, power_db) -> dict:
+    """GPU measurements + the Hz quantities derived from the caller's frequency axis (un-rounded)."""
+    return add_hz(freqs, _features.measure(power_db))
 
 
 def classify_signal_simple(freqs, power_db):
@@ -161,9 +166,11 @@ def with_hz(freqs, m: dict) -> dict:
     return m
 
 
-def classify_from_measurements(freqs, m: dict, n_bins: int):
+def classify_from_measurements(freqs, m: dict, n_bins: int, smooth: bool = True):
     """Label rules + temporal smoothing (classifier.py:60-161) on measurements already taken (``measure`` or
-    ``with_hz``): scalar host logic only."""
+    ``with_hz``): scalar host logic only.  ``smooth=False`` applies the rules alone and leaves the module-global history
+    untouched, for spectra that are not one signal over time (e.g. the channels of a channel scan); the label and
+    confidence are then the rule table's and the reported stability is 1."""
     power_db = range(n_bins)   # only its length is used below
     v = _V()
     v.snr, v.sfm, v.kurt = float(m["snr_db"]), float(m["flatness"]), float(m["kurtosis"])
@@ -176,7 +183,10 @@ def classify_from_measurements(freqs, m: dict, n_bins: int):
     v.occ = v.bw20 / span_hz if span_hz > 0 else 0.0
 
     label, confidence, reasons = _apply_rules(v)
-    label, confidence, stability = _smooth(label, confidence, reasons)
+    if smooth:
+        label, confidence, stability = _smooth(label, confidence, reasons)
+    else:
+        stability = 1.0
 
     explanation = (
         f"SNR={v.snr:.1f} dB | peaks={v.peaks} (density {v.density:.3f}) | flat={v.sfm:.2f} | kurt={v.kurt:.2f} "

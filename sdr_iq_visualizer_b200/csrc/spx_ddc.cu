@@ -18,6 +18,7 @@
 
 #include "spx_ddc_device.cuh"
 #include "spx_internal.h"
+#include "spx_pieces.h"
 #include "spx_plan.h"
 
 namespace spx {
@@ -255,16 +256,6 @@ struct spx_ddc {
 
 namespace spx {
 
-static int ddc_event(spx_ddc* d, size_t i, cudaEvent_t* out) {
-    while (d->events.size() <= i) {
-        cudaEvent_t e;
-        SPX_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        d->events.push_back(e);
-    }
-    *out = d->events[i];
-    return SPX_OK;
-}
-
 static long long ddc_out_count(long long L, int T, int D) { return L < T ? 0 : (L - T) / D + 1; }
 
 // K9 over samples [0, L) of `in` (device), global index of sample 0 = n0, outputs -> out (device)
@@ -303,48 +294,24 @@ static int ddc_launch(spx_ddc* d, const void* in, long long L, unsigned long lon
     return SPX_OK;
 }
 
-// Host memory: pieces of about piece_bytes of input, cut at output boundaries with the T - D halo, uploaded on s_h2d into
-// two alternating buffers (the upload of piece k + 1 overlaps the kernel of piece k); each piece's outputs drain on s_d2h.
-static int ddc_exec_host(spx_ddc* d, const void* in, long long L, long long M, unsigned long long n0, float* out,
-                         int64_t* h2d_out, int64_t* d2h_out) {
+// Host memory: pieces of about piece_bytes of input (host_pieces, spx_pieces.h); the outputs land in one device buffer
+// and each piece's outputs drain on s_d2h.
+static int ddc_exec_host(spx_ddc* d, const void* in, long long M, unsigned long long n0, float* out, int64_t* h2d_out,
+                         int64_t* d2h_out) {
     const int T = d->cfg.n_taps, D = d->cfg.decim;
     const size_t elt = d->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
-    long long per = ((long long)(d->piece_bytes / elt) - T) / D + 1;   // outputs per piece
-    if (per < 1) per = 1;
-    if (per > M) per = M;
-    const long long span = (per - 1) * D + T;   // input samples of a full piece
-    SPX_TRY(d->st_in.reserve(2 * (size_t)span * elt));
     SPX_TRY(d->st_out.reserve((size_t)M * 8));
-    char* d_in[2] = {(char*)d->st_in.ptr, (char*)d->st_in.ptr + (size_t)span * elt};
     float* d_out = (float*)d->st_out.ptr;
-    long long h2d = 0, d2h = 0;
-    size_t ev = 0;
-    cudaEvent_t e_done[2] = {nullptr, nullptr};
-    for (long long m0 = 0, k = 0; m0 < M; m0 += per, ++k) {
-        const long long nm = M - m0 < per ? M - m0 : per;
-        const long long a = m0 * D, n = (nm - 1) * D + T;
-        const int b = (int)(k & 1);
-        cudaEvent_t e_in, e_k;
-        SPX_TRY(ddc_event(d, ev++, &e_in));
-        SPX_TRY(ddc_event(d, ev++, &e_k));
-        if (e_done[b]) SPX_CUDA(cudaStreamWaitEvent(d->s_h2d, e_done[b], 0));   // the kernel that last read this buffer
-        SPX_CUDA(cudaMemcpyAsync(d_in[b], (const char*)in + (size_t)a * elt, (size_t)n * elt, cudaMemcpyHostToDevice, d->s_h2d));
-        h2d += n * (long long)elt;
-        SPX_CUDA(cudaEventRecord(e_in, d->s_h2d));
-        SPX_CUDA(cudaStreamWaitEvent(d->s_compute, e_in, 0));
-        SPX_TRY(ddc_launch(d, d_in[b], n, n0 + (unsigned long long)a, d_out + 2 * m0, d->s_compute));
-        SPX_CUDA(cudaEventRecord(e_k, d->s_compute));
-        e_done[b] = e_k;
-        SPX_CUDA(cudaStreamWaitEvent(d->s_d2h, e_k, 0));
-        SPX_CUDA(cudaMemcpyAsync(out + 2 * m0, d_out + 2 * m0, (size_t)nm * 8, cudaMemcpyDeviceToHost, d->s_d2h));
-        d2h += nm * 8;
-    }
-    SPX_CUDA(cudaStreamSynchronize(d->s_h2d));
-    SPX_CUDA(cudaStreamSynchronize(d->s_compute));
-    SPX_CUDA(cudaStreamSynchronize(d->s_d2h));
-    *h2d_out = h2d;
-    *d2h_out = d2h;
-    return SPX_OK;
+    const HostPieces hp{d->s_h2d, d->s_compute, d->s_d2h, &d->events, &d->st_in, d->piece_bytes, false};
+    auto launch = [&](const void* d_in, long long n, long long a, long long m0, long long, int, cudaStream_t st) {
+        return ddc_launch(d, d_in, n, n0 + (unsigned long long)a, d_out + 2 * m0, st);
+    };
+    auto drain = [&](long long m0, long long nm, int, cudaStream_t st, long long* bytes) {
+        SPX_CUDA(cudaMemcpyAsync(out + 2 * m0, d_out + 2 * m0, (size_t)nm * 8, cudaMemcpyDeviceToHost, st));
+        *bytes = nm * 8;
+        return SPX_OK;
+    };
+    return host_pieces(hp, in, elt, T, D, M, piece_outputs(d->piece_bytes, elt, T, D, M), launch, drain, h2d_out, d2h_out);
 }
 
 }  // namespace spx
@@ -445,7 +412,7 @@ int spx_ddc_exec(spx_ddc* d, int32_t mem, const void* in, int64_t n_samples, int
     if (mem == SPX_MEM_DEVICE)
         return ddc_launch(d, in, n_samples, (unsigned long long)first_sample, out, stream ? (cudaStream_t)stream : d->s_compute);
     int64_t h2d = 0, d2h = 0;
-    SPX_TRY(ddc_exec_host(d, in, n_samples, M, (unsigned long long)first_sample, out, &h2d, &d2h));
+    SPX_TRY(ddc_exec_host(d, in, M, (unsigned long long)first_sample, out, &h2d, &d2h));
     if (h2d_bytes_out) *h2d_bytes_out = h2d;
     if (d2h_bytes_out) *d2h_bytes_out = d2h;
     return SPX_OK;

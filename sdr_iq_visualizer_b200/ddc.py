@@ -10,6 +10,9 @@ it belongs to time ``(first_sample + m decim + (T - 1) / 2) / fs``.  The default
 free of aliasing (``usable_span_hz``); the outer 10 % of each side of the zoomed span is roll-off.  One stage takes up to
 8192 taps (decim 256 with the default design); for more decimation cascade two plans, the second with ``shift_hz=0``.
 Compute is libspx only (no CPU fallback); the filter design is numpy only.
+
+A ``Channelizer`` does the M down-conversions of a uniform channel grid at once (a polyphase filter bank): channel j is the
+``DdcPlan`` at shift ``(j - M/2) fs / M``, and its channel-major output feeds ``SpectralPlan.stft`` as M streams.
 """
 from __future__ import annotations
 
@@ -157,5 +160,111 @@ class DdcPlan:
         n_out, h2d, d2h = C.c_int64(), C.c_int64(), C.c_int64()
         nat.check(nat.lib().spx_ddc_exec(self._h, mem, in_ptr, L, int(first_sample), nat.as_ptr(out)[0], C.byref(n_out),
                                          C.byref(h2d), C.byref(d2h), stream or None))
+        self.last_h2d_bytes, self.last_d2h_bytes = int(h2d.value), int(d2h.value)
+        return out
+
+
+class Channelizer:
+    """Polyphase filter-bank channelizer (libspx K10, ``spx_chan_*``): splits a ``sample_rate`` stream into
+    ``n_channels`` (M, a power of two in [16, 4096]) baseband channels in one pass on one GPU.  Channel j (fftshift order)
+    is the ``DdcPlan`` at shift ``(j - M/2) fs / M`` with the same taps and decimation, centred at ``fc + (j - M/2) fs / M``
+    and running at ``fs / decim``; a tone at its centre comes out at 0 Hz.
+
+    ``decim``: M / 2 (2x oversampled, the default) or M (critically sampled).  Default taps: ``design_taps(M // 2,
+    transition=0.5)`` for M / 2 (cutoff fs / M, the whole channel band |f| <= fs / (2M) alias-free) and ``design_taps(M)``
+    for M (the usual compromise: |f| <= 0.4 fs / M alias-free, the channel edges roll off).  Up to 32 M caller taps."""
+
+    def __init__(self, sample_rate: float, n_channels: int, decim: Optional[int] = None, taps=None,
+                 in_fmt: int = FMT_CF32, in_scale: float = 1.0, device: int = 0):
+        self.sample_rate = float(sample_rate)
+        M = int(n_channels)
+        if M < 16 or M > 4096 or M & (M - 1):
+            raise ValueError(f"n_channels {M} must be a power of two in [16, 4096]")
+        self.n_channels = M
+        self.decim = M // 2 if decim is None else int(decim)
+        if self.decim not in (M, M // 2):
+            raise ValueError(f"decim {self.decim} must be n_channels ({M}) or n_channels / 2")
+        if taps is None:
+            taps = design_taps(M // 2, transition=0.5) if self.decim == M // 2 else design_taps(M)
+        self.taps = np.ascontiguousarray(taps, dtype=np.float64).ravel()
+        if not 1 <= self.taps.size <= 32 * M:
+            raise ValueError(f"{self.taps.size} taps: the channelizer takes 1 .. 32 n_channels = {32 * M}")
+        if in_fmt not in (FMT_CF32, FMT_CI16):
+            raise ValueError(f"unknown in_fmt {in_fmt}")
+        self.in_fmt, self.in_scale, self.device = int(in_fmt), float(in_scale), int(device)
+        self._h = None
+        nat.require_device()
+        cfg = nat.spx_chan_config(C.sizeof(nat.spx_chan_config), self.device, self.in_fmt, self.in_scale, M, self.decim,
+                                  self.n_taps, self.taps.ctypes.data)
+        h = C.c_void_p()
+        nat.check(nat.lib().spx_chan_create(C.byref(h), C.byref(cfg)))
+        self._h = h
+
+    @property
+    def n_taps(self) -> int:
+        return int(self.taps.size)
+
+    @property
+    def out_rate(self) -> float:
+        return self.sample_rate / self.decim
+
+    def out_count(self, n_samples: int) -> int:
+        """n_out = (n - T) // decim + 1 outputs per channel of n input samples (0 if n < T)."""
+        n = int(n_samples)
+        return 0 if n < self.n_taps else (n - self.n_taps) // self.decim + 1
+
+    def channel_freqs(self, center_freq: float = 0.0) -> np.ndarray:
+        """Centre frequency of each channel, float64 [M] in fftshift order: fc + (j - M/2) fs / M."""
+        M = self.n_channels
+        return center_freq + (np.arange(M) - M // 2) * (self.sample_rate / M)
+
+    def close(self) -> None:
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            nat.lib().spx_chan_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def sync(self) -> None:
+        nat.check(nat.lib().spx_chan_sync(self._h))
+
+    def exec(self, x, first_sample: int = 0, out=True, stream: int = 0, n_samples: Optional[int] = None):
+        """Channels of ``x`` as complex64 [M][n_out] (numpy input: staged through pinned pieces, returns numpy; DeviceArray
+        / CUDA tensor: enqueued on ``stream``, returns a DeviceArray).  ``first_sample``: the global index of x's first
+        sample, so that pieces that overlap by ``n_taps - decim`` samples give the outputs of one call.  ``out``: True
+        (allocate) or a caller buffer [M][S] complex64 with S >= n_out in x's memory space; columns n_out .. S - 1 are
+        left untouched."""
+        if int(first_sample) < 0:
+            raise ValueError("first_sample must be >= 0")
+        if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
+            x = SpectralPlan._host_input(self, x)
+        in_ptr, mem = nat.as_ptr(x)
+        L = int(n_samples) if n_samples is not None else SpectralPlan._samples_per_stream(self, x, 1)
+        M, n_out = self.n_channels, self.out_count(L)
+        if out is True:
+            out = np.empty((M, n_out), np.complex64) if mem == MEM_HOST else DeviceArray((M, n_out), np.complex64,
+                                                                                          self.device)
+            S = n_out
+        else:
+            if nat.as_ptr(out)[1] != mem:
+                raise ValueError("out must live where the input lives")
+            shape = tuple(out.shape)
+            if len(shape) != 2 or shape[0] != M or shape[1] < n_out:
+                raise ValueError(f"out: expected shape ({M}, S) with S >= {n_out}, got {shape}")
+            _check_buffer(out, shape, np.complex64, "out")
+            S = shape[1]
+        n, h2d, d2h = C.c_int64(), C.c_int64(), C.c_int64()
+        nat.check(nat.lib().spx_chan_exec(self._h, mem, in_ptr, L, int(first_sample), nat.as_ptr(out)[0], max(S, 1),
+                                          C.byref(n), C.byref(h2d), C.byref(d2h), stream or None))
         self.last_h2d_bytes, self.last_d2h_bytes = int(h2d.value), int(d2h.value)
         return out

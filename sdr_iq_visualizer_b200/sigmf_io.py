@@ -429,6 +429,89 @@ def _process_zoomed(rec, zoom, zoom_taps, nfft, hop, window, waterfall, vmin, vm
     return out
 
 
+@dataclass
+class ChannelScan:
+    """What ``scan_channels`` measured: one row per channel, channels in fftshift order (lowest frequency first)."""
+    channel_freqs: np.ndarray      # float64 [M] RF centre of each channel
+    out_rate: float                # channel sample rate fs / D
+    freqs: np.ndarray              # float64 [nfft] baseband axis of one channel (add channel_freqs[j] for RF)
+    pxx: np.ndarray                # float64 [M, nfft] Welch density of each channel (mlab.psd, two-sided)
+    pxx_db: np.ndarray             # float64 [M, nfft] 10 log10 pxx
+    maxhold: Optional[np.ndarray]  # float32 [M, nfft] max over frames of |X|^2
+    n_frames: int                  # frames per channel
+    measurements: list             # per channel: features.measure_batch dict of the measured band, plus bw3/10/20, spacing
+    classification: list           # per channel: classify_signal_advanced's result dict (no temporal smoothing)
+    band: tuple = (0, 0)           # bins [lo, hi) of each channel's spectrum that were measured and classified
+
+
+def scan_channels(path_or_rec, n_channels: int = 64, decim: Optional[int] = None, nfft: int = 256, hop: Optional[int] = None,
+                  window="hann", maxhold: bool = True, taps=None, max_chunk_samples: int = 1 << 24,
+                  device: int = 0) -> ChannelScan:
+    """Channel scan of a recording: which channels of the band are occupied, and by what.  The capture is split on the GPU
+    into ``n_channels`` baseband channels (``ddc.Channelizer``, default decim n_channels / 2), and every channel gets a
+    Welch spectrum (``nfft``, ``hop`` default nfft, ``window``), a max-hold, the classifier measurements and a verdict.
+
+    The file is read chunk by chunk.  Each chunk yields ``nfft + (k - 1) hop`` channel outputs that start on an STFT frame
+    boundary, so consecutive chunks overlap by ``(nfft - hop) D + (T - D)`` input samples, and the per-chunk STFT over the
+    M channel streams accumulates the Welch sums and max-holds of one pass over the file.  With D = M / 2 only the centre
+    nfft / 2 bins (the channel's own fs / M) are measured and classified, so that neighbours seen in the oversampled
+    margin do not count; with D = M all bins are.  The classifier runs without its temporal smoothing: M channels are not
+    one signal over time."""
+    from . import classifier as cls_mod
+    from . import ddc as ddc_mod
+    from . import features
+    from ._native import DeviceArray, DeviceView
+    nat = sp.nat
+    rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
+    nfft = int(nfft)
+    hop = int(hop or nfft)
+    nat.require_device()
+    ch = ddc_mod.Channelizer(rec.sample_rate, n_channels, decim, taps, rec.in_fmt, rec.in_scale, device)
+    try:
+        M, D, T = ch.n_channels, ch.decim, ch.n_taps
+        n_total = ch.out_count(rec.n_samples)
+        F = (n_total - nfft) // hop + 1 if n_total >= nfft else 0
+        if F == 0:
+            raise ValueError(f"recording too short: {rec.n_samples} samples give {n_total} channel outputs, fewer than "
+                             f"nfft = {nfft}")
+        pl = sp.get_plan(nfft, hop, window, FMT_CF32, 1.0, sp.DB_EPS_REFERENCE, device)
+        st = pl.stream
+        kf = max(1, (((max_chunk_samples - T) // D + 1) - nfft) // hop + 1)   # frames per chunk
+        S = (min(kf, F) - 1) * hop + nfft                                    # channel outputs of the largest chunk
+        d_raw = DeviceArray(((S - 1) * D + T,), np.complex64 if rec.in_fmt == FMT_CF32 else np.uint32, device)
+        d_y = DeviceArray((M, S), np.complex64, device)
+        d_we = DeviceArray((M, nfft), np.float64, device)
+        d_mh = DeviceArray((M, nfft), np.float32, device) if maxhold else False
+        for f0 in range(0, F, kf):
+            nf = min(kf, F - f0)
+            m0, n_y = f0 * hop, (nf - 1) * hop + nfft
+            raw = np.ascontiguousarray(rec.raw_slice(m0 * D, (n_y - 1) * D + T))
+            nat.check(nat.lib().spx_stream_sync(device, st))   # the previous chunk's kernels are done with d_raw / d_y
+            nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
+            ch.exec(DeviceView(d_raw.ptr, (raw.nbytes // d_raw.dtype.itemsize,), d_raw.dtype, device), first_sample=m0 * D,
+                    out=d_y, stream=st)
+            pl.stft(DeviceView(d_y.ptr, (M * S,), np.complex64, device), n_streams=M, stream_stride=S, n_samples=n_y,
+                    welch=d_we, maxhold=d_mh, accumulate=f0 > 0, stream=st)
+        pxx, pdb = pl.welch_finalize(DeviceView(d_we.ptr, (M * nfft,), np.float64, device), F, ch.out_rate, n_streams=M,
+                                     stream=st)
+        nat.check(nat.lib().spx_stream_sync(device, st))
+        pxx, pdb = pxx.to_host().reshape(M, nfft), pdb.to_host().reshape(M, nfft)
+        mh = d_mh.to_host() if maxhold else None
+        freqs = sp.freq_axis(nfft, ch.out_rate, 0.0)
+        chan_f = ch.channel_freqs(rec.center_freq)
+    finally:
+        ch.close()
+    lo, hi = (nfft // 4, nfft - nfft // 4) if D == M // 2 else (0, nfft)
+    band = np.ascontiguousarray(pdb[:, lo:hi])
+    meas = features.measure_batch(band, device=device)
+    out_m, out_c = [], []
+    for j, m in enumerate(meas):
+        fj = chan_f[j] + freqs[lo:hi]
+        out_m.append(cls_mod.add_hz(fj, m))
+        out_c.append(cls_mod.classify_from_measurements(fj, m, hi - lo, smooth=False))
+    return ChannelScan(chan_f, ch.out_rate, freqs, pxx, pdb, mh, F, out_m, out_c, (lo, hi))
+
+
 def psd(path_or_rec, NFFT: int = 1024, noverlap: int = 0, max_samples: Optional[int] = None, device: int = 0):
     """``plt.psd(data, NFFT=1024, Fs=sample_rate, Fc=center_freq)`` of a recording (:188): returns
     ``(Pxx, freqs)`` in matplotlib's order."""

@@ -198,7 +198,8 @@ class SpectralPlan:
     def stft(self, x, *, n_streams: int = 1, db_rows=False, wf_rows=False, spectrum=False, welch=False,
              maxhold=False, vmin: float = -100.0, vmax: float = 0.0, accumulate: bool = False,
              stream: int = 0, n_samples: Optional[int] = None, peer_outputs: int = 0, persistence=False,
-             pool=None, pool_acc=True, pool_first_frame: int = 0, _time=None) -> StftResult:
+             pool=None, pool_acc=True, pool_first_frame: int = 0, stream_stride: Optional[int] = None,
+             _time=None) -> StftResult:
         """Windowed STFT of ``x`` (1 stream, or ``n_streams`` equal-length streams laid out back to
         back).  Each output flag is False (not wanted), True (allocate) or a caller buffer to fill
         (numpy for host input, DeviceArray / CUDA tensor for device input).
@@ -213,7 +214,11 @@ class SpectralPlan:
         float64 ``[n_streams, G, nfft / B]`` accumulator (True: allocate with G = ceil((pool_first_frame + F) / K)); it
         is an accumulator like ``welch``, so calls on consecutive pieces of a capture pool into one image, and
         ``pool_finalize`` turns it into dB and levels.  It does not need ``db_rows``: without them the rows stay on the
-        GPU."""
+        GPU.
+
+        ``stream_stride``: samples between the starts of consecutive streams (default: the stream length, streams back to
+        back), e.g. the row pitch of a channel-major ``Channelizer`` output whose rows are longer than the samples used;
+        ``n_samples`` then gives the samples per stream."""
         if persistence is not False and persistence is not None and _time is not None:
             raise ValueError("persistence cannot be timed with _time (spx_stft_time runs spx_stft_exec)")
         if pool is not None:
@@ -280,7 +285,9 @@ class SpectralPlan:
         a.mem = mem
         a.in_ = in_ptr
         a.n_samples = L
-        a.stream_stride = L
+        a.stream_stride = L if stream_stride is None else int(stream_stride)
+        if a.stream_stride < L:
+            raise ValueError(f"stream_stride {a.stream_stride} < samples per stream {L}")
         a.n_streams = n_streams
         a.accumulate = 1 if accumulate else 0
         a.db_rows = nat.as_ptr(o_db)[0]

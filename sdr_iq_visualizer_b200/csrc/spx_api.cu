@@ -97,13 +97,25 @@ int DeviceCtx::carve(std::initializer_list<size_t> bytes, void** part) {
     return SPX_OK;
 }
 
-int device_ctx(int device, DeviceCtx** out) {
-    static DeviceCtx ctx[64];
+int check_device(int device) {
     int ndev = 0;
     SPX_TRY(spx_device_count(&ndev));
     if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (device < 0 || device >= ndev || device >= 64) return spx_set_error(SPX_E_INVALID, "bad device %d", device);
+    if (device < 0 || device >= ndev) return spx_set_error(SPX_E_INVALID, "device %d out of range (%d devices)", device, ndev);
     SPX_CUDA(cudaSetDevice(device));
+    return SPX_OK;
+}
+
+size_t env_bytes(const char* name, size_t fallback, long long min) {
+    const char* e = getenv(name);
+    const long long v = e ? atoll(e) : 0;
+    return v >= min ? (size_t)v : fallback;
+}
+
+int device_ctx(int device, DeviceCtx** out) {
+    static DeviceCtx ctx[64];
+    SPX_TRY(check_device(device));
+    if (device >= 64) return spx_set_error(SPX_E_INVALID, "device %d: at most 64 devices", device);
     DeviceCtx& c = ctx[device];
     std::lock_guard<std::mutex> g(c.mu);
     if (!c.st) {
@@ -114,13 +126,13 @@ int device_ctx(int device, DeviceCtx** out) {
     return SPX_OK;
 }
 
-int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out) {
-    while (pl->events.size() <= i) {
+int event_at(std::vector<cudaEvent_t>& events, size_t i, cudaEvent_t* out) {
+    while (events.size() <= i) {
         cudaEvent_t e;
         SPX_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        pl->events.push_back(e);
+        events.push_back(e);
     }
-    *out = pl->events[i];
+    *out = events[i];
     return SPX_OK;
 }
 
@@ -365,8 +377,8 @@ static int stft_exec_host(spx_plan* pl, spx_stft_args* a, long long F, const Row
             if (hi == L) f_hi = F;
             if (f_hi <= f_lo) continue;
             cudaEvent_t e_in, e_k;
-            SPX_TRY(plan_event(pl, ev++, &e_in));
-            SPX_TRY(plan_event(pl, ev++, &e_k));
+            SPX_TRY(event_at(pl->events, ev++, &e_in));
+            SPX_TRY(event_at(pl->events, ev++, &e_k));
             SPX_CUDA(cudaEventRecord(e_in, pl->s_h2d));
             SPX_CUDA(cudaStreamWaitEvent(pl->s_compute, e_in, 0));
             NvtxRange r_k("spx STFT kernel piece");
@@ -469,8 +481,8 @@ static int stft_exec_device_peer(spx_plan* pl, spx_stft_args* a, long long F, cu
     }
     cudaEvent_t e_k[2], e_c[2];
     for (int i = 0; i < 2; ++i) {
-        SPX_TRY(plan_event(pl, (size_t)i, &e_k[i]));
-        SPX_TRY(plan_event(pl, (size_t)(2 + i), &e_c[i]));
+        SPX_TRY(event_at(pl->events, (size_t)i, &e_k[i]));
+        SPX_TRY(event_at(pl->events, (size_t)(2 + i), &e_c[i]));
     }
     const StftOut local{nullptr, a->wf_rows, nullptr, w_local, m_local, a->vmin, a->vmax};
     long long idx = 0;
@@ -685,28 +697,18 @@ int spx_plan_create(spx_plan** out, const spx_plan_config* cfg) {
     if (cfg->in_fmt != SPX_FMT_CF32 && cfg->in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt %d", cfg->in_fmt);
     if (cfg->variant != 0 && cfg->variant != 1 && cfg->variant != 12 && cfg->variant != 22)
         return spx_set_error(SPX_E_INVALID, "unknown variant %d: accepted values are 0, 1, 12 and 22 (see spx.h)", cfg->variant);
-    int ndev = 0;
-    SPX_TRY(spx_device_count(&ndev));
-    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (cfg->device < 0 || cfg->device >= ndev) return spx_set_error(SPX_E_INVALID, "device %d out of range (%d devices)", cfg->device, ndev);
-    SPX_CUDA(cudaSetDevice(cfg->device));
+    SPX_TRY(check_device(cfg->device));
 
     spx_plan* pl = new (std::nothrow) spx_plan();
     if (!pl) return spx_set_error(SPX_E_NOMEM, "out of host memory");
     pl->cfg = *cfg;
     if (!(pl->cfg.in_scale != 0.0f)) pl->cfg.in_scale = 1.0f;
-    if (const char* e = getenv("SPX_PEER_PIECE_BYTES")) { long long v = atoll(e); if (v >= 4096) pl->peer_piece_bytes = (size_t)v; }
-    if (const char* e = getenv("SPX_H2D_PIECE_BYTES")) { long long v = atoll(e); if (v >= 65536) pl->piece_bytes = (size_t)v; }
-    if (const char* e = getenv("SPX_BIG_SCRATCH_BYTES")) { long long v = atoll(e); if (v >= (1 << 20)) pl->big_scratch_bytes = (size_t)v; }
-    if (const char* e = getenv("SPX_PERSIST_ROWS_BYTES")) {   // at least one row
-        long long v = atoll(e);
-        if (v > 0) pl->persist_rows_bytes = (size_t)v > (size_t)cfg->nfft ? (size_t)v : (size_t)cfg->nfft;
-    }
-    if (const char* e = getenv("SPX_POOL_ROWS_BYTES")) {   // at least one row
-        long long v = atoll(e);
-        const size_t row = (size_t)cfg->nfft * sizeof(float);
-        if (v > 0) pl->pool_rows_bytes = (size_t)v > row ? (size_t)v : row;
-    }
+    pl->peer_piece_bytes = env_bytes("SPX_PEER_PIECE_BYTES", pl->peer_piece_bytes, 4096);
+    pl->piece_bytes = env_bytes("SPX_H2D_PIECE_BYTES", pl->piece_bytes, 65536);
+    pl->big_scratch_bytes = env_bytes("SPX_BIG_SCRATCH_BYTES", pl->big_scratch_bytes, 1 << 20);
+    // the row buffers hold at least one row
+    pl->persist_rows_bytes = std::max(env_bytes("SPX_PERSIST_ROWS_BYTES", pl->persist_rows_bytes, 1), (size_t)cfg->nfft);
+    pl->pool_rows_bytes = std::max(env_bytes("SPX_POOL_ROWS_BYTES", pl->pool_rows_bytes, 1), (size_t)cfg->nfft * sizeof(float));
     int rc = SPX_OK;
     do {
         cudaError_t e;

@@ -14,17 +14,12 @@
 //            offsets ((F - 1) D + TB samples a block); the partial folds stay in registers from block to block, so every
 //            class is summed in the same order as in the ring mode.  A sample is read about T / (F D) times, from L2.
 // The reversed taps sit in shared memory when they fit next to the ring, else they are read from global memory.
-#include <stdlib.h>
-#include <string.h>
-
 #include <mutex>
 #include <new>
-#include <vector>
 
 #include "spx_chan_device.cuh"
+#include "spx_fir.h"
 #include "spx_internal.h"
-#include "spx_pieces.h"
-#include "spx_plan.h"
 #include "spx_tables.h"
 
 namespace spx {
@@ -211,29 +206,18 @@ static const void* chan_kernel_ptr(int M) {
 
 using namespace spx;
 
-struct spx_chan {
-    spx_chan_config cfg{};
-    int sm_count = 0, occ = 1;
-    const void* kern = nullptr;
-    float* d_taps = nullptr;    // reversed, float32
+struct spx_chan : FirHandle {
+    int n_channels = 0, occ = 1;
     float2* d_tw = nullptr;     // M-point twiddle table
     ChanLaunch launch{};
-    cudaStream_t s_compute = nullptr, s_h2d = nullptr, s_d2h = nullptr;
-    std::vector<cudaEvent_t> events;
-    size_t piece_bytes = 16u << 20;   // H2D piece of the host path (SPX_H2D_PIECE_BYTES)
-    DevBuf st_in, st_out;
-    std::mutex mu;
 };
 
 namespace spx {
 
-static long long chan_out_count(long long L, int T, int D) { return L < T ? 0 : (L - T) / D + 1; }
-
 // K10 over samples [0, L) of `in` (device), global index of sample 0 = n0, outputs -> out[M][out_stride] (device)
 static int chan_launch(spx_chan* h, const void* in, long long L, unsigned long long n0, float2* out, long long out_stride,
                        cudaStream_t st) {
-    const int T = h->cfg.n_taps, D = h->cfg.decim;
-    const long long n_out = chan_out_count(L, T, D);
+    const long long n_out = h->out_count(L);
     if (n_out <= 0) return SPX_OK;
     const ChanLaunch& G = h->launch;
     ChanParams p;
@@ -246,9 +230,9 @@ static int chan_launch(spx_chan* h, const void* in, long long L, unsigned long l
     p.out_stride = out_stride;
     p.n_out = n_out;
     p.n_sub = (n_out + G.F - 1) / G.F;
-    p.scale = h->cfg.in_scale;
-    p.T = T;
-    p.D = D;
+    p.scale = h->in_scale;
+    p.T = h->n_taps;
+    p.D = h->decim;
     p.F = G.F;
     p.ring = G.ring;
     p.taps_smem = G.taps_smem;
@@ -260,17 +244,15 @@ static int chan_launch(spx_chan* h, const void* in, long long L, unsigned long l
     return SPX_OK;
 }
 
-// Host memory: pieces of about piece_bytes of input (host_pieces, spx_pieces.h).  Piece k's [M][per] block goes to one of
+// Host memory: pieces of about piece_bytes of input (FirHandle::host_pieces).  Piece k's [M][per] block goes to one of
 // two device buffers and drains into the caller's [M][out_stride] rows with one 2-D copy.
 static int chan_exec_host(spx_chan* h, const void* in, long long n_out, unsigned long long n0, float2* out,
                           long long out_stride, int64_t* h2d_out, int64_t* d2h_out) {
-    const int T = h->cfg.n_taps, D = h->cfg.decim, M = h->cfg.n_channels;
-    const size_t elt = h->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
-    const long long per = piece_outputs(h->piece_bytes, elt, T, D, n_out);
+    const int M = h->n_channels;
+    const long long per = h->piece_outputs(n_out);
     const size_t block = (size_t)M * (size_t)per;
     SPX_TRY(h->st_out.reserve(2 * block * 8));
     float2* d_out[2] = {(float2*)h->st_out.ptr, (float2*)h->st_out.ptr + block};
-    const HostPieces hp{h->s_h2d, h->s_compute, h->s_d2h, &h->events, &h->st_in, h->piece_bytes, true};
     auto launch = [&](const void* d_in, long long n, long long a, long long, long long, int b, cudaStream_t st) {
         return chan_launch(h, d_in, n, n0 + (unsigned long long)a, d_out[b], per, st);
     };
@@ -280,7 +262,15 @@ static int chan_exec_host(spx_chan* h, const void* in, long long n_out, unsigned
         *bytes = nm * 8 * (long long)M;
         return SPX_OK;
     };
-    return host_pieces(hp, in, elt, T, D, n_out, per, launch, drain, h2d_out, d2h_out);
+    return h->host_pieces(in, n_out, per, true, launch, drain, h2d_out, d2h_out);
+}
+
+// the twiddle table, and the occupancy that caps the grid (after FirHandle::setup raised the kernel's limit)
+static int chan_setup(spx_chan* h) {
+    SPX_TRY(upload(&h->d_tw, build_twiddles(h->n_channels)));
+    SPX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->occ, h->kern, h->launch.threads, h->launch.smem));
+    if (h->occ < 1) h->occ = 1;
+    return SPX_OK;
 }
 
 }  // namespace spx
@@ -301,42 +291,17 @@ int spx_chan_create(spx_chan** out, const spx_chan_config* cfg) {
         return spx_set_error(SPX_E_INVALID, "n_taps %d must be in [1, 32 n_channels = %d]", cfg->n_taps, 32 * M);
     if (!cfg->taps) return spx_set_error(SPX_E_INVALID, "taps is NULL");
     if (cfg->in_fmt != SPX_FMT_CF32 && cfg->in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt %d", cfg->in_fmt);
-    int ndev = 0;
-    SPX_TRY(spx_device_count(&ndev));
-    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (cfg->device < 0 || cfg->device >= ndev) return spx_set_error(SPX_E_INVALID, "device %d out of range (%d devices)", cfg->device, ndev);
-    SPX_CUDA(cudaSetDevice(cfg->device));
     int max_smem = 0, sms = 0;
-    SPX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device));
-    SPX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device));
+    SPX_TRY(fir_device(cfg->device, &max_smem, &sms));
     ChanLaunch launch;
     chan_plan_launch(M, cfg->n_taps, cfg->decim, max_smem, &launch);
     spx_chan* h = new (std::nothrow) spx_chan();
     if (!h) return spx_set_error(SPX_E_NOMEM, "out of host memory");
-    h->cfg = *cfg;
-    h->cfg.taps = nullptr;   // the handle keeps its own float32 copy
-    if (!(h->cfg.in_scale != 0.0f)) h->cfg.in_scale = 1.0f;
-    h->sm_count = sms;
+    h->n_channels = M;
     h->launch = launch;
-    h->kern = cfg->in_fmt == SPX_FMT_CI16 ? chan_kernel_ptr<SPX_FMT_CI16>(M) : chan_kernel_ptr<SPX_FMT_CF32>(M);
-    if (const char* e = getenv("SPX_H2D_PIECE_BYTES")) { long long v = atoll(e); if (v >= 65536) h->piece_bytes = (size_t)v; }
-    int rc = SPX_OK;
-    do {
-        cudaError_t e;
-        std::vector<float> g((size_t)cfg->n_taps);
-        for (int j = 0; j < cfg->n_taps; ++j) g[(size_t)j] = (float)cfg->taps[cfg->n_taps - 1 - j];   // rounded once
-        const std::vector<float2> tw = build_twiddles(M);
-        if ((e = cudaMalloc(&h->d_taps, g.size() * sizeof(float))) != cudaSuccess ||
-            (e = cudaMalloc(&h->d_tw, tw.size() * sizeof(float2))) != cudaSuccess) { rc = spx_set_error(SPX_E_NOMEM, "%s", cudaGetErrorString(e)); break; }
-        if ((e = cudaMemcpy(h->d_taps, g.data(), g.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess ||
-            (e = cudaMemcpy(h->d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-        if ((e = cudaFuncSetAttribute(h->kern, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)) != cudaSuccess ||
-            (e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->occ, h->kern, launch.threads, launch.smem)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-        if (h->occ < 1) h->occ = 1;
-        if ((e = cudaStreamCreateWithFlags(&h->s_compute, cudaStreamNonBlocking)) != cudaSuccess ||
-            (e = cudaStreamCreateWithFlags(&h->s_h2d, cudaStreamNonBlocking)) != cudaSuccess ||
-            (e = cudaStreamCreateWithFlags(&h->s_d2h, cudaStreamNonBlocking)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-    } while (0);
+    const void* kern = cfg->in_fmt == SPX_FMT_CI16 ? chan_kernel_ptr<SPX_FMT_CI16>(M) : chan_kernel_ptr<SPX_FMT_CF32>(M);
+    int rc = h->setup(*cfg, kern, max_smem, sms);
+    if (rc == SPX_OK) rc = chan_setup(h);
     if (rc != SPX_OK) {
         spx_chan_destroy(h);
         return rc;
@@ -347,54 +312,29 @@ int spx_chan_create(spx_chan** out, const spx_chan_config* cfg) {
 
 int spx_chan_destroy(spx_chan* h) {
     if (!h) return SPX_OK;
-    cudaSetDevice(h->cfg.device);
-    for (cudaStream_t s : {h->s_compute, h->s_h2d, h->s_d2h})
-        if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
-    for (cudaEvent_t e : h->events) cudaEventDestroy(e);
-    if (h->d_taps) cudaFree(h->d_taps);
+    h->release();
     if (h->d_tw) cudaFree(h->d_tw);
-    h->st_in.release();
-    h->st_out.release();
     delete h;
     return SPX_OK;
 }
 
 int spx_chan_sync(spx_chan* h) {
     if (!h) return spx_set_error(SPX_E_INVALID, "channelizer is NULL");
-    std::lock_guard<std::mutex> g(h->mu);
-    SPX_CUDA(cudaSetDevice(h->cfg.device));
-    SPX_CUDA(cudaStreamSynchronize(h->s_h2d));
-    SPX_CUDA(cudaStreamSynchronize(h->s_compute));
-    SPX_CUDA(cudaStreamSynchronize(h->s_d2h));
-    return SPX_OK;
+    return h->sync();
 }
 
 int spx_chan_exec(spx_chan* h, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
                   int64_t out_stride, int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream) {
     if (!h) return spx_set_error(SPX_E_INVALID, "channelizer is NULL");
-    if (mem != SPX_MEM_HOST && mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", mem);
-    if (n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
-    if (first_sample < 0) return spx_set_error(SPX_E_INVALID, "first_sample < 0");
-    const long long M = chan_out_count(n_samples, h->cfg.n_taps, h->cfg.decim);
-    if (n_out) *n_out = M;
-    if (h2d_bytes_out) *h2d_bytes_out = 0;
-    if (d2h_bytes_out) *d2h_bytes_out = 0;
+    long long M = 0;
+    std::unique_lock<std::mutex> lock;
+    SPX_TRY(h->exec_begin(mem, in, n_samples, first_sample, out, 8, &M, n_out, h2d_bytes_out, d2h_bytes_out, &lock));
     if (M == 0) return SPX_OK;
     if (out_stride < M) return spx_set_error(SPX_E_INVALID, "out_stride %lld < n_out %lld", (long long)out_stride, M);
-    if (!out) return spx_set_error(SPX_E_INVALID, "out is NULL");
-    if (!in) return spx_set_error(SPX_E_INVALID, "in is NULL");
-    if (((uintptr_t)in & 3u) || ((uintptr_t)out & 7u))
-        return spx_set_error(SPX_E_INVALID, "in must be 4-byte and out 8-byte aligned");
-    std::lock_guard<std::mutex> g(h->mu);
-    SPX_CUDA(cudaSetDevice(h->cfg.device));
     if (mem == SPX_MEM_DEVICE)
         return chan_launch(h, in, n_samples, (unsigned long long)first_sample, (float2*)out, out_stride,
                            stream ? (cudaStream_t)stream : h->s_compute);
-    int64_t h2d = 0, d2h = 0;
-    SPX_TRY(chan_exec_host(h, in, M, (unsigned long long)first_sample, (float2*)out, out_stride, &h2d, &d2h));
-    if (h2d_bytes_out) *h2d_bytes_out = h2d;
-    if (d2h_bytes_out) *d2h_bytes_out = d2h;
-    return SPX_OK;
+    return chan_exec_host(h, in, M, (unsigned long long)first_sample, (float2*)out, out_stride, h2d_bytes_out, d2h_bytes_out);
 }
 
 }  // extern "C"

@@ -9,17 +9,12 @@
 // window that slides over the outputs (spx_ddc_device.cuh), so one shared load of a sample and one of a tap feed 32
 // FMAs.  A reduce-scatter over the lanes leaves output l / 2, component l % 2 in lane l; WR warps that split the tap
 // classes of the same outputs are added in a fixed order before the store.
-#include <stdlib.h>
-#include <string.h>
-
 #include <mutex>
 #include <new>
-#include <vector>
 
 #include "spx_ddc_device.cuh"
+#include "spx_fir.h"
 #include "spx_internal.h"
-#include "spx_pieces.h"
-#include "spx_plan.h"
 
 namespace spx {
 
@@ -242,41 +237,31 @@ static int ddc_plan_launch(int T, int D, int max_smem, DdcLaunch* out) {
 
 using namespace spx;
 
-struct spx_ddc {
-    spx_ddc_config cfg{};
-    int sm_count = 0, max_smem = 0;
-    float* d_taps = nullptr;   // reversed, float32
+struct spx_ddc : FirHandle {
+    unsigned long long phase_inc = 0;
     DdcLaunch launch{};
-    cudaStream_t s_compute = nullptr, s_h2d = nullptr, s_d2h = nullptr;
-    std::vector<cudaEvent_t> events;
-    size_t piece_bytes = 16u << 20;   // H2D piece of the host path (SPX_H2D_PIECE_BYTES)
-    DevBuf st_in, st_out;
-    std::mutex mu;
 };
 
 namespace spx {
 
-static long long ddc_out_count(long long L, int T, int D) { return L < T ? 0 : (L - T) / D + 1; }
-
 // K9 over samples [0, L) of `in` (device), global index of sample 0 = n0, outputs -> out (device)
 static int ddc_launch(spx_ddc* d, const void* in, long long L, unsigned long long n0, float* out, cudaStream_t st) {
-    const int T = d->cfg.n_taps, D = d->cfg.decim;
-    const long long M = ddc_out_count(L, T, D);
+    const long long M = d->out_count(L);
     if (M <= 0) return SPX_OK;
     const DdcLaunch& G = d->launch;
     DdcParams p;
     p.in = in;
     p.L = L;
     p.n0 = n0;
-    p.inc = (unsigned long long)d->cfg.phase_inc;
+    p.inc = d->phase_inc;
     p.taps = d->d_taps;
     p.out = out;
     p.M = M;
     p.sub = G.sub;
     p.n_sub = (M + G.sub - 1) / G.sub;
-    p.scale = d->cfg.in_scale;
-    p.T = T;
-    p.D = D;
+    p.scale = d->in_scale;
+    p.T = d->n_taps;
+    p.D = d->decim;
     p.ring = G.ring;
     p.taps_pad = G.taps_pad;
     p.s = G.G.s;
@@ -286,23 +271,17 @@ static int ddc_launch(spx_ddc* d, const void* in, long long L, unsigned long lon
     const int per_sm = G.smem <= DDC_SMEM_TWO_PER_SM ? 2 : 1;
     const long long cap = (long long)per_sm * (d->sm_count > 0 ? d->sm_count : 148);
     const unsigned grid = (unsigned)(p.n_sub < cap ? p.n_sub : cap);
-    if (d->cfg.in_fmt == SPX_FMT_CI16)
-        ddc_kernel<SPX_FMT_CI16><<<grid, DDC_THREADS, G.smem, st>>>(p);
-    else
-        ddc_kernel<SPX_FMT_CF32><<<grid, DDC_THREADS, G.smem, st>>>(p);
-    SPX_CUDA(cudaGetLastError());
+    void* args[] = {&p};
+    SPX_CUDA(cudaLaunchKernel(d->kern, dim3(grid), dim3(DDC_THREADS), args, G.smem, st));
     return SPX_OK;
 }
 
-// Host memory: pieces of about piece_bytes of input (host_pieces, spx_pieces.h); the outputs land in one device buffer
-// and each piece's outputs drain on s_d2h.
+// Host memory: pieces of about piece_bytes of input (FirHandle::host_pieces); the outputs land in one device buffer and
+// each piece's outputs drain on s_d2h.
 static int ddc_exec_host(spx_ddc* d, const void* in, long long M, unsigned long long n0, float* out, int64_t* h2d_out,
                          int64_t* d2h_out) {
-    const int T = d->cfg.n_taps, D = d->cfg.decim;
-    const size_t elt = d->cfg.in_fmt == SPX_FMT_CI16 ? 4 : 8;
     SPX_TRY(d->st_out.reserve((size_t)M * 8));
     float* d_out = (float*)d->st_out.ptr;
-    const HostPieces hp{d->s_h2d, d->s_compute, d->s_d2h, &d->events, &d->st_in, d->piece_bytes, false};
     auto launch = [&](const void* d_in, long long n, long long a, long long m0, long long, int, cudaStream_t st) {
         return ddc_launch(d, d_in, n, n0 + (unsigned long long)a, d_out + 2 * m0, st);
     };
@@ -311,7 +290,7 @@ static int ddc_exec_host(spx_ddc* d, const void* in, long long M, unsigned long 
         *bytes = nm * 8;
         return SPX_OK;
     };
-    return host_pieces(hp, in, elt, T, D, M, piece_outputs(d->piece_bytes, elt, T, D, M), launch, drain, h2d_out, d2h_out);
+    return d->host_pieces(in, M, d->piece_outputs(M), false, launch, drain, h2d_out, d2h_out);
 }
 
 }  // namespace spx
@@ -330,38 +309,16 @@ int spx_ddc_create(spx_ddc** out, const spx_ddc_config* cfg) {
                              "shift 0", cfg->n_taps, DDC_MAX_TAPS);
     if (!cfg->taps) return spx_set_error(SPX_E_INVALID, "taps is NULL");
     if (cfg->in_fmt != SPX_FMT_CF32 && cfg->in_fmt != SPX_FMT_CI16) return spx_set_error(SPX_E_INVALID, "unknown in_fmt %d", cfg->in_fmt);
-    int ndev = 0;
-    SPX_TRY(spx_device_count(&ndev));
-    if (ndev == 0) return spx_set_error(SPX_E_NODEVICE, "no CUDA device (libspx has no CPU fallback)");
-    if (cfg->device < 0 || cfg->device >= ndev) return spx_set_error(SPX_E_INVALID, "device %d out of range (%d devices)", cfg->device, ndev);
-    SPX_CUDA(cudaSetDevice(cfg->device));
     int max_smem = 0, sms = 0;
-    SPX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device));
-    SPX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device));
+    SPX_TRY(fir_device(cfg->device, &max_smem, &sms));
     DdcLaunch launch;
     SPX_TRY(ddc_plan_launch(cfg->n_taps, cfg->decim, max_smem, &launch));
     spx_ddc* d = new (std::nothrow) spx_ddc();
     if (!d) return spx_set_error(SPX_E_NOMEM, "out of host memory");
-    d->cfg = *cfg;
-    d->cfg.taps = nullptr;   // the handle keeps its own float32 copy
-    if (!(d->cfg.in_scale != 0.0f)) d->cfg.in_scale = 1.0f;
-    d->sm_count = sms;
-    d->max_smem = max_smem;
+    d->phase_inc = (unsigned long long)cfg->phase_inc;
     d->launch = launch;
-    if (const char* e = getenv("SPX_H2D_PIECE_BYTES")) { long long v = atoll(e); if (v >= 65536) d->piece_bytes = (size_t)v; }
-    int rc = SPX_OK;
-    do {
-        cudaError_t e;
-        std::vector<float> g((size_t)cfg->n_taps);
-        for (int j = 0; j < cfg->n_taps; ++j) g[(size_t)j] = (float)cfg->taps[cfg->n_taps - 1 - j];   // rounded once
-        if ((e = cudaMalloc(&d->d_taps, g.size() * sizeof(float))) != cudaSuccess) { rc = spx_set_error(SPX_E_NOMEM, "%s", cudaGetErrorString(e)); break; }
-        if ((e = cudaMemcpy(d->d_taps, g.data(), g.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-        if ((e = cudaFuncSetAttribute(ddc_kernel<SPX_FMT_CF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)) != cudaSuccess ||
-            (e = cudaFuncSetAttribute(ddc_kernel<SPX_FMT_CI16>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-        if ((e = cudaStreamCreateWithFlags(&d->s_compute, cudaStreamNonBlocking)) != cudaSuccess ||
-            (e = cudaStreamCreateWithFlags(&d->s_h2d, cudaStreamNonBlocking)) != cudaSuccess ||
-            (e = cudaStreamCreateWithFlags(&d->s_d2h, cudaStreamNonBlocking)) != cudaSuccess) { rc = spx_set_error(SPX_E_CUDA, "%s", cudaGetErrorString(e)); break; }
-    } while (0);
+    const void* kern = cfg->in_fmt == SPX_FMT_CI16 ? (const void*)ddc_kernel<SPX_FMT_CI16> : (const void*)ddc_kernel<SPX_FMT_CF32>;
+    const int rc = d->setup(*cfg, kern, max_smem, sms);
     if (rc != SPX_OK) {
         spx_ddc_destroy(d);
         return rc;
@@ -372,50 +329,26 @@ int spx_ddc_create(spx_ddc** out, const spx_ddc_config* cfg) {
 
 int spx_ddc_destroy(spx_ddc* d) {
     if (!d) return SPX_OK;
-    cudaSetDevice(d->cfg.device);
-    for (cudaStream_t s : {d->s_compute, d->s_h2d, d->s_d2h})
-        if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
-    for (cudaEvent_t e : d->events) cudaEventDestroy(e);
-    if (d->d_taps) cudaFree(d->d_taps);
-    d->st_in.release();
-    d->st_out.release();
+    d->release();
     delete d;
     return SPX_OK;
 }
 
 int spx_ddc_sync(spx_ddc* d) {
     if (!d) return spx_set_error(SPX_E_INVALID, "ddc is NULL");
-    std::lock_guard<std::mutex> g(d->mu);
-    SPX_CUDA(cudaSetDevice(d->cfg.device));
-    SPX_CUDA(cudaStreamSynchronize(d->s_h2d));
-    SPX_CUDA(cudaStreamSynchronize(d->s_compute));
-    SPX_CUDA(cudaStreamSynchronize(d->s_d2h));
-    return SPX_OK;
+    return d->sync();
 }
 
 int spx_ddc_exec(spx_ddc* d, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
                  int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream) {
     if (!d) return spx_set_error(SPX_E_INVALID, "ddc is NULL");
-    if (mem != SPX_MEM_HOST && mem != SPX_MEM_DEVICE) return spx_set_error(SPX_E_INVALID, "unknown mem %d", mem);
-    if (n_samples < 0) return spx_set_error(SPX_E_INVALID, "n_samples < 0");
-    if (first_sample < 0) return spx_set_error(SPX_E_INVALID, "first_sample < 0");
-    const long long M = ddc_out_count(n_samples, d->cfg.n_taps, d->cfg.decim);
-    if (n_out) *n_out = M;
-    if (h2d_bytes_out) *h2d_bytes_out = 0;
-    if (d2h_bytes_out) *d2h_bytes_out = 0;
+    long long M = 0;
+    std::unique_lock<std::mutex> lock;
+    SPX_TRY(d->exec_begin(mem, in, n_samples, first_sample, out, 4, &M, n_out, h2d_bytes_out, d2h_bytes_out, &lock));
     if (M == 0) return SPX_OK;
-    if (!out) return spx_set_error(SPX_E_INVALID, "out is NULL");
-    if (!in) return spx_set_error(SPX_E_INVALID, "in is NULL");
-    if (((uintptr_t)in & 3u) || ((uintptr_t)out & 3u)) return spx_set_error(SPX_E_INVALID, "in and out must be 4-byte aligned");
-    std::lock_guard<std::mutex> g(d->mu);
-    SPX_CUDA(cudaSetDevice(d->cfg.device));
     if (mem == SPX_MEM_DEVICE)
         return ddc_launch(d, in, n_samples, (unsigned long long)first_sample, out, stream ? (cudaStream_t)stream : d->s_compute);
-    int64_t h2d = 0, d2h = 0;
-    SPX_TRY(ddc_exec_host(d, in, M, (unsigned long long)first_sample, out, &h2d, &d2h));
-    if (h2d_bytes_out) *h2d_bytes_out = h2d;
-    if (d2h_bytes_out) *d2h_bytes_out = d2h;
-    return SPX_OK;
+    return ddc_exec_host(d, in, M, (unsigned long long)first_sample, out, h2d_bytes_out, d2h_bytes_out);
 }
 
 }  // extern "C"

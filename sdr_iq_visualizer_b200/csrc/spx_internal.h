@@ -33,6 +33,12 @@ struct NvtxRange {
         if (_rc != SPX_OK) return _rc; \
     } while (0)
 
+// SPX_E_NODEVICE without a CUDA device, SPX_E_INVALID unless 0 <= device < device count; else makes `device` current.
+int check_device(int device);
+
+// The byte size in environment variable `name` when it is set and at least `min` (>= 1), else `fallback`.
+size_t env_bytes(const char* name, size_t fallback, long long min);
+
 // Blocks of `kern` resident per SM at `threads` threads and `smem` bytes of dynamic shared memory on the current
 // device (occ may be NULL); the first call per kernel and device raises the kernel's dynamic shared-memory limit to smem.
 int kernel_setup(const void* kern, int threads, size_t smem, int* occ);

@@ -82,7 +82,8 @@ struct spx_plan {
 };
 
 namespace spx {
-int plan_event(spx_plan* pl, size_t i, cudaEvent_t* out);
+// *out = events[i], creating events up to i on demand
+int event_at(std::vector<cudaEvent_t>& events, size_t i, cudaEvent_t* out);
 // Plan-owned scratch (K2 halves, the K2v2 scratch and its counters, the Bluestein buffers) is shared by every call on the
 // plan, whatever stream it runs on.  A call that uses it brackets its kernels on `st`: scratch_wait makes `st` wait for
 // the last such call if that one ran on another stream, scratch_record marks `st` as the stream now using it.

@@ -75,9 +75,77 @@ def phase_increment(shift_hz: float, sample_rate: float) -> tuple:
     return int(inc), float(Fraction(inc) * fs / (1 << 64))
 
 
-class DdcPlan:
+class _FirHandle:
+    """What ``DdcPlan`` and ``Channelizer`` share: the lifetime of a libspx FIR handle (``spx_<_native>_*``), ``sync``,
+    the output count and the part of ``exec`` that marshals the input and calls libspx."""
+    _native = ""   # the handle's libspx name: "ddc" or "chan"
+
+    def _fn(self, name: str):
+        return getattr(nat.lib(), f"spx_{self._native}_{name}")
+
+    def _create(self, cfg) -> None:
+        self._h = None
+        nat.require_device()
+        h = C.c_void_p()
+        nat.check(self._fn("create")(C.byref(h), C.byref(cfg)))
+        self._h = h
+
+    @property
+    def n_taps(self) -> int:
+        return int(self.taps.size)
+
+    @property
+    def out_rate(self) -> float:
+        return self.sample_rate / self.decim
+
+    def out_count(self, n_samples: int) -> int:
+        """(n - T) // decim + 1 outputs (per channel) of n input samples (0 if n < T)."""
+        n = int(n_samples)
+        return 0 if n < self.n_taps else (n - self.n_taps) // self.decim + 1
+
+    def close(self) -> None:
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            self._fn("destroy")(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def sync(self) -> None:
+        nat.check(self._fn("sync")(self._h))
+
+    def _exec(self, x, out, first_sample, stream, n_samples):
+        """exec of either handle; the subclass's ``_output(out, mem, n_out)`` allocates or checks the output and returns
+        it with the libspx arguments that follow it."""
+        if int(first_sample) < 0:
+            raise ValueError("first_sample must be >= 0")
+        if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
+            x = SpectralPlan._host_input(self, x)
+        in_ptr, mem = nat.as_ptr(x)
+        L = int(n_samples) if n_samples is not None else SpectralPlan._samples_per_stream(self, x, 1)
+        if out is not True and nat.as_ptr(out)[1] != mem:
+            raise ValueError("out must live where the input lives")
+        out, out_args = self._output(out, mem, self.out_count(L))
+        n, h2d, d2h = C.c_int64(), C.c_int64(), C.c_int64()
+        nat.check(self._fn("exec")(self._h, mem, in_ptr, L, int(first_sample), nat.as_ptr(out)[0], *out_args, C.byref(n),
+                                   C.byref(h2d), C.byref(d2h), stream or None))
+        self.last_h2d_bytes, self.last_d2h_bytes = int(h2d.value), int(d2h.value)
+        return out
+
+
+class DdcPlan(_FirHandle):
     """NCO mix by ``-shift_hz``, FIR ``taps`` (default ``design_taps(decim)``) and decimation by ``decim`` of a
     ``sample_rate`` stream, on one GPU.  ``in_fmt`` / ``in_scale`` as in ``SpectralPlan``."""
+    _native = "ddc"
 
     def __init__(self, sample_rate: float, shift_hz: float, decim: int, taps=None, in_fmt: int = FMT_CF32,
                  in_scale: float = 1.0, device: int = 0):
@@ -93,78 +161,29 @@ class DdcPlan:
             raise ValueError(f"unknown in_fmt {in_fmt}")
         self.phase_inc, self.shift_hz = phase_increment(shift_hz, self.sample_rate)
         self.in_fmt, self.in_scale, self.device = int(in_fmt), float(in_scale), int(device)
-        self._h = None
-        nat.require_device()
-        cfg = nat.spx_ddc_config(C.sizeof(nat.spx_ddc_config), self.device, self.in_fmt, self.in_scale, self.decim,
-                                 self.n_taps, self.taps.ctypes.data, self.phase_inc)
-        h = C.c_void_p()
-        nat.check(nat.lib().spx_ddc_create(C.byref(h), C.byref(cfg)))
-        self._h = h
-
-    @property
-    def n_taps(self) -> int:
-        return int(self.taps.size)
-
-    @property
-    def out_rate(self) -> float:
-        return self.sample_rate / self.decim
+        self._create(nat.spx_ddc_config(C.sizeof(nat.spx_ddc_config), self.device, self.in_fmt, self.in_scale,
+                                        self.decim, self.n_taps, self.taps.ctypes.data, self.phase_inc))
 
     @property
     def usable_span_hz(self) -> float:
         """Alias-free span of the output around its centre with the default filter: 0.8 fs / decim."""
         return 0.8 * self.out_rate
 
-    def out_count(self, n_samples: int) -> int:
-        """M = (n - T) // decim + 1 outputs of n input samples (0 if n < T)."""
-        n = int(n_samples)
-        return 0 if n < self.n_taps else (n - self.n_taps) // self.decim + 1
-
-    def close(self) -> None:
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            nat.lib().spx_ddc_destroy(h)
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def sync(self) -> None:
-        nat.check(nat.lib().spx_ddc_sync(self._h))
-
     def exec(self, x, out=True, first_sample: int = 0, stream: int = 0, n_samples: Optional[int] = None):
         """Outputs of ``x`` (numpy: staged through pinned pieces, returns numpy; DeviceArray / CUDA tensor: enqueued on
         ``stream``, returns a DeviceArray) as complex64 [M].  ``first_sample``: the global index of x's first sample, so
         that pieces of a capture that overlap by ``n_taps - decim`` samples give the outputs of one call.  ``out``: True
         (allocate) or a caller buffer of M complex64 in x's memory space."""
-        if int(first_sample) < 0:
-            raise ValueError("first_sample must be >= 0")
-        if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
-            x = SpectralPlan._host_input(self, x)
-        in_ptr, mem = nat.as_ptr(x)
-        L = int(n_samples) if n_samples is not None else SpectralPlan._samples_per_stream(self, x, 1)
-        M = self.out_count(L)
+        return self._exec(x, out, first_sample, stream, n_samples)
+
+    def _output(self, out, mem, M):
         if out is True:
-            out = np.empty(M, np.complex64) if mem == MEM_HOST else DeviceArray((M,), np.complex64, self.device)
-        else:
-            if nat.as_ptr(out)[1] != mem:
-                raise ValueError("out must live where the input lives")
-            _check_buffer(out, (M,), np.complex64, "out")
-        n_out, h2d, d2h = C.c_int64(), C.c_int64(), C.c_int64()
-        nat.check(nat.lib().spx_ddc_exec(self._h, mem, in_ptr, L, int(first_sample), nat.as_ptr(out)[0], C.byref(n_out),
-                                         C.byref(h2d), C.byref(d2h), stream or None))
-        self.last_h2d_bytes, self.last_d2h_bytes = int(h2d.value), int(d2h.value)
-        return out
+            return (np.empty(M, np.complex64) if mem == MEM_HOST else DeviceArray((M,), np.complex64, self.device)), ()
+        _check_buffer(out, (M,), np.complex64, "out")
+        return out, ()
 
 
-class Channelizer:
+class Channelizer(_FirHandle):
     """Polyphase filter-bank channelizer (libspx K10, ``spx_chan_*``): splits a ``sample_rate`` stream into
     ``n_channels`` (M, a power of two in [16, 4096]) baseband channels in one pass on one GPU.  Channel j (fftshift order)
     is the ``DdcPlan`` at shift ``(j - M/2) fs / M`` with the same taps and decimation, centred at ``fc + (j - M/2) fs / M``
@@ -173,6 +192,7 @@ class Channelizer:
     ``decim``: M / 2 (2x oversampled, the default) or M (critically sampled).  Default taps: ``design_taps(M // 2,
     transition=0.5)`` for M / 2 (cutoff fs / M, the whole channel band |f| <= fs / (2M) alias-free) and ``design_taps(M)``
     for M (the usual compromise: |f| <= 0.4 fs / M alias-free, the channel edges roll off).  Up to 32 M caller taps."""
+    _native = "chan"
 
     def __init__(self, sample_rate: float, n_channels: int, decim: Optional[int] = None, taps=None,
                  in_fmt: int = FMT_CF32, in_scale: float = 1.0, device: int = 0):
@@ -192,51 +212,13 @@ class Channelizer:
         if in_fmt not in (FMT_CF32, FMT_CI16):
             raise ValueError(f"unknown in_fmt {in_fmt}")
         self.in_fmt, self.in_scale, self.device = int(in_fmt), float(in_scale), int(device)
-        self._h = None
-        nat.require_device()
-        cfg = nat.spx_chan_config(C.sizeof(nat.spx_chan_config), self.device, self.in_fmt, self.in_scale, M, self.decim,
-                                  self.n_taps, self.taps.ctypes.data)
-        h = C.c_void_p()
-        nat.check(nat.lib().spx_chan_create(C.byref(h), C.byref(cfg)))
-        self._h = h
-
-    @property
-    def n_taps(self) -> int:
-        return int(self.taps.size)
-
-    @property
-    def out_rate(self) -> float:
-        return self.sample_rate / self.decim
-
-    def out_count(self, n_samples: int) -> int:
-        """n_out = (n - T) // decim + 1 outputs per channel of n input samples (0 if n < T)."""
-        n = int(n_samples)
-        return 0 if n < self.n_taps else (n - self.n_taps) // self.decim + 1
+        self._create(nat.spx_chan_config(C.sizeof(nat.spx_chan_config), self.device, self.in_fmt, self.in_scale, M,
+                                         self.decim, self.n_taps, self.taps.ctypes.data))
 
     def channel_freqs(self, center_freq: float = 0.0) -> np.ndarray:
         """Centre frequency of each channel, float64 [M] in fftshift order: fc + (j - M/2) fs / M."""
         M = self.n_channels
         return center_freq + (np.arange(M) - M // 2) * (self.sample_rate / M)
-
-    def close(self) -> None:
-        h, self._h = getattr(self, "_h", None), None
-        if h:
-            nat.lib().spx_chan_destroy(h)
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def sync(self) -> None:
-        nat.check(nat.lib().spx_chan_sync(self._h))
 
     def exec(self, x, first_sample: int = 0, out=True, stream: int = 0, n_samples: Optional[int] = None):
         """Channels of ``x`` as complex64 [M][n_out] (numpy input: staged through pinned pieces, returns numpy; DeviceArray
@@ -244,27 +226,16 @@ class Channelizer:
         sample, so that pieces that overlap by ``n_taps - decim`` samples give the outputs of one call.  ``out``: True
         (allocate) or a caller buffer [M][S] complex64 with S >= n_out in x's memory space; columns n_out .. S - 1 are
         left untouched."""
-        if int(first_sample) < 0:
-            raise ValueError("first_sample must be >= 0")
-        if isinstance(x, np.ndarray) or not (isinstance(x, (DeviceArray, nat.DeviceView)) or hasattr(x, "data_ptr")):
-            x = SpectralPlan._host_input(self, x)
-        in_ptr, mem = nat.as_ptr(x)
-        L = int(n_samples) if n_samples is not None else SpectralPlan._samples_per_stream(self, x, 1)
-        M, n_out = self.n_channels, self.out_count(L)
+        return self._exec(x, out, first_sample, stream, n_samples)
+
+    def _output(self, out, mem, n_out):
+        M = self.n_channels
         if out is True:
             out = np.empty((M, n_out), np.complex64) if mem == MEM_HOST else DeviceArray((M, n_out), np.complex64,
                                                                                           self.device)
-            S = n_out
-        else:
-            if nat.as_ptr(out)[1] != mem:
-                raise ValueError("out must live where the input lives")
-            shape = tuple(out.shape)
-            if len(shape) != 2 or shape[0] != M or shape[1] < n_out:
-                raise ValueError(f"out: expected shape ({M}, S) with S >= {n_out}, got {shape}")
-            _check_buffer(out, shape, np.complex64, "out")
-            S = shape[1]
-        n, h2d, d2h = C.c_int64(), C.c_int64(), C.c_int64()
-        nat.check(nat.lib().spx_chan_exec(self._h, mem, in_ptr, L, int(first_sample), nat.as_ptr(out)[0], max(S, 1),
-                                          C.byref(n), C.byref(h2d), C.byref(d2h), stream or None))
-        self.last_h2d_bytes, self.last_d2h_bytes = int(h2d.value), int(d2h.value)
-        return out
+            return out, (max(n_out, 1),)
+        shape = tuple(out.shape)
+        if len(shape) != 2 or shape[0] != M or shape[1] < n_out:
+            raise ValueError(f"out: expected shape ({M}, S) with S >= {n_out}, got {shape}")
+        _check_buffer(out, shape, np.complex64, "out")
+        return out, (max(shape[1], 1),)

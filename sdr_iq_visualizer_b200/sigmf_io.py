@@ -334,6 +334,23 @@ def process_recording(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, 
     return out
 
 
+def _fir_chunk_runner(fir, rec, max_samples: int, st: int):
+    """``run(raw, first_sample, out)``: FIR handle ``fir`` (``ddc.DdcPlan`` or ``ddc.Channelizer``) on a host chunk
+    ``raw`` of ``rec`` (up to ``max_samples`` samples, global index of its first sample ``first_sample``) into the device
+    buffer ``out``, on the plan stream ``st``.  The chunk is staged in one device buffer of the largest chunk's bytes;
+    each run first waits for ``st``, so that the previous chunk's kernels are done with that buffer and with ``out``."""
+    from ._native import DeviceArray, DeviceView
+    nat, device = sp.nat, fir.device
+    d_raw = DeviceArray((max_samples * rec.bytes_per_sample,), np.uint8, device)
+
+    def run(raw, first_sample: int, out) -> None:
+        raw = np.ascontiguousarray(raw)
+        nat.check(nat.lib().spx_stream_sync(device, st))
+        nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
+        fir.exec(DeviceView(d_raw.ptr, raw.shape, raw.dtype, device), out=out, first_sample=first_sample, stream=st)
+    return run
+
+
 def _process_zoomed(rec, zoom, zoom_taps, nfft, hop, window, waterfall, vmin, vmax, maxhold, hist_r, max_chunk_samples,
                     device, persistence, overview, overview_mode) -> RecordingSpectra:
     """process_recording(zoom=...): each file chunk (``frame_chunks(T, D)``, halo T - D) is uploaded and down-converted
@@ -384,17 +401,13 @@ def _process_zoomed(rec, zoom, zoom_taps, nfft, hop, window, waterfall, vmin, vm
         d_acc = DeviceArray((1, -(-F // K), nfft // B), np.float64, device)
     per = max(1, (max_chunk_samples - T) // D + 1)            # outputs per file chunk, at most
     bufs = [DeviceArray((nfft - 1 + per,), np.complex64, device) for _ in range(2)]
-    d_raw = DeviceArray(((per - 1) * D + T,), np.complex64, device)   # the largest chunk, 8 bytes a sample
+    run_chunk = _fir_chunk_runner(dd, rec, (per - 1) * D + T, st)
     both = persistence and overview is not None   # pooling and persistence cannot share a call
     carry = k = f0 = 0
     for m0, nm, raw in rec.frame_chunks(T, D, max_chunk_samples):
         buf, other = bufs[k & 1], bufs[(k + 1) & 1]
         k += 1
-        raw = np.ascontiguousarray(raw)
-        nat.check(nat.lib().spx_stream_sync(device, st))   # the previous chunk's kernels are done with d_raw
-        nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
-        dd.exec(DeviceView(d_raw.ptr, raw.shape, raw.dtype, device),
-                out=DeviceView(buf.ptr + 8 * carry, (nm,), np.complex64, device), first_sample=m0 * D, stream=st)
+        run_chunk(raw, m0 * D, DeviceView(buf.ptr + 8 * carry, (nm,), np.complex64, device))
         n_avail = carry + nm
         nf = pl.frame_count(n_avail)
         if nf > 0:
@@ -478,18 +491,14 @@ def scan_channels(path_or_rec, n_channels: int = 64, decim: Optional[int] = None
         st = pl.stream
         kf = max(1, (((max_chunk_samples - T) // D + 1) - nfft) // hop + 1)   # frames per chunk
         S = (min(kf, F) - 1) * hop + nfft                                    # channel outputs of the largest chunk
-        d_raw = DeviceArray(((S - 1) * D + T,), np.complex64 if rec.in_fmt == FMT_CF32 else np.uint32, device)
+        run_chunk = _fir_chunk_runner(ch, rec, (S - 1) * D + T, st)
         d_y = DeviceArray((M, S), np.complex64, device)
         d_we = DeviceArray((M, nfft), np.float64, device)
         d_mh = DeviceArray((M, nfft), np.float32, device) if maxhold else False
         for f0 in range(0, F, kf):
             nf = min(kf, F - f0)
             m0, n_y = f0 * hop, (nf - 1) * hop + nfft
-            raw = np.ascontiguousarray(rec.raw_slice(m0 * D, (n_y - 1) * D + T))
-            nat.check(nat.lib().spx_stream_sync(device, st))   # the previous chunk's kernels are done with d_raw / d_y
-            nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
-            ch.exec(DeviceView(d_raw.ptr, (raw.nbytes // d_raw.dtype.itemsize,), d_raw.dtype, device), first_sample=m0 * D,
-                    out=d_y, stream=st)
+            run_chunk(rec.raw_slice(m0 * D, (n_y - 1) * D + T), m0 * D, d_y)
             pl.stft(DeviceView(d_y.ptr, (M * S,), np.complex64, device), n_streams=M, stream_stride=S, n_samples=n_y,
                     welch=d_we, maxhold=d_mh, accumulate=f0 > 0, stream=st)
         pxx, pdb = pl.welch_finalize(DeviceView(d_we.ptr, (M * nfft,), np.float64, device), F, ch.out_rate, n_streams=M,

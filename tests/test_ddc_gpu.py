@@ -231,6 +231,7 @@ def test_errors():
         assert rc == nat.E_INVALID, kw
     rc, _ = create(n_taps=8192, taps=C.cast((C.c_double * 8192)(), C.c_void_p), decim=4096)
     assert rc == nat.E_UNSUPPORTED
+    assert lib.spx_ddc_create(None, None) == nat.E_INVALID
     rc, p = create()
     assert rc == nat.OK
     x = np.zeros(64, np.complex64)
@@ -242,6 +243,8 @@ def test_errors():
     assert ex(p, 0, x.ctypes.data, 64, -1, out.ctypes.data, C.byref(n), None, None, None) == nat.E_INVALID
     assert ex(p, 0, x.ctypes.data, 64, 0, None, C.byref(n), None, None, None) == nat.E_INVALID
     assert ex(p, 0, None, 64, 0, out.ctypes.data, C.byref(n), None, None, None) == nat.E_INVALID
+    assert ex(p, 0, x.ctypes.data + 2, 64, 0, out.ctypes.data, C.byref(n), None, None, None) == nat.E_INVALID
+    assert ex(p, 0, x.ctypes.data, 64, 0, out.ctypes.data + 2, C.byref(n), None, None, None) == nat.E_INVALID
     assert ex(p, 0, None, 2, 0, None, C.byref(n), None, None, None) == nat.OK and n.value == 0
     assert ex(None, 0, x.ctypes.data, 64, 0, out.ctypes.data, C.byref(n), None, None, None) == nat.E_INVALID
     assert lib.spx_ddc_sync(None) == nat.E_INVALID

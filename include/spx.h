@@ -386,22 +386,26 @@ SPX_API int spx_plan_window_sums(spx_plan* plan, double* sum_w2, double* sum_w);
 /* What classify_signal_advanced / classify_signal_simple measure on one spectrum
  * (/root/reference/app/processing/classifier.py:45-58 and :18-23; helpers :163-219).
  * Bin indices are exact; the host layer turns them into Hz with the caller's `freqs` array and
- * applies the label rules + temporal smoothing (:60-161). */
+ * applies the label rules + temporal smoothing (:60-161).
+ * Non-finite bins follow numpy: NaN (either sign bit) is the maximum and sorts after +inf; every comparison
+ * with a NaN threshold is false, so a NaN peak gives no edges and no peaks; ±inf enter the sums as numpy's do. */
 typedef struct {
     int32_t n;                 /* bins */
-    int32_t argmax;            /* first index of the maximum */
-    double peak_db;            /* np.max(power_db) (:46) */
-    double noise_floor_db;     /* np.percentile(power_db, 20), 'linear' (:181) */
+    int32_t argmax;            /* np.argmax: the first NaN if any, else the first index of the maximum (0 for all -inf) */
+    double peak_db;            /* np.max(power_db) (:46): NaN if any bin is NaN */
+    double noise_floor_db;     /* np.percentile(power_db, 20), 'linear' (:181): NaN if any bin is NaN; numpy's lerp
+                                  otherwise, so inf - inf inside it (e.g. all -inf, or n == 1 and infinite) is NaN */
     double snr_db;             /* peak - noise floor (:46), un-rounded */
-    double adaptive_thr;       /* max(nf + 5, peak - 0.9 snr + 5) (:53) */
-    double p20_lo, p20_hi;     /* the two order statistics the percentile interpolates */
+    double adaptive_thr;       /* max(nf + 5, peak - 0.9 snr + 5) (:53) with Python's max: nf + 5 unless the second
+                                  term is greater, so a NaN second term (one +inf bin) leaves nf + 5 */
+    double p20_lo, p20_hi;     /* the two order statistics the percentile interpolates, NaN sorted last */
     int32_t min_distance_bins; /* max(3, n // 300) (:54) */
     int32_t first_3db, last_3db;   /* first/last bin with p >= peak - 3  (:163-170); -1 if none */
     int32_t first_10db, last_10db;
     int32_t first_20db, last_20db;
     int32_t simple_first, simple_last; /* first/last bin with p > peak - 20 (strict, :18-21) */
     double flatness;           /* exp(mean(ln p)) / mean(p), p = max(10^(dB/10), 1e-15), clipped to [0,1] (:183-189) */
-    double kurtosis;           /* mean(((x - mu)/sigma)^4), 0 if sigma < 1e-9 (:191-198) */
+    double kurtosis;           /* mean(((x - mu)/sigma)^4), 0 if sigma < 1e-9 (:191-198); NaN if sigma is NaN */
     double mean_db, std_db;
     int32_t n_candidates;      /* strict local maxima above adaptive_thr */
     int32_t peak_count;        /* after greedy min-distance thinning (:200-212) */

@@ -103,8 +103,10 @@ __device__ void block_min8(int* v, int (*sh)[FT / 32]) {
     }
 }
 
-// order-preserving map double -> uint64
+// order-preserving map double -> uint64; every NaN, whatever its sign bit or payload, maps to the largest key, so NaN
+// sorts last as in np.sort
 __device__ __forceinline__ unsigned long long key_of(double x) {
+    if (x != x) return ~0ull;
     unsigned long long b = (unsigned long long)__double_as_longlong(x);
     return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
@@ -135,12 +137,14 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
     const int tid = threadIdx.x;
 
     // ---- pass 1: max / argmax (first occurrence), mean, flatness sums (classifier.py:46,183-189)
-    double vmax = -DBL_MAX;
+    // np.max / np.argmax: the first NaN wins over everything; otherwise the first index of the largest value.  A thread
+    // takes its first bin unconditionally, so a row of -inf gives argmax 0.
+    double vmax = -INFINITY;
     int imax = 0x7fffffff;
     double s1 = 0.0, slog = 0.0, slin = 0.0;
     for (int i = tid; i < n; i += FT) {
         const double v = (double)x[i];
-        if (v > vmax) { vmax = v; imax = i; }
+        if (imax == 0x7fffffff || (vmax == vmax && !(v <= vmax))) { vmax = v; imax = i; }
         s1 += v;
         // p = max(10^(v/10), 1e-15) and ln p (classifier.py:185-187): one exp; ln p is v ln(10)/10 unless clipped
         const double lnp = v * 0.23025850929940456840;   // ln(10)/10
@@ -153,7 +157,8 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
     // one combined block reduction: exact maximum (order-preserving 64-bit key), then first index of it, and the sums
     const unsigned long long kmax = block_max_u64(key_of(vmax), shu);
     const double peak = val_of(kmax);
-    const int argmax = (int)block_min_ll(vmax == peak ? (long long)imax : (long long)0x7fffffff, shl);
+    const bool is_max = vmax == peak || (vmax != vmax && peak != peak);
+    const int argmax = (int)block_min_ll(is_max ? (long long)imax : (long long)0x7fffffff, shl);
     double sums[3] = {s1, slog, slin};
     block_sum3(sums, shd3);
     const double sum_x = sums[0], sum_log = sums[1], sum_lin = sums[2];
@@ -183,9 +188,9 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
         l3 = -mm[4]; l10 = -mm[5]; l20 = -mm[6]; ls = -mm[7];
     }
 
-    // ---- pass 3: kurtosis (classifier.py:191-198)
+    // ---- pass 3: kurtosis (classifier.py:191-198); a NaN sigma (any non-finite bin) gives NaN, as `if sd < 1e-9` does
     double kurt = 0.0;
-    if (sd >= 1e-9) {
+    if (!(sd < 1e-9)) {
         double s4 = 0.0;
         for (int i = tid; i < n; i += FT) {
             const double z = ((double)x[i] - mu) / sd;
@@ -278,17 +283,19 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
         low = block_min_ll(low, shl);
         vhi = val_of(((unsigned long long)b1 << 1) | (unsigned long long)low);
     }
-    // numpy _lerp: a + (b-a)*t, or b - (b-a)*(1-t) when t >= 0.5 (no fused multiply-add)
+    // numpy _lerp: a + (b-a)*t, or b - (b-a)*(1-t) when t >= 0.5 (no fused multiply-add); also for n == 1, where
+    // a == b and an infinite a gives NaN as in numpy.  np.percentile is NaN when any bin is NaN, i.e. when the peak is.
     const double diff = __dsub_rn(vhi, vlo);
     double nf = __dadd_rn(vlo, __dmul_rn(diff, gamma));
     if (gamma >= 0.5) nf = __dsub_rn(vhi, __dmul_rn(diff, __dsub_rn(1.0, gamma)));
-    if (lo + 1 >= n) nf = vlo;
+    if (peak != peak) nf = peak;
 
     const double snr = __dsub_rn(peak, nf);
-    // max(nf + 5, peak - 0.9*snr + 5)  (classifier.py:53)
+    // max(nf + 5, peak - 0.9*snr + 5)  (classifier.py:53), as Python's max: the second only when it is greater, so a
+    // NaN second term (one +inf bin: inf - 0.9 inf) leaves nf + 5
     const double thr_a = __dadd_rn(nf, 5.0);
     const double thr_b = __dadd_rn(__dsub_rn(peak, __dmul_rn(0.9, snr)), 5.0);
-    double thr = thr_a > thr_b ? thr_a : thr_b;
+    double thr = thr_b > thr_a ? thr_b : thr_a;
     if (opts.use_peak_threshold) thr = opts.peak_threshold_db;
     const int min_dist = opts.min_distance_bins > 0 ? opts.min_distance_bins : max(3, n / 300);
 
@@ -315,7 +322,7 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
                     m &= m - 1;
                     const int idx = base + 32 * w + bit;
                     ++nc;
-                    if (idx - last >= min_dist) {
+                    if ((long long)idx - last >= min_dist) {   // 64-bit: last starts at -min_dist, up to -INT32_MAX
                         if (cnt > 0) { const double d = (double)(idx - last); sdv += d; sd2v += d * d; }
                         if (pk && cnt < peaks_cap) pk[cnt] = idx;
                         ++cnt;

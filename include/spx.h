@@ -436,6 +436,35 @@ SPX_API int spx_classify_features_dev(int32_t device, const void* power_db_dev, 
                                       int64_t stride, spx_features* out_dev, int32_t* peaks_dev, int32_t peaks_cap,
                                       const spx_feature_opts* opts, void* stream);
 
+/* ---------------------------------------------------------------- signal detection (regions of a dB image)
+ * For a float32 dB image db[rows][cols] (row r at db + r * stride; a row is one time slice, columns in fftshift order):
+ *   floor[r]   = np.percentile(float64(db[r]), 20): spx_features.noise_floor_db of the row, with its NaN rules (a row
+ *                holding a NaN, or all -inf, has a NaN floor)
+ *   mask[r][c] = float64(db[r][c]) >= floor[r] + threshold_db, compared in float64 (false for NaN cells and NaN floors)
+ *   regions    = scipy.ndimage.label(mask, structure=np.ones((3, 3))): 8-connected, numbered in raster order of their
+ *                first cell; regions of fewer than min_cells cells are dropped and the rest renumbered 1 .. n in that order
+ * Every field below except power_sum, the labels and the floors are exact and identical from run to run. */
+typedef struct {
+    int32_t row0, row1, col0, col1;   /* inclusive bounding box */
+    int64_t n_cells;                  /* cells in the region */
+    int32_t peak_row, peak_col;       /* the cell of the largest dB; ties -> smallest raster index (r * cols + c) */
+    double peak_db, peak_floor_db;    /* db at the peak (as float64); peak_floor_db = floor[peak_row] */
+    double power_sum;                 /* sum of 10^(dB/10) over the region's cells, float64, accumulated with float64
+                                         atomics: within ~1e-12 relative of an exact sum, but not bit-reproducible */
+} spx_region;
+
+/* Labels the regions of one image (K11).  `db` and the optional outputs `labels` (int32 [rows][cols]: region number
+ * 1 .. n, 0 for cells outside every kept region) and `row_floor_db` (float64 [rows]) are in `mem` space; `regions` and
+ * `n_regions_out` are HOST buffers in both memory modes, and the call returns after they have landed.  *n_regions_out =
+ * the total n; the first min(n, max_regions) regions, in numbering order, go to regions[].  SPX_MEM_DEVICE work runs on
+ * `stream` (NULL = the library's stream of the device).  rows == 0 or cols == 0: zero regions.
+ * SPX_E_INVALID: a bad device or mem; negative rows or cols; rows * cols > INT32_MAX (checked before anything is
+ * allocated); stride < cols; min_cells < 1; max_regions < 0; NULL db or n_regions_out; NULL regions with max_regions > 0.
+ * SPX_E_NODEVICE without a CUDA device. */
+SPX_API int spx_detect_regions(int32_t device, int32_t mem, const float* db, int32_t rows, int32_t cols, int64_t stride,
+                               double threshold_db, int32_t min_cells, spx_region* regions, int32_t max_regions,
+                               int32_t* n_regions_out, int32_t* labels, double* row_floor_db, void* stream);
+
 /* ---------------------------------------------------------------- time-domain / constellation views */
 /* 2-D I/Q density histogram with np.histogram2d(I, Q, bins, range=[[-R,R],[-R,R]]) semantics
  * (SURVEY.md A10; replaces the 2000-point scatter of app/dashboard/callbacks.py:199-214).

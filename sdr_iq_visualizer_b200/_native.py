@@ -83,6 +83,12 @@ class spx_features(C.Structure):
                 ("peaks_stored", C.c_int32), ("reserved", C.c_int32)]
 
 
+class spx_region(C.Structure):
+    _fields_ = [("row0", C.c_int32), ("row1", C.c_int32), ("col0", C.c_int32), ("col1", C.c_int32), ("n_cells", C.c_int64),
+                ("peak_row", C.c_int32), ("peak_col", C.c_int32), ("peak_db", C.c_double), ("peak_floor_db", C.c_double),
+                ("power_sum", C.c_double)]
+
+
 class spx_ring_config(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("n_slots", C.c_int32), ("slot_samples", C.c_int64),
                 ("want_wf_rows", C.c_int32), ("want_db_rows", C.c_int32), ("want_welch", C.c_int32),
@@ -155,6 +161,9 @@ _SIGNATURES = {
                                         C.c_void_p]),
     "spx_classify_features_dev": (C.c_int, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_void_p,
                                             C.c_void_p, C.c_int32, C.POINTER(spx_feature_opts), C.c_void_p]),
+    "spx_detect_regions": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_double,
+                                     C.c_int32, C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p,
+                                     C.c_void_p]),
     "spx_iq_hist2d": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_double, C.c_int64, C.c_double,
                                 C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "spx_frame_stats": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_float, C.c_int64, C.c_int32,

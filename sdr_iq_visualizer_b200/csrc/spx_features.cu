@@ -374,7 +374,7 @@ features_kernel(const T* __restrict__ data, int n, long long stride, spx_feature
 
 // features_kernel over `batch` spectra of n bins, `stride` apart, in float32 (dtype 0) or float64 (dtype 1, checked by the
 // caller); NULL user_opts: the reference's options
-static int features_launch(const void* in, int dtype, int n, int batch, long long stride, spx_features* out, int* peaks,
+int features_launch(const void* in, int dtype, int n, int batch, long long stride, spx_features* out, int* peaks,
                            int peaks_cap, const spx_feature_opts* user_opts, cudaStream_t st) {
     spx_feature_opts opts;
     memset(&opts, 0, sizeof(opts));

@@ -43,4 +43,9 @@ size_t env_bytes(const char* name, size_t fallback, long long min);
 // device (occ may be NULL); the first call per kernel and device raises the kernel's dynamic shared-memory limit to smem.
 int kernel_setup(const void* kern, int threads, size_t smem, int* occ);
 
+// K3 (features_kernel) over `batch` spectra of n bins `stride` apart, float32 (dtype 0) or float64 (dtype 1), on `st`;
+// NULL user_opts: the reference's options
+int features_launch(const void* in, int dtype, int n, int batch, long long stride, spx_features* out, int* peaks,
+                    int peaks_cap, const spx_feature_opts* user_opts, cudaStream_t st);
+
 }  // namespace spx

@@ -521,6 +521,69 @@ def scan_channels(path_or_rec, n_channels: int = 64, decim: Optional[int] = None
     return ChannelScan(chan_f, ch.out_rate, freqs, pxx, pdb, mh, F, out_m, out_c, (lo, hi))
 
 
+GENERATOR = "sdr_iq_visualizer_b200"
+
+
+def region_annotation(region: dict, frames_per_row: int, bins_per_col: int, n_frames: int, nfft: int, hop: int,
+                      sample_rate: float, center_freq: float, label: str = "signal") -> dict:
+    """The SigMF annotation of a region of an overview whose row g pools frames [gK, min((g+1)K, F)) and column c bins
+    [cB, (c+1)B) of an nfft-point STFT with hop `hop`.  Bin k covers [fc + (k - N/2 - 1/2) fs/N, fc + (k - N/2 + 1/2) fs/N);
+    the samples are those of every frame of the region's rows."""
+    K, B, F, N = int(frames_per_row), int(bins_per_col), int(n_frames), int(nfft)
+    start = int(region["row0"]) * K * int(hop)
+    last_frame = min((int(region["row1"]) + 1) * K, F) - 1
+    df = float(sample_rate) / N
+    return {
+        "core:sample_start": start,
+        "core:sample_count": last_frame * int(hop) + N - start,
+        "core:freq_lower_edge": float(center_freq) + (int(region["col0"]) * B - N / 2 - 0.5) * df,
+        "core:freq_upper_edge": float(center_freq) + ((int(region["col1"]) + 1) * B - N / 2 - 0.5) * df,
+        "core:label": label,
+        "core:comment": f"peak {region['peak_db'] - region['peak_floor_db']:.1f} dB above its row's noise floor",
+        "core:generator": GENERATOR,
+    }
+
+
+def detect_signals(path_or_rec, nfft: int = 1024, hop: Optional[int] = None, window="hann", overview: tuple = (512, 1024),
+                   overview_mode: str = "mean", threshold_db: float = 6.0, min_cells: int = 4, label: str = "signal",
+                   device: int = 0):
+    """Where in time and frequency a recording holds signals: the pooled overview of the whole file
+    (``process_recording(..., overview=overview)``), its regions at least ``threshold_db`` above each row's noise floor
+    (``detect.detect_regions``), and one SigMF annotation per region (``region_annotation``), sorted by sample_start.
+    Returns ``(Detections, annotations)``; ``write_annotations`` stores the annotations with the recording."""
+    from . import detect
+    rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
+    hop = int(hop or nfft)
+    out = process_recording(rec, nfft, hop, window, maxhold=False, overview=overview, overview_mode=overview_mode,
+                            device=device)
+    det = detect.detect_regions(out.overview_db, threshold_db, min_cells, device=device)
+    K, B = out.overview_frames_per_row, out.overview_bins_per_col
+    F = out.n_frames if out.overview_db.shape[0] else 0
+    ann = [region_annotation(r, K, B, F, nfft, hop, rec.sample_rate, rec.center_freq, label) for r in det.regions]
+    return det, sorted(ann, key=lambda a: a["core:sample_start"])
+
+
+def write_annotations(path_or_rec, annotations) -> str:
+    """Replace the ``annotations`` of a recording's ``<base>.sigmf-meta`` (sorted by core:sample_start, as SigMF asks),
+    keeping every other field; the meta file is replaced atomically and the data file is not touched."""
+    base = path_or_rec.base if isinstance(path_or_rec, SigMFRecording) else resolve_base(path_or_rec)
+    meta_path = base + ".sigmf-meta"
+    with open(meta_path, "r") as fh:
+        meta = json.load(fh)
+    meta["annotations"] = sorted((dict(a) for a in annotations), key=lambda a: a.get("core:sample_start", 0))
+    tmp = f"{meta_path}.tmp.{os.getpid()}"
+    try:
+        with open(tmp, "w") as fh:
+            json.dump(meta, fh, indent=2)
+        os.replace(tmp, meta_path)
+    finally:
+        if os.path.exists(tmp):
+            os.remove(tmp)
+    if isinstance(path_or_rec, SigMFRecording):
+        path_or_rec.meta["annotations"] = meta["annotations"]
+    return base
+
+
 def psd(path_or_rec, NFFT: int = 1024, noverlap: int = 0, max_samples: Optional[int] = None, device: int = 0):
     """``plt.psd(data, NFFT=1024, Fs=sample_rate, Fc=center_freq)`` of a recording (:188): returns
     ``(Pxx, freqs)`` in matplotlib's order."""

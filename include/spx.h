@@ -307,6 +307,32 @@ SPX_API int spx_ddc_sync(spx_ddc* ddc);
 SPX_API int spx_ddc_exec(spx_ddc* ddc, int32_t mem, const void* in, int64_t n_samples, int64_t first_sample, float* out,
                          int64_t* n_out, int64_t* h2d_bytes_out, int64_t* d2h_bytes_out, void* stream);
 
+/* Many down-conversions of one capture in one launch: each job is the DDC above with its own NCO and its own span, and all
+ * share the handle's in_fmt, in_scale, taps (T) and decimation (D).  Job j computes
+ *   y_j[m] = sum_k h[k] mix_j[first_sample_j + m D + T - 1 - k],   m = m0_j .. m0_j + n_out_j - 1
+ * where mix_j uses phase_inc_j and the global sample index exactly as spx_ddc_exec does (the handle's own phase_inc is
+ * not used), so y_j[m] has the bits of output m of spx_ddc_exec on a DDC with phase_inc_j called with
+ * first_sample = first_sample_j. */
+typedef struct {
+    int64_t first_sample;  /* global index of the job's sample 0: its output m starts at first_sample + m*D */
+    int64_t phase_inc;     /* the job's NCO, as spx_ddc_config.phase_inc */
+    int64_t m0;            /* first output of the job written by this call */
+    int64_t n_out;         /* outputs written by this call (0 allowed) */
+    int64_t out_offset;    /* output m goes to out[out_offset + m - m0] (complex, float32 I,Q) */
+} spx_ddc_job;
+
+/* The jobs over `in` (device), whose sample 0 has global index in_first_sample, into `out` (device), enqueued on `stream`
+ * (NULL = the handle's stream); nothing is synchronised.  `jobs` is host memory; it is copied to the device on `stream`
+ * through a pinned staging buffer of the handle, and may be reused once the call returns.  Every window
+ * [first_sample + m D, first_sample + m D + T) of a job must lie in [in_first_sample, in_first_sample + n_samples).
+ * Columns of out that no job writes are left untouched.  The output regions of different jobs must not overlap; this is
+ * not checked.  SPX_E_INVALID, with nothing launched, for n_samples, in_first_sample or n_jobs < 0, jobs NULL with
+ * n_jobs > 0, a job with a negative first_sample, m0, n_out or out_offset, a window outside the input, or (when some job
+ * has outputs) in or out NULL or not 4-byte aligned.  Jobs with n_out = 0 are skipped; a call without outputs launches
+ * nothing. */
+SPX_API int spx_ddc_exec_jobs(spx_ddc* ddc, const void* in, int64_t n_samples, int64_t in_first_sample,
+                              const spx_ddc_job* jobs, int32_t n_jobs, float* out, void* stream);
+
 /* ---------------------------------------------------------------- polyphase channelizer (channel scan)
  * Splits a wideband capture into M baseband channels in one pass: all M down-conversions of the DDC above at once.  With
  * the DDC's names (x = in_fmt samples times in_scale, sample n has global index first_sample + n, real taps h[0 .. T-1]),

@@ -67,6 +67,11 @@ class spx_ddc_config(C.Structure):
                 ("decim", C.c_int32), ("n_taps", C.c_int32), ("taps", C.c_void_p), ("phase_inc", C.c_int64)]
 
 
+class spx_ddc_job(C.Structure):
+    _fields_ = [("first_sample", C.c_int64), ("phase_inc", C.c_int64), ("m0", C.c_int64), ("n_out", C.c_int64),
+                ("out_offset", C.c_int64)]
+
+
 class spx_chan_config(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("device", C.c_int32), ("in_fmt", C.c_int32), ("in_scale", C.c_float),
                 ("n_channels", C.c_int32), ("decim", C.c_int32), ("n_taps", C.c_int32), ("taps", C.c_void_p)]
@@ -145,6 +150,8 @@ _SIGNATURES = {
     "spx_ddc_sync": (C.c_int, [C.c_void_p]),
     "spx_ddc_exec": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.POINTER(C.c_int64),
                                C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_void_p]),
+    "spx_ddc_exec_jobs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
+                                    C.c_void_p]),
     "spx_chan_create": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(spx_chan_config)]),
     "spx_chan_destroy": (C.c_int, [C.c_void_p]),
     "spx_chan_sync": (C.c_int, [C.c_void_p]),

@@ -91,6 +91,36 @@ __host__ __device__ inline int ddc_lane_taps(int T, int c, int lane, int rho) {
     return j0 >= T ? 0 : (T - 1 - j0) / (32 * c) + 1;
 }
 
+// Work split of a call.  The call's outputs are cut into sub-tiles of SUB outputs, and CTA b of `grid` takes the
+// contiguous run [b n / grid, (b + 1) n / grid) of the n sub-tiles.
+__host__ __device__ inline void ddc_cta_run(long long b, long long grid, long long n, long long* s0, long long* s1) {
+    *s0 = b * n / grid;
+    *s1 = (b + 1) * n / grid;
+}
+
+// Multi-job calls (spx_ddc_exec_jobs; the walk is run on the host by tests/emul/ddc_jobs_emul.cu): job j owns the global sub-tiles [tile0[j], tile0[j + 1]), ceil(n_out_j / SUB) of
+// them, and tile0[n_jobs] is their total.  The job of global sub-tile t < tile0[n_jobs] is the largest j with
+// tile0[j] <= t; a job without outputs owns no sub-tile and is never the answer.
+__host__ __device__ inline int ddc_job_of(const long long* tile0, int n_jobs, long long t) {
+    int lo = 0, hi = n_jobs;   // tile0[lo] <= t < tile0[hi]
+    while (hi - lo > 1) {
+        const int mid = lo + (hi - lo) / 2;
+        if (tile0[mid] <= t) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// The part of a CTA's run [t, t1) that lies in one job: *job, its local first sub-tile *k0, and (returned) the global
+// end of the part, where the CTA goes on with the next job.
+__host__ __device__ inline long long ddc_segment(const long long* tile0, int n_jobs, long long t, long long t1, int* job,
+                                                 long long* k0) {
+    const int j = ddc_job_of(tile0, n_jobs, t);
+    *job = j;
+    *k0 = t - tile0[j];
+    return tile0[j + 1] < t1 ? tile0[j + 1] : t1;
+}
+
 // tree sum of 32 lane partials (in place; the result is v[0])
 __host__ __device__ inline float ddc_lane_tree(float* v) {
     for (int o = 16; o >= 1; o >>= 1)

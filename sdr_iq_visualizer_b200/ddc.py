@@ -28,6 +28,9 @@ from ._native import FMT_CF32, FMT_CI16, MEM_HOST, DeviceArray
 from .spectral import SpectralPlan, _check_buffer
 
 MAX_TAPS = 8192
+# one job of DdcPlan.exec_jobs (the layout of spx_ddc_job)
+JOB_DTYPE = np.dtype([("first_sample", "<i8"), ("phase_inc", "<i8"), ("m0", "<i8"), ("n_out", "<i8"),
+                      ("out_offset", "<i8")])
 
 
 def kaiser_order(atten_db: float, width: float) -> tuple:
@@ -142,6 +145,15 @@ class _FirHandle:
         return out
 
 
+def as_jobs(jobs) -> np.ndarray:
+    """Jobs of ``DdcPlan.exec_jobs`` as a contiguous ``JOB_DTYPE`` array; ``phase_inc`` of tuples may be given mod 2^64."""
+    if isinstance(jobs, np.ndarray) and jobs.dtype == JOB_DTYPE:
+        return np.ascontiguousarray(jobs)
+    rows = [tuple(int(v) for v in j) for j in jobs]
+    rows = [(a, (p + (1 << 63)) % (1 << 64) - (1 << 63), m0, n, o) for a, p, m0, n, o in rows]
+    return np.array(rows, dtype=JOB_DTYPE).reshape(-1)
+
+
 class DdcPlan(_FirHandle):
     """NCO mix by ``-shift_hz``, FIR ``taps`` (default ``design_taps(decim)``) and decimation by ``decim`` of a
     ``sample_rate`` stream, on one GPU.  ``in_fmt`` / ``in_scale`` as in ``SpectralPlan``."""
@@ -175,6 +187,32 @@ class DdcPlan(_FirHandle):
         that pieces of a capture that overlap by ``n_taps - decim`` samples give the outputs of one call.  ``out``: True
         (allocate) or a caller buffer of M complex64 in x's memory space."""
         return self._exec(x, out, first_sample, stream, n_samples)
+
+    def exec_jobs(self, x_dev, jobs, out, in_first_sample: int = 0, stream: int = 0):
+        """Many down-conversions of one device-resident capture in one launch (``spx_ddc_exec_jobs``): every job is this
+        plan's DDC (taps, decimation, format) with its own NCO ``phase_inc`` and span.  Job ``(first_sample, phase_inc,
+        m0, n_out, out_offset)`` writes its outputs ``m0 .. m0 + n_out - 1`` (output m of ``DdcPlan.exec`` on a plan with
+        that increment called with ``first_sample``, bit for bit) to ``out[out_offset + m - m0]``.  ``x_dev``: DeviceArray /
+        DeviceView / CUDA tensor whose sample 0 has global index ``in_first_sample``; every window a job reads must lie in
+        it.  ``jobs``: a structured array of ``JOB_DTYPE`` or a list of 5-tuples.  ``out``: complex64 device buffer;
+        the outputs of different jobs must not overlap, and elements no job writes are left untouched.  Enqueued on
+        ``stream``; returns ``out``."""
+        if isinstance(x_dev, np.ndarray) or not (isinstance(x_dev, (DeviceArray, nat.DeviceView)) or hasattr(x_dev, "data_ptr")):
+            raise TypeError("exec_jobs takes device input (DeviceArray, DeviceView or a CUDA tensor)")
+        jobs = as_jobs(jobs)
+        in_ptr, _ = nat.as_ptr(x_dev)
+        L = SpectralPlan._samples_per_stream(self, x_dev, 1)
+        out_ptr, mem = nat.as_ptr(out)
+        if mem == MEM_HOST:
+            raise ValueError("out must be a device buffer")
+        live = jobs[jobs["n_out"] > 0]
+        need = int((live["out_offset"] + live["n_out"]).max()) if live.size else 0
+        have = (out.numel() * out.element_size() if hasattr(out, "data_ptr") else out.nbytes) // 8
+        if have < need:
+            raise ValueError(f"out holds {have} complex64 outputs; the jobs write up to element {need - 1}")
+        nat.check(nat.lib().spx_ddc_exec_jobs(self._h, in_ptr, L, int(in_first_sample), jobs.ctypes.data, len(jobs),
+                                              out_ptr, stream or None))
+        return out
 
     def _output(self, out, mem, M):
         if out is True:

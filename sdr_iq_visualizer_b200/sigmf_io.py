@@ -584,6 +584,217 @@ def write_annotations(path_or_rec, annotations) -> str:
     return base
 
 
+def signal_jobs(annotations, sample_rate, center_freq, n_samples, max_decim: int = 256) -> list:
+    """The down-conversion that extracts each annotated region of a recording: one ``(shift_hz, phase_inc, D,
+    first_sample, n_out)`` per annotation.  The band's centre, ``(core:freq_lower_edge + core:freq_upper_edge) / 2 -
+    center_freq``, is tuned with ``ddc.phase_increment`` (``shift_hz`` is the shift it tunes).  D is the largest power of
+    two with D <= max_decim and fs / D >= 2 bw (bw = upper - lower edge), at least 1, so that the region fills at most the
+    centre half of its baseband; the taps are ``ddc.design_taps(D)`` (T of them).  The input span is
+    ``[sample_start - (T - 1) / 2, sample_start + sample_count + (T - 1) / 2)`` clipped to ``[0, n_samples)``, so that the
+    outputs cover the annotated span, and it gives ``n_out = (len - T) // D + 1`` outputs (0 when len < T)."""
+    from . import ddc as ddc_mod
+    fs, fc, L = float(sample_rate), float(center_freq), int(n_samples)
+    max_decim = int(max_decim)
+    if max_decim < 1:
+        raise ValueError(f"max_decim {max_decim} must be >= 1")
+    top = 1 << (max_decim.bit_length() - 1)
+    n_taps = {}
+
+    def taps_of(D):
+        if D not in n_taps:
+            n_taps[D] = ddc_mod.design_taps(D).size
+        return n_taps[D]
+    if taps_of(top) > ddc_mod.MAX_TAPS:
+        raise ValueError(f"max_decim {max_decim}: the default filter of decimation {top} has {taps_of(top)} taps, more than "
+                         f"one DDC stage takes ({ddc_mod.MAX_TAPS}); 256 is the largest decimation that fits")
+    plans = []
+    for a in annotations:
+        lo, hi = float(a["core:freq_lower_edge"]), float(a["core:freq_upper_edge"])
+        inc, shift = ddc_mod.phase_increment(0.5 * (lo + hi) - fc, fs)
+        D = 1
+        while 2 * D <= top and fs / (2 * D) >= 2 * (hi - lo):
+            D *= 2
+        T = taps_of(D)
+        s0 = int(a["core:sample_start"])
+        s1 = s0 + int(a.get("core:sample_count", L - s0))
+        first = min(L, max(0, s0 - (T - 1) // 2))
+        n = min(L, s1 + (T - 1) // 2) - first
+        plans.append((shift, inc, D, first, (n - T) // D + 1 if n >= T else 0))
+    return plans
+
+
+def extract_schedule(spans, n_samples: int, max_chunk_samples: int):
+    """The passes of ``extract_signals`` over a file of ``n_samples``: ``spans`` holds ``(first_sample, n_out, D, T)`` per
+    job.  Chunks of ``max(max_chunk_samples, T_max)`` samples overlap by ``T_max - 1``, so every window of every job lies
+    whole in some chunk.  Yields ``(c0, c1, parts)`` for each chunk ``[c0, c1)`` that produces outputs, with ``parts`` a
+    list of ``(job, m0, n)``: the outputs ``m0 .. m0 + n - 1`` of the job whose windows lie in the chunk and that no earlier
+    chunk produced."""
+    live = [T for _, n_out, _, T in spans if n_out > 0]
+    if not live:
+        return
+    L, T_max = int(n_samples), max(live)
+    chunk = max(int(max_chunk_samples), T_max)
+    done = [0] * len(spans)
+    c0 = 0
+    while True:
+        c1 = min(L, c0 + chunk)
+        parts = []
+        for j, (first, n_out, D, T) in enumerate(spans):
+            if done[j] < n_out and c1 - T - first >= 0:
+                hi = min(n_out, (c1 - T - first) // D + 1)
+                if hi > done[j]:
+                    parts.append((j, done[j], hi - done[j]))
+                    done[j] = hi
+        if parts:
+            yield c0, c1, parts
+        if c1 >= L:
+            return
+        c0 += chunk - T_max + 1
+
+
+@dataclass
+class ExtractedSignal:
+    """One annotated region of a recording, down-converted to baseband and classified (``extract_signals``)."""
+    annotation: dict                       # the region's SigMF annotation
+    center_freq: float                     # RF centre of the baseband: the recording's fc + the tuned shift
+    sample_rate: float                     # fs / decim
+    decim: int                             # D
+    n_taps: int                            # T (ddc.design_taps(D))
+    first_sample: int                      # the recording's sample where output 0's window starts
+    iq: np.ndarray                         # complex64 [n_out] baseband outputs
+    pxx: Optional[np.ndarray]              # float64 [nfft] Welch density of iq (mlab.psd, two-sided); None without outputs
+    measurements: Optional[dict]           # features.measure_batch of 10 log10 pxx over the centre nfft / 2 bins, + Hz
+    classification: Optional[dict]         # classify_from_measurements of those bins (no temporal smoothing)
+
+    @property
+    def label(self) -> Optional[str]:
+        return self.classification["label"] if self.classification else None
+
+
+def extract_signals(path_or_rec, annotations=None, nfft: int = 256, window="hann", out_dir=None, label_parent: bool = False,
+                    max_chunk_samples: int = 1 << 26, device: int = 0) -> list:
+    """Down-convert every annotated region of a recording to its own baseband on the GPU, classify it and optionally write
+    it as a SigMF recording of its own.  ``annotations``: SigMF annotations (default: ``detect_signals`` with its
+    defaults).  Each region becomes one job of ``signal_jobs``; the jobs are grouped by decimation, one ``ddc.DdcPlan``
+    per group, and the file is read once in chunks (``extract_schedule``), each uploaded once and down-converted by one
+    ``DdcPlan.exec_jobs`` launch per group into one device buffer.  Each signal's baseband gets a Welch spectrum (``nfft``,
+    no overlap, ``window``; zero-padded to one frame like mlab when shorter than nfft), the classifier measurements of
+    the centre nfft / 2 bins (the band the region fills; one launch for all signals) and the rule table's verdict on the
+    RF axis, without temporal smoothing.  A region without a full window gets empty IQ, no spectrum and no label.
+
+    ``out_dir``: write signal k as ``<out_dir>/<recording name>.sig<k>.sigmf-{data,meta}`` (cf32_le) with its exact
+    sample rate and centre frequency, a description naming the parent and the region, and one annotation carrying the
+    label.  ``label_parent``: rewrite the recording's annotations (``write_annotations``) with each label as core:label.
+    Returns one ``ExtractedSignal`` per annotation, in order."""
+    from . import classifier as cls_mod
+    from . import ddc as ddc_mod
+    from . import features
+    from ._native import DeviceArray, DeviceView
+    nat = sp.nat
+    rec = path_or_rec if isinstance(path_or_rec, SigMFRecording) else fromfile(path_or_rec)
+    nat.require_device()
+    if annotations is None:
+        _, annotations = detect_signals(rec, device=device)
+    annotations = [dict(a) for a in annotations]
+    fs, fc, L, nfft = rec.sample_rate, rec.center_freq, rec.n_samples, int(nfft)
+    plans = signal_jobs(annotations, fs, fc, L)
+    taps = {D: ddc_mod.design_taps(D) for D in sorted({p[2] for p in plans})}
+    offs = np.concatenate([[0], np.cumsum([p[4] for p in plans], dtype=np.int64)]).astype(np.int64)
+    pl = sp.get_plan(nfft, nfft, window, FMT_CF32, 1.0, sp.DB_EPS_REFERENCE, device)
+    st = pl.stream
+    d_y = DeviceArray((max(int(offs[-1]), 1),), np.complex64, device)
+    handles = {}
+    try:
+        for D, h in taps.items():
+            handles[D] = ddc_mod.DdcPlan(fs, 0.0, D, h, rec.in_fmt, rec.in_scale, device)
+        sched = list(extract_schedule([(p[3], p[4], p[2], taps[p[2]].size) for p in plans], L, max_chunk_samples))
+        if sched:
+            d_raw = DeviceArray((max(c1 - c0 for c0, c1, _ in sched) * rec.bytes_per_sample,), np.uint8, device)
+        for c0, c1, parts in sched:
+            raw = np.ascontiguousarray(rec.raw_slice(c0, c1 - c0))
+            nat.check(nat.lib().spx_stream_sync(device, st))   # the previous chunk's kernels are done with d_raw
+            nat.check(nat.lib().spx_memcpy_h2d(device, d_raw.ptr, raw.ctypes.data, raw.nbytes))
+            x = DeviceView(d_raw.ptr, raw.shape, raw.dtype, device)
+            groups = {}
+            for j, m0, n in parts:
+                _, inc, D, first, _ = plans[j]
+                groups.setdefault(D, []).append((first, inc, m0, n, int(offs[j]) + m0))
+            for D, jobs in groups.items():
+                handles[D].exec_jobs(x, jobs, d_y, in_first_sample=c0, stream=st)
+    finally:
+        for hd in handles.values():
+            hd.close()
+    nat.check(nat.lib().spx_stream_sync(device, st))
+    y_all = d_y.to_host()
+    live = [k for k, p in enumerate(plans) if p[4] > 0]
+    d_acc = DeviceArray((max(len(live), 1), nfft), np.float64, device)
+    d_pxx = DeviceArray((max(len(live), 1), nfft), np.float64, device)
+    keep = []
+    for r, k in enumerate(live):
+        n, rate = plans[k][4], fs / plans[k][2]
+        if n >= nfft:
+            y = DeviceView(d_y.ptr + 8 * int(offs[k]), (n,), np.complex64, device)
+        else:   # mlab zero-pads a short input to one frame
+            pad = np.zeros(nfft, np.complex64)
+            pad[:n] = y_all[offs[k]:offs[k] + n]
+            y = DeviceArray.from_host(pad, device)
+            keep.append(y)
+        acc = DeviceView(d_acc.ptr + 8 * nfft * r, (1, nfft), np.float64, device)
+        res = pl.stft(y, welch=acc, stream=st)
+        pl.welch_finalize(DeviceView(acc.ptr, (nfft,), np.float64, device), res.n_frames, rate, want_db=False,
+                          pxx=DeviceView(d_pxx.ptr + 8 * nfft * r, (nfft,), np.float64, device), stream=st)
+    nat.check(nat.lib().spx_stream_sync(device, st))
+    del keep
+    pxx = d_pxx.to_host()[:len(live)]
+    lo, hi = nfft // 4, nfft - nfft // 4
+    with np.errstate(divide="ignore"):   # row by row: the dB of each returned spectrum's contiguous centre slice
+        band = np.array([10.0 * np.log10(p[lo:hi]) for p in pxx], np.float64).reshape(len(live), hi - lo)
+    meas = features.measure_batch(band, device=device) if live else []
+    out = []
+    for k, (a, (shift, _, D, first, n)) in enumerate(zip(annotations, plans)):
+        sig = ExtractedSignal(a, fc + shift, fs / D, D, int(taps[D].size), first,
+                              y_all[offs[k]:offs[k] + n].copy(), None, None, None)
+        if n:
+            r = live.index(k)
+            fj = sig.center_freq + sp.freq_axis(nfft, sig.sample_rate, 0.0)[lo:hi]
+            sig.pxx = pxx[r]
+            sig.measurements = cls_mod.add_hz(fj, meas[r])
+            sig.classification = cls_mod.classify_from_measurements(fj, meas[r], hi - lo, smooth=False)
+        out.append(sig)
+    if out_dir is not None:
+        os.makedirs(out_dir, exist_ok=True)
+        name = os.path.basename(rec.base)
+        for k, sig in enumerate(out):
+            _write_signal(os.path.join(out_dir, f"{name}.sig{k}"), sig, name)
+    if label_parent:
+        write_annotations(rec, [dict(s.annotation, **({"core:label": s.label} if s.label else {})) for s in out])
+    return out
+
+
+def _write_signal(base: str, sig: ExtractedSignal, parent: str) -> None:
+    """``<base>.sigmf-{data,meta}`` of an extracted signal: build_metadata's fields, with the exact sample rate and centre
+    (floats where they are not whole numbers) and one annotation over the whole file with the signal's label."""
+    def exact(v):
+        return int(v) if float(v).is_integer() else float(v)
+    a = sig.annotation
+    meta = build_metadata(sig.sample_rate, sig.center_freq, "cf32_le", description=(
+        f"signal extracted from {parent}: samples {a['core:sample_start']} .. "
+        f"{a['core:sample_start'] + a.get('core:sample_count', 0)}, {a['core:freq_lower_edge']:.1f} .. "
+        f"{a['core:freq_upper_edge']:.1f} Hz; down-converted by {sig.decim} from sample {sig.first_sample}"))
+    meta["global"]["core:sample_rate"] = exact(sig.sample_rate)
+    meta["captures"][0]["core:frequency"] = exact(sig.center_freq)
+    ann = {"core:sample_start": 0, "core:sample_count": int(sig.iq.size),
+           "core:freq_lower_edge": float(a["core:freq_lower_edge"]), "core:freq_upper_edge": float(a["core:freq_upper_edge"]),
+           "core:generator": GENERATOR}
+    if sig.label:
+        ann["core:label"] = sig.label
+    meta["annotations"] = [ann]
+    with open(base + ".sigmf-data", "wb") as fh:
+        fh.write(_data_bytes(sig.iq, "cf32_le"))
+    with open(base + ".sigmf-meta", "w") as fh:
+        json.dump(meta, fh, indent=2)
+
+
 def psd(path_or_rec, NFFT: int = 1024, noverlap: int = 0, max_samples: Optional[int] = None, device: int = 0):
     """``plt.psd(data, NFFT=1024, Fs=sample_rate, Fc=center_freq)`` of a recording (:188): returns
     ``(Pxx, freqs)`` in matplotlib's order."""

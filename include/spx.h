@@ -500,7 +500,9 @@ SPX_API int spx_iq_hist2d(int32_t device, int32_t mem, const void* in, int32_t i
                           double r, int32_t bins, uint32_t* hist, int32_t accumulate, void* stream);
 
 /* per-frame mean and peak of I^2+Q^2 (SURVEY.md A9; scripts/pyad-iio-test.py:93 prints the mean per
- * buffer); frames as in spx_frame_count(n, frame_len, hop); outputs float32 [F] each. */
+ * buffer); frames as in spx_frame_count(n, frame_len, hop); outputs float32 [F] each.  Non-finite powers follow
+ * numpy's mean and max: when any I^2+Q^2 of a frame is NaN, its mean_pow and peak_pow are both NaN (the peak does not
+ * skip NaN); otherwise an infinite power makes both +inf. */
 SPX_API int spx_frame_stats(int32_t device, int32_t mem, const void* in, int32_t in_fmt, float in_scale, int64_t n,
                             int32_t frame_len, int32_t hop, float* mean_pow, float* peak_pow, int64_t* n_frames_out,
                             void* stream);

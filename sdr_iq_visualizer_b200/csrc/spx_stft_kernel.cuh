@@ -230,24 +230,34 @@ inline bool stage_ok(const StftLaunch& L) {
     return true;
 }
 
-template <int N, int TWM, int OCC, bool STAGE, int TUNE = 0>
-int launch_stft_fmt(StftLaunch& L) {
-    const bool acc = L.p.welch_acc != nullptr || L.p.maxhold != nullptr;
-    if (L.in_fmt == FMT_CF32) {
-        return acc ? launch_stft_inst<N, FMT_CF32, true, TWM, OCC, STAGE, TUNE>(L)
-                   : launch_stft_inst<N, FMT_CF32, false, TWM, OCC, STAGE, TUNE>(L);
+// ACCS: which accumulator instances to build.  ACC_ANY picks at run time; a caller that has already branched on the
+// accumulators passes ACC_OFF / ACC_ON so that the other instance, which it can never launch, is not compiled.
+enum { ACC_ANY = 0, ACC_OFF = 1, ACC_ON = 2 };
+
+template <int N, int FMT, int TWM, int OCC, bool STAGE, int TUNE, int ACCS>
+int launch_stft_acc(StftLaunch& L) {
+    if constexpr (ACCS == ACC_ANY) {
+        const bool acc = L.p.welch_acc != nullptr || L.p.maxhold != nullptr;
+        return acc ? launch_stft_inst<N, FMT, true, TWM, OCC, STAGE, TUNE>(L)
+                   : launch_stft_inst<N, FMT, false, TWM, OCC, STAGE, TUNE>(L);
+    } else {
+        return launch_stft_inst<N, FMT, ACCS == ACC_ON, TWM, OCC, STAGE, TUNE>(L);
     }
-    return acc ? launch_stft_inst<N, FMT_CI16, true, TWM, OCC, STAGE, TUNE>(L)
-               : launch_stft_inst<N, FMT_CI16, false, TWM, OCC, STAGE, TUNE>(L);
+}
+
+template <int N, int TWM, int OCC, bool STAGE, int TUNE = 0, int ACCS = ACC_ANY>
+int launch_stft_fmt(StftLaunch& L) {
+    if (L.in_fmt == FMT_CF32) return launch_stft_acc<N, FMT_CF32, TWM, OCC, STAGE, TUNE, ACCS>(L);
+    return launch_stft_acc<N, FMT_CI16, TWM, OCC, STAGE, TUNE, ACCS>(L);
 }
 
 // STAGE_WANTED: use the TMA-staged kernel when the input is suitably aligned, else direct loads
-template <int N, int TWM, int OCC, bool STAGE_WANTED = false, int TUNE = 0>
+template <int N, int TWM, int OCC, bool STAGE_WANTED = false, int TUNE = 0, int ACCS = ACC_ANY>
 int launch_stft_n(StftLaunch& L) {
     if constexpr (STAGE_WANTED && StftCfg<N>::CAN_STAGE) {
-        if (stage_ok(L)) return launch_stft_fmt<N, TWM, OCC, true, TUNE>(L);
+        if (stage_ok(L)) return launch_stft_fmt<N, TWM, OCC, true, TUNE, ACCS>(L);
     }
-    return launch_stft_fmt<N, TWM, OCC, false, TUNE>(L);
+    return launch_stft_fmt<N, TWM, OCC, false, TUNE, ACCS>(L);
 }
 
 // one translation unit per size group instantiates these

@@ -362,6 +362,9 @@ __global__ void __launch_bounds__(256) hist_zero_kernel(unsigned int* __restrict
     for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) hist[i] = 0u;
 }
 
+// max that returns NaN when either operand is NaN (np.max's rule); fmaxf would skip it
+__device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
+
 template <int FMT>
 __global__ void __launch_bounds__(256) frame_stats_kernel(const void* __restrict__ in, long long n_frames, int frame_len,
                                                           int hop, float scale, float* __restrict__ mean_pow,
@@ -383,12 +386,12 @@ __global__ void __launch_bounds__(256) frame_stats_kernel(const void* __restrict
             }
             const float p = re * re + im * im;
             sum += (double)p;
-            mx = fmaxf(mx, p);
+            mx = max_nan(mx, p);
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
             sum += __shfl_xor_sync(0xffffffffu, sum, o);
-            mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+            mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         }
         __syncthreads();
         if ((threadIdx.x & 31) == 0) { s_sum[threadIdx.x >> 5] = sum; s_max[threadIdx.x >> 5] = mx; }
@@ -396,7 +399,7 @@ __global__ void __launch_bounds__(256) frame_stats_kernel(const void* __restrict
         if (threadIdx.x == 0) {
             double t = 0.0;
             float m = 0.f;
-            for (int w = 0; w < 8; ++w) { t += s_sum[w]; m = fmaxf(m, s_max[w]); }
+            for (int w = 0; w < 8; ++w) { t += s_sum[w]; m = max_nan(m, s_max[w]); }
             mean_pow[f] = (float)(t / (double)frame_len);
             peak_pow[f] = m;
         }
